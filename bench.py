@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- throughput of the dsp_icpc hot path (waveforms/s, 8192-sample UInt16 ICPC waveforms).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload W] [--batch B]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload W] [--batch B] [--dump-outputs DIR]
 
 One "step" = one pass of the chain over one batch of synthetic waveforms.
   value            the batch is already resident in HBM (CUDA events on the launching stream, max over ranks)
@@ -211,6 +211,33 @@ class CpuArm:
                 f"-march=native -fopenmp, OpenMP over events): {what}; not Julia")
 
 
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(torch, outdir, arrays, seed=0):
+    """np.save each device array of `arrays` (events on axis 0) as outdir/<name>.npy with its non-finite entries set to 0, and
+    beside it outdir/<name>_nonfinite.npy (float32, same shape): 0 finite, 1 NaN, 2 +inf, 3 -inf.  The chain's NaN / inf
+    results are real outputs; this keeps every file finite without losing them.  When the files together would exceed
+    DUMP_BYTES, each keeps the same seeded sample of events, in event order"""
+    import numpy as np
+    first = next(iter(arrays.values()))
+    n = first.shape[0]
+    per_event = sum(a[0].numel() * (a.element_size() + 4) for a in arrays.values())
+    keep = min(n, (DUMP_BYTES - 2 * 1024 * len(arrays)) // per_event)   # 1 KB per file for the .npy header
+    idx = None
+    if keep < n:
+        idx = torch.from_numpy(np.sort(np.random.default_rng(seed).choice(n, keep, replace=False))).to(first.device)
+    os.makedirs(outdir, exist_ok=True)
+    for name, a in arrays.items():
+        a = a if idx is None else a.index_select(0, idx)
+        code = torch.zeros(a.shape, dtype=torch.float32, device=a.device)
+        code[torch.isnan(a)] = 1.0
+        code[torch.isposinf(a)] = 2.0
+        code[torch.isneginf(a)] = 3.0
+        np.save(os.path.join(outdir, name + ".npy"), torch.where(code == 0, a, torch.zeros_like(a)).cpu().numpy())
+        np.save(os.path.join(outdir, name + "_nonfinite.npy"), code.cpu().numpy())
+
+
 WL_NAME = {"dsp_icpc": "full dsp_icpc, 49 columns incl. CUSP+ZAC (BASELINE configs[2]/[4])",
            "pz_trap": "pole-zero + trapezoid energy / t0 only: blmean, t0, t50, e_trap, e_10410 (BASELINE configs[1])",
            "trap_sweep": "20x10 trapezoid (rt, ft) sweep, 200 variants (BASELINE configs[3])",
@@ -235,7 +262,15 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip extra_workloads / e2e variants / value_with_gather")
     ap.add_argument("--groups", default=None, help="override the column-group mask (hex), for per-stage timing experiments")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the output arrays of the last timed step (rank 0) as DIR/<name>.npy with non-finite entries "
+                         "as 0 and their kind in DIR/<name>_nonfinite.npy; above 64 MB in all, the same fixed seeded sample "
+                         "of events from every array")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = max(args.warmup, 1)
 
@@ -404,6 +439,17 @@ def main():
     ms_max, launches = timed(step, args.steps, 0)
     clocks = sampler.stop() if rank == 0 else None
     value = world * B * args.steps / (ms_max * 1e-3)
+    if args.dump_outputs and rank == 0:
+        # before anything below reuses the output buffers
+        if args.workload == "sipm":
+            arrays = {"rows": out.view(-1)[:B * L._abi.SIPM_NCOL].view(B, L._abi.SIPM_NCOL), "triggers": out_t}
+        elif args.workload == "compressed":
+            arrays = {"rows_presummed": out, "rows_windowed": out_w, "window_stats": out_s}
+        elif args.workload == "trap_sweep":
+            arrays = {"trap_sweep": out}
+        else:
+            arrays = {"rows": out}
+        dump_outputs(torch, args.dump_outputs, arrays)
 
     # ---- e2e through the host C-ABI call (H2D + kernels + D2H inside the timed region) ----
     Be = min(B, 131072)
