@@ -131,6 +131,15 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t phase)
     while (!mbar_try_wait(bar, phase)) {}
 }
 
+// ---- cp.async (LDGSTS): 8-byte copies global -> shared, completed by commit / wait groups of the issuing thread ----
+__device__ __forceinline__ void cp_async_8(void* dst_smem, const void* src_gmem)
+{
+    asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(smem_u32(dst_smem)), "l"(src_gmem) : "memory");
+}
+__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
+template <int N>
+__device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
+
 // ---- warp / block reductions (results broadcast to all threads) ----
 constexpr unsigned FULL = 0xffffffffu;
 

@@ -720,16 +720,9 @@ struct CzStream {
         t = tn;
         return d;
     }
-    // the same with the load of the following step issued one step ahead (tpre = p[k] on entry; reads p[k + 1] <= TT[n + 1])
-    double tpre;
-    __device__ __forceinline__ void prime() { tpre = p[0]; }
-    __device__ __forceinline__ double next_fast_pf(double r, int k)
+    // the same from a prefix sum TT[j + 1] read elsewhere (the finish kernel's shared-memory slab); j is not advanced
+    __device__ __forceinline__ double next_from(double r, double tn)
     {
-        const double tn = tpre;
-        tpre = p[k + 1];
-        // every fourth step: the sector three ahead of this lane's stream into L1 (the finish kernel's lanes walk 32 different
-        // chunks, 32 sectors per load; measured in the pipeline: 6.32 -> 6.47 M wf/s, distances 8 / 12 / 20 within 0.5 %)
-        if ((k & 3) == 0) asm volatile("prefetch.global.L1 [%0];" ::"l"(p + min(k + 12, CH)));
         const double y = tn - t;
         const double d = fma(-r, yprev, y);
         yprev = y;
@@ -750,10 +743,35 @@ struct CzStream {
     }
 };
 
+// the CUSP and ZAC outputs of the current window state (s3 = the y[m-L] stream) and the state update by one step from the
+// four stream inputs a..d; shared by cz_out_each and cz_out_staged
+template <typename F>
+__device__ __forceinline__ void cz_emit(const CzDev& Z, const CzState& S, const CzStream& s3, int k, F&& f)
+{
+    const double ylast = s3.yprev;   // y[m-L]
+    const double Dc = (S.EpL - S.EmL + S.EpR - S.EmR) + S.W0F;
+    const double poly = (S.W2L - Z.h2 * S.W1L) + (S.V2 - Z.h2 * S.V1);
+    f(k, fma(Z.g, Dc, Z.gclast_cusp * ylast), fma(Z.g, fma(Z.B, poly, Dc), Z.gclast_zac * ylast));
+}
+__device__ __forceinline__ void cz_update(const CzDev& Z, CzState& S, double a, double b, double c, double d)
+{
+    S.EmL = fma(Z.rho, S.EmL, fma(Z.cA, a, -Z.cA_rho_lt * b));
+    S.EpL = fma(Z.rho_inv, S.EpL, fma(Z.cA, a, -Z.cA_rhoinv_lt * b));
+    S.W2L = S.W2L + 2.0 * S.W1L + S.W0L - Z.lt2_d * b;
+    S.W1L = S.W1L + S.W0L - Z.lt_d * b;
+    S.W0L = S.W0L + a - b;
+    S.W0F = S.W0F + b - c;
+    S.V2 = S.V2 - 2.0 * S.V1 + S.V0 + Z.Rn2_d * c;
+    S.V1 = S.V1 - S.V0 + Z.Rn_d * c;
+    S.V0 = S.V0 + c - d;
+    S.EpR = fma(Z.rho, S.EpR, fma(Z.cA_rhoinv_Rn, c, -Z.cA * d));
+    S.EmR = fma(Z.rho_inv, S.EmR, fma(Z.cA_rho_Rn, c, -Z.cA * d));
+}
+
 // CH recurrence steps of one candidate chunk: the CUSP and ZAC outputs go to obuf[k][0..1] (-inf where m0+k is not a
 // valid output); maxima, argmaxima and the pick-off windows are taken from there by a block-parallel pass.  No
 // compares or branches in the loop: the only loop-carried dependency is the state update.
-template <bool PF = false, typename F>
+template <typename F>
 __device__ __forceinline__ void cz_out_each(const CzDev& Z, const double* TT, int n, int tid, CzState& S, F&& f)
 {
     const int m0 = tid * CH;
@@ -764,51 +782,106 @@ __device__ __forceinline__ void cz_out_each(const CzDev& Z, const double* TT, in
     s1.init(TT, m0 + 1 - lt);
     s2.init(TT, m0 - lt - F_);
     s3.init(TT, m0 + 1 - L);
-    auto emit = [&](int k) {
-        const double ylast = s3.yprev;   // y[m-L]
-        const double Dc = (S.EpL - S.EmL + S.EpR - S.EmR) + S.W0F;
-        const double poly = (S.W2L - Z.h2 * S.W1L) + (S.V2 - Z.h2 * S.V1);
-        f(k, fma(Z.g, Dc, Z.gclast_cusp * ylast), fma(Z.g, fma(Z.B, poly, Dc), Z.gclast_zac * ylast));
-    };
-    auto update = [&](double a, double b, double c, double d) {
-        S.EmL = fma(Z.rho, S.EmL, fma(Z.cA, a, -Z.cA_rho_lt * b));
-        S.EpL = fma(Z.rho_inv, S.EpL, fma(Z.cA, a, -Z.cA_rhoinv_lt * b));
-        S.W2L = S.W2L + 2.0 * S.W1L + S.W0L - Z.lt2_d * b;
-        S.W1L = S.W1L + S.W0L - Z.lt_d * b;
-        S.W0L = S.W0L + a - b;
-        S.W0F = S.W0F + b - c;
-        S.V2 = S.V2 - 2.0 * S.V1 + S.V0 + Z.Rn2_d * c;
-        S.V1 = S.V1 - S.V0 + Z.Rn_d * c;
-        S.V0 = S.V0 + c - d;
-        S.EpR = fma(Z.rho, S.EpR, fma(Z.cA_rhoinv_Rn, c, -Z.cA * d));
-        S.EmR = fma(Z.rho_inv, S.EmR, fma(Z.cA_rho_Rn, c, -Z.cA * d));
-    };
     const bool interior = (m0 - L >= 1) && (m0 + CH + 1 <= n);
-    if (interior && PF) {
-        // loads one step ahead (global-memory prefix sums: the finish kernel of the split pipeline)
-        s0.prime(); s1.prime(); s2.prime(); s3.prime();
+    if (interior) {
 #pragma unroll 1
         for (int k = 0; k < CH; ++k) {
-            emit(k);
-            const double a = s0.next_fast_pf(r, k), b = s1.next_fast_pf(r, k), c = s2.next_fast_pf(r, k), d = s3.next_fast_pf(r, k);
-            update(a, b, c, d);
-        }
-    } else if (interior) {
-#pragma unroll 1
-        for (int k = 0; k < CH; ++k) {
-            emit(k);
+            cz_emit(Z, S, s3, k, f);
             const double a = s0.next_fast(r, k), b = s1.next_fast(r, k), c = s2.next_fast(r, k), d = s3.next_fast(r, k);
-            update(a, b, c, d);
+            cz_update(Z, S, a, b, c, d);
         }
     } else {
 #pragma unroll 1
         for (int k = 0; k < CH; ++k) {
             const int m = m0 + k;
-            if (m >= L - 1 && m < n) emit(k);
+            if (m >= L - 1 && m < n) cz_emit(Z, S, s3, k, f);
             else f(k, -CUDART_INF, -CUDART_INF);
             const double a = s0.next_safe(TT, r, n), b = s1.next_safe(TT, r, n), c = s2.next_safe(TT, r, n),
                          d = s3.next_safe(TT, r, n);
-            update(a, b, c, d);
+            cz_update(Z, S, a, b, c, d);
+        }
+    }
+}
+
+// The same CH steps for the candidate chunks of a whole warp, one lane each, with TT in global memory (the finish kernel of
+// the split pipeline).  Lane-private loads there would make every load instruction touch 32 unrelated sectors and leave the
+// recurrence waiting on L2 each step; instead the warp stages steps 1..CH-1 in pieces of CZ_STAGE steps into a
+// double-buffered slab in shared memory, cooperatively: one cp.async instruction fetches CZ_STAGE consecutive prefix sums
+// of 32 / CZ_STAGE candidates, and the next piece is in flight while the current one is stepped.  Slab layout
+// [buffer][stream][step][lane ^ swizzle(step)]: a step of all 32 lanes is one conflict-free LDS.64 row, and the swizzle
+// makes the cooperative stores conflict-free too.  Every lane reads TT[clamp(j + 1, 0, n)] as next_safe does, so chunks at
+// the trace ends take the same values as in cz_out_each (for interior chunks the clamp is void), and every float64
+// operation keeps its operands and order.  All 32 lanes must call it (warp-synchronous); lanes without a candidate
+// (has == false, chunk 0) help to stage and never call f.  nact: candidates of the warp (lanes 0..nact-1).
+#ifndef LGDSP_CZ_STAGE
+#define LGDSP_CZ_STAGE 4
+#endif
+constexpr int CZ_STAGE = LGDSP_CZ_STAGE;   // steps per staged piece (a power of two dividing CH - 1 = 32)
+static_assert(CZ_STAGE >= 1 && CZ_STAGE <= 32 && (CZ_STAGE & (CZ_STAGE - 1)) == 0 && (CH - 1) % CZ_STAGE == 0, "stage piece");
+constexpr int CZ_SLAB = 2 * 4 * CZ_STAGE * 32;   // doubles of one warp's slab
+template <typename F>
+__device__ __forceinline__ void cz_out_staged(const CzDev& Z, const double* TT, int n, int chunk, bool has, int nact, CzState& S,
+                                              double* slab, int lane, F&& f)
+{
+    constexpr int G = 32 / CZ_STAGE;   // candidates per cp.async instruction
+    const int m0 = chunk * CH;
+    const int L = Z.L, lt = Z.lt, F_ = Z.F;
+    const double r = Z.r;
+    const int jofs[4] = {1, 1 - lt, -lt - F_, 1 - L};   // stream starts j0 - m0 (CzStream::init)
+    // staging piece p = steps 1 + p * CZ_STAGE + i, i < CZ_STAGE; this lane copies step i = lane % CZ_STAGE of candidates
+    // g * G + lane / CZ_STAGE
+    const int si = lane % CZ_STAGE;
+    auto stage = [&](int p) {
+        double* b = slab + (p & 1) * (4 * CZ_STAGE * 32) + si * 32;
+        const int kk = 2 + p * CZ_STAGE + si;   // TT index of this step's input = j0 + 1 + k
+#pragma unroll
+        for (int g = 0; g < CZ_STAGE; ++g) {
+            const int c = g * G + lane / CZ_STAGE;
+            const int mc = __shfl_sync(FULL, m0, c);
+            if (c < nact) {
+#pragma unroll
+                for (int s = 0; s < 4; ++s)
+                    cp_async_8(b + s * (CZ_STAGE * 32) + (c ^ (si * G)), TT + min(max(mc + jofs[s] + kk, 0), n));
+            }
+        }
+        cp_async_commit();
+    };
+    stage(0);
+    CzStream s0, s1, s2, s3;
+    s0.init(TT, m0 + jofs[0]);
+    s1.init(TT, m0 + jofs[1]);
+    s2.init(TT, m0 + jofs[2]);
+    s3.init(TT, m0 + jofs[3]);
+    auto out = [&](int k) {
+        const int m = m0 + k;
+        if (m >= L - 1 && m < n) cz_emit(Z, S, s3, k, f);   // always so for interior chunks
+        else f(k, -CUDART_INF, -CUDART_INF);
+    };
+    if (has) out(0);
+    {
+        const double a = s0.next_safe(TT, r, n), b = s1.next_safe(TT, r, n), c = s2.next_safe(TT, r, n), d = s3.next_safe(TT, r, n);
+        cz_update(Z, S, a, b, c, d);
+    }
+    constexpr int NP = (CH - 1) / CZ_STAGE;
+#pragma unroll 1
+    for (int p = 0; p < NP; ++p) {
+        if (p + 1 < NP) {
+            __syncwarp();   // every lane is done with the buffer of piece p - 1
+            stage(p + 1);
+            cp_async_wait<1>();
+        } else {
+            cp_async_wait<0>();
+        }
+        __syncwarp();       // piece p of every lane has landed
+        const double* b = slab + (p & 1) * (4 * CZ_STAGE * 32);
+#pragma unroll 1
+        for (int i = 0; i < CZ_STAGE; ++i) {
+            const int k = 1 + p * CZ_STAGE + i;
+            if (has) out(k);
+            const int col = i * 32 + (lane ^ (i * G));
+            const double a = s0.next_from(r, b[col]), bb = s1.next_from(r, b[CZ_STAGE * 32 + col]),
+                         c = s2.next_from(r, b[2 * CZ_STAGE * 32 + col]), d = s3.next_from(r, b[3 * CZ_STAGE * 32 + col]);
+            cz_update(Z, S, a, bb, c, d);
         }
     }
 }

@@ -1076,11 +1076,12 @@ enum { K3S_PKP = 0 /* 2 */, K3S_PP0 = 2, K3S_YMAX = 3 };
 
 // Candidate selection of one structured pass: closed-form window states at every chunk
 // start (tab_c / tab_a read the prefix tables), coarse CUSP / ZAC values, Lipschitz bound against the best coarse value,
-// candidate records + header -> cg.  Contains two block barriers; every thread of the block must call it.
-template <typename TC, typename TA>
+// candidate records + header -> cg.  Contains two block barriers; every thread of the block must call it.  tt_dead() runs in
+// every thread right behind the first of them, from where on nothing here reads TT.
+template <typename TC, typename TA, typename TD>
 __device__ __forceinline__ void cz_select(const CzDev& Z, const double* TT, int n, int nw, double pp0, double Ymax, const int* pk_from,
                                           const double* pk_p, bool want_cusp, bool want_zac, double* czco, double* red, int* czn,
-                                          double* cg, TC&& tab_c, TA&& tab_a)
+                                          double* cg, TC&& tab_c, TA&& tab_a, TD&& tt_dead)
 {
     const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
     const int i0 = tid * CH;
@@ -1104,6 +1105,7 @@ __device__ __forceinline__ void cz_select(const CzDev& Z, const double* TT, int 
         }
     }
     __syncthreads();   // tables are dead, coarse values complete
+    tt_dead();
     double Mc, Mz;
     int Ac, Az;
     red_argmax(red, K3R_CZMAX0, K3R_CZARG0, Mc, Ac);
@@ -1194,14 +1196,23 @@ icpc_cuspzac_kernel(const __grid_constant__ IcpcDev P, const double* __restrict_
     }
     __syncthreads();
 
+    // one bulk copy of TT per event, one expect_tx per mbarrier phase (it & 1); the issuing thread orders the generic-proxy
+    // reads of the previous event (made visible to it by a block barrier) before the copy with fence_proxy_async
+    auto load_tt = [&](long long ee) {
+        fence_proxy_async();
+        mbar_expect_tx(bar, tt_bytes);
+        tma_load_1d(TT, ttg + ee * TTG_LEN, tt_bytes, bar);
+        // the event after it into L2 while this one computes: its bulk copy then runs at L2 speed (+2 %)
+        if (ee + gridDim.x < n_events) tma_prefetch_l2(ttg + (ee + gridDim.x) * TTG_LEN, tt_bytes);
+    };
+    // structured passes: the first event's copy is issued here and every further one as soon as the last pass of the event
+    // before has stopped reading TT (cz_select's tt_dead), so that it lands while that event's candidates are selected
+    if (npass != 0 && tid == 0 && blockIdx.x < n_events) load_tt(blockIdx.x);
+
     uint32_t it = 0;
     for (long long e = blockIdx.x; e < n_events; e += gridDim.x, ++it) {
         if (tid == 0) {
-            fence_proxy_async();
-            mbar_expect_tx(bar, tt_bytes);
-            tma_load_1d(TT, ttg + e * TTG_LEN, tt_bytes, bar);
-            // the next event of this CTA into L2 while this one computes: its bulk copy then runs at L2 speed (+2 %)
-            if (e + gridDim.x < n_events) tma_prefetch_l2(ttg + (e + gridDim.x) * TTG_LEN, tt_bytes);
+            if (npass == 0) load_tt(e);
             ibuf[K3I_CZN] = 0;
         }
         mbar_wait(bar, it & 1u);
@@ -1274,7 +1285,7 @@ icpc_cuspzac_kernel(const __grid_constant__ IcpcDev P, const double* __restrict_
         }
         // One pass of the structured evaluation up to the candidate selection.  The descriptor index is a compile-time
         // constant so that its fields are immediate constant-bank operands.
-        auto cz_pass = [&](auto psc, const bool want_cusp, const bool want_zac, const bool rescan) {
+        auto cz_pass = [&](auto psc, const bool want_cusp, const bool want_zac, const bool rescan, const bool last) {
             constexpr int ps = decltype(psc)::value;
             const CzDev& Z = P.cz[ps];
             double* cg = czg + e * CZG_LEN + ps * CZP_LEN;
@@ -1288,20 +1299,26 @@ icpc_cuspzac_kernel(const __grid_constant__ IcpcDev P, const double* __restrict_
             cz_select(Z, TT, n, nw, scr[K3S_PP0], scr[K3S_YMAX], pk_from, scr + K3S_PKP, want_cusp, want_zac, czco, red,
                       &ibuf[K3I_CZN], cg,
                       [&](int q, int kind, int c) -> double { return tabA[(q * 3 + kind) * NT + c]; },
-                      [&](int q, int c) -> double { return tabA[(12 + q) * NT + c]; });
+                      [&](int q, int c) -> double { return tabA[(12 + q) * NT + c]; },
+                      [&]() {
+                          // Past this barrier of the last pass nothing of this event reads TT again: the pick-off windows,
+                          // the scan (cz_scan), the window states (cz_init_with) and the coarse grid (cz_coarse) are all
+                          // behind it, and the rest of cz_select works on registers, czco, red, scr and the header.
+                          if (last && tid == 0 && e + gridDim.x < n_events) load_tt(e + gridDim.x);
+                      });
         };
         if (npass == 2) {
-            cz_pass(std::integral_constant<int, 1>{}, false, true, false);
-            cz_pass(std::integral_constant<int, 0>{}, true, false, true);
+            cz_pass(std::integral_constant<int, 1>{}, false, true, false, false);
+            cz_pass(std::integral_constant<int, 0>{}, true, false, true, true);
         } else {
-            cz_pass(std::integral_constant<int, 0>{}, true, true, false);
+            cz_pass(std::integral_constant<int, 0>{}, true, true, false, true);
         }
-        __syncthreads();   // TT, scr, ibuf may be overwritten by the next event
+        __syncthreads();   // scr, ibuf may be overwritten by the next event
     }
 }
 
 // finish: one lane per candidate chunk, one warp per event -- and up to K4_NBLK warps for an event with more than 32
-// candidates.  The kernel is bound by the latency of a round (33 dependent recurrence steps on prefix sums in L2 / HBM), and
+// candidates.  The kernel is bound by the latency of a round (33 dependent recurrence steps; cz_out_staged feeds them from shared memory), and
 // 93 % of the events need one round (median 11 candidates) while the 3 % noise-only events, where all 248 chunks are
 // candidates, needed eight rounds on one warp: they set the duration of every launch.  Warp w < n_events takes the first 32
 // candidates of event w; the warps behind take the further blocks of the few events that have them (and exit at once
@@ -1314,6 +1331,7 @@ icpc_cuspzac_finish_kernel(const __grid_constant__ IcpcDev P, const double* __re
                            double* __restrict__ czg, long long n_events, double* __restrict__ rows)
 {
     __shared__ double stash_s[K4_WARPS][2][LGDSP_MAX_DNI];
+    __shared__ __align__(16) double slab_s[K4_WARPS][CZ_SLAB];   // cz_out_staged
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
     const int n = P.n;
     const int nw = P.sig_dni.n_w;
@@ -1339,14 +1357,12 @@ icpc_cuspzac_finish_kernel(const __grid_constant__ IcpcDev P, const double* __re
         const double* TT = ttg + e * TTG_LEN;
         double czmax[2] = {-CUDART_INF, -CUDART_INF};
         int czarg[2] = {0x7fffffff, 0x7fffffff};
-        double pk_p[2] = {0.0, 0.0};
         int pk_from[2] = {0, 0};
         auto pass = [&](auto psc, const bool want_cusp, const bool want_zac) {
             constexpr int ps = decltype(psc)::value;
             const CzDev& Z = P.cz[ps];
             const double* cg = ce + ps * CZP_LEN;
             const int ncand = (int)cg[CZH_N];
-            pk_p[0] = cg[CZH_PKP0]; pk_p[1] = cg[CZH_PKP1];
             pk_from[0] = (int)cg[CZH_PKF0]; pk_from[1] = (int)cg[CZH_PKF1];
             if (lane == 0 && kb == 0) {
                 // the coarse points are outputs themselves
@@ -1355,15 +1371,21 @@ icpc_cuspzac_finish_kernel(const __grid_constant__ IcpcDev P, const double* __re
             }
 #pragma unroll 1
             for (int c0 = 32 * kb; c0 < ncand; c0 += 32 * nwork) {
-                if (c0 + lane < ncand) {
+                const bool has = c0 + lane < ncand;
+                CzState st;
+                int chunk = 0;
+                if (has) {
                     const double* r = cg + CZ_HDR + (size_t)(c0 + lane) * CZ_REC;
-                    CzState st;
                     st.EmL = r[0]; st.EpL = r[1]; st.W0L = r[2]; st.W1L = r[3]; st.W2L = r[4]; st.W0F = r[5];
                     st.V0 = r[6]; st.V1 = r[7]; st.V2 = r[8]; st.EpR = r[9]; st.EmR = r[10];
-                    st.active = true;
-                    const int chunk = (int)r[11];
+                    chunk = (int)r[11];
+                } else {
+                    st.EmL = st.EpL = st.W0L = st.W1L = st.W2L = st.W0F = st.V0 = st.V1 = st.V2 = st.EpR = st.EmR = 0.0;
+                }
+                st.active = has;
+                {
                     const int jb = chunk * CH - Z.L + 1;
-                    cz_out_each<true>(Z, TT, n, chunk, st, [&](int k, double o_c, double o_z) {
+                    cz_out_staged(Z, TT, n, chunk, has, min(32, ncand - c0), st, slab_s[wid], lane, [&](int k, double o_c, double o_z) {
                         const int j = jb + k;
                         if (want_cusp) {
                             if (o_c > czmax[0] || (o_c == czmax[0] && j < czarg[0])) { czmax[0] = o_c; czarg[0] = j; }
@@ -1414,8 +1436,9 @@ icpc_cuspzac_finish_kernel(const __grid_constant__ IcpcDev P, const double* __re
             __syncwarp();
             win = sm;
         }
-        const double vc = dni_eval_warp(A_sig, nw, P.sig_dni.m, win, pk_p[0] - (double)pk_from[0], lane);
-        const double vz = dni_eval_warp(A_sig, nw, P.sig_dni.m, win + LGDSP_MAX_DNI, pk_p[1] - (double)pk_from[1], lane);
+        // (the pick-off positions of the last pass, pass 0, read only here: they would hold four registers in the recurrence)
+        const double vc = dni_eval_warp(A_sig, nw, P.sig_dni.m, win, ce[CZH_PKP0] - (double)pk_from[0], lane);
+        const double vz = dni_eval_warp(A_sig, nw, P.sig_dni.m, win + LGDSP_MAX_DNI, ce[CZH_PKP1] - (double)pk_from[1], lane);
         if (lane == 0 && auxg[e * AUX_LEN + AX_BAD] != 0.0) {
             double* ro = rows + e * LGDSP_NCOL;
             ro[LGDSP_COL_e_cusp_max] = ro[LGDSP_COL_t_cusp_max] = ro[LGDSP_COL_e_cusp] = CUDART_NAN;
