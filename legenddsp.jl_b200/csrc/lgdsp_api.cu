@@ -6,6 +6,7 @@
 #include <cstdarg>
 #include <cstdio>
 #include <cstring>
+#include <functional>
 #include <string>
 #include <thread>
 #include <vector>
@@ -14,6 +15,7 @@
 using namespace lgdsp;
 
 #define LGDSP_SPLIT_MAX_STREAMS 6
+#define LGDSP_HOST_ARRAYS 5   // per-event arrays one host entry point moves (dsp_icpc_compressed: 2 in, 3 out)
 
 struct lgdsp_handle {
     int device = 0;
@@ -31,7 +33,7 @@ struct lgdsp_handle {
     int phase_grid = 0;
     bool phase_on = false;
     SweepVar* d_vars = nullptr;
-    int vars_cap = 0;
+    size_t vars_cap = 0;
     double* d_taps = nullptr;      // differenced FIR / SG taps of the sweep variants
     size_t taps_cap = 0;
     IcpcDev icpc{};
@@ -42,18 +44,12 @@ struct lgdsp_handle {
     double* d_dniA_w = nullptr;
     double* d_cusp_g_w = nullptr;
     double* d_zac_g_w = nullptr;
-    void* d_cin[2][2] = {{nullptr, nullptr}, {nullptr, nullptr}};   // [buffer][pre, wdw] staging of the compressed host path
-    size_t cin_cap[2] = {0, 0};
-    double* d_crows = nullptr;
-    size_t crows_cap = 0;
-    // host-path staging
-    uint16_t* d_in[2] = {nullptr, nullptr};
-    double* d_rows = nullptr;
-    double* d_aux = nullptr;   // per-event external baselines / shifts (two chunks)
-    size_t aux_cap = 0;
-    int* d_win = nullptr;      // window list of lgdsp_window_stats_run
-    void* d_sweep_out = nullptr;
-    size_t in_cap = 0, rows_cap = 0, sweep_out_cap = 0;
+    int* d_win = nullptr;      // window list of the window statistics: [LGDSP_MAX_STAT_WINDOWS][2]
+    // device slots of the chunked host paths (run_chunked): [buffer][array], the dense rows of one chunk
+    void* d_slot[2][LGDSP_HOST_ARRAYS] = {};
+    size_t slot_cap[2][LGDSP_HOST_ARRAYS] = {};
+    double* d_prim = nullptr;  // trace in, results out of the single-trace primitives
+    size_t prim_cap = 0;
     cudaStream_t s_copy = nullptr;
     cudaEvent_t ev_ready[2] = {nullptr, nullptr}, ev_free[2] = {nullptr, nullptr};
     // pinned staging of the host paths (HostIO below): pageable caller memory goes through these double buffers
@@ -66,12 +62,12 @@ struct lgdsp_handle {
     int64_t host_chunk_direct = 8192;   // the same for raw samples copied directly from page-locked caller memory
     int64_t host_chunk = 16384;    // events per chunk of the host paths (4096 / 8192 / 16384 / 32768 measured: 16384 is the best of the four for pageable, pinned and encoded input)
     // encoded-waveform staging (decode_data on the device)
-    uint8_t* d_enc[2][2] = {{nullptr, nullptr}, {nullptr, nullptr}};   // [buffer][stream]
-    size_t enc_cap[2] = {0, 0};
-    long long* d_off[2][2] = {{nullptr, nullptr}, {nullptr, nullptr}};
-    size_t off_cap = 0;
-    void* d_dec[2] = {nullptr, nullptr};                               // decoded waveforms of the current chunk
-    size_t dec_cap[2] = {0, 0};
+    uint8_t* d_enc[2][2] = {};     // [buffer][input]
+    size_t enc_cap[2][2] = {};
+    long long* d_off[2][2] = {};
+    size_t off_cap[2][2] = {};
+    void* d_dec[2] = {};           // [input] decoded waveforms of the current chunk
+    size_t dec_cap[2] = {};
     int* d_dstat = nullptr;
     size_t dstat_cap = 0;
     // timing
@@ -173,6 +169,7 @@ int lgdsp_create(int device, void* stream, lgdsp_handle** out)
     ok = ok && cudaMalloc(&h->d_cusp_g, sizeof(double) * (LGDSP_MAX_FIR + 1)) == cudaSuccess;
     ok = ok && cudaMalloc(&h->d_zac_g, sizeof(double) * (LGDSP_MAX_FIR + 1)) == cudaSuccess;
     ok = ok && cudaMalloc(&h->d_sweep_dniA, sizeof(double) * LGDSP_MAX_DNI * 4) == cudaSuccess;
+    ok = ok && cudaMalloc(&h->d_win, sizeof(int) * 2 * LGDSP_MAX_STAT_WINDOWS) == cudaSuccess;
     if (!ok) { fail(nullptr, LGDSP_ERR_CUDA, "lgdsp_create: resource allocation failed: %s", cudaGetErrorString(cudaGetLastError())); return bail(LGDSP_ERR_CUDA); }
     if ((e = icpc_configure(&h->icpc_bps)) != cudaSuccess || (e = sweep_configure(&h->sweep_bps)) != cudaSuccess) {
         fail(nullptr, LGDSP_ERR_CUDA, "kernel configuration failed: %s (is the library built for this GPU?)", cudaGetErrorString(e));
@@ -224,11 +221,10 @@ void lgdsp_destroy(lgdsp_handle* h)
     cudaFree(h->d_tt); cudaFree(h->d_saux); cudaFree(h->d_scz);
     cudaFree(h->d_phase);
     cudaFree(h->d_dniA); cudaFree(h->d_cusp_g); cudaFree(h->d_zac_g); cudaFree(h->d_sweep_dniA); cudaFree(h->d_vars); cudaFree(h->d_taps);
-    cudaFree(h->d_in[0]); cudaFree(h->d_in[1]); cudaFree(h->d_rows); cudaFree(h->d_sweep_out);
-    cudaFree(h->d_aux); cudaFree(h->d_win);
-    cudaFree(h->d_dniA_w); cudaFree(h->d_cusp_g_w); cudaFree(h->d_zac_g_w); cudaFree(h->d_crows);
-    for (int b = 0; b < 2; ++b) for (int k = 0; k < 2; ++k) cudaFree(h->d_cin[b][k]);
+    cudaFree(h->d_win); cudaFree(h->d_prim);
+    cudaFree(h->d_dniA_w); cudaFree(h->d_cusp_g_w); cudaFree(h->d_zac_g_w);
     for (int i = 0; i < 2; ++i) {
+        for (int k = 0; k < LGDSP_HOST_ARRAYS; ++k) cudaFree(h->d_slot[i][k]);
         if (h->ev_ready[i]) cudaEventDestroy(h->ev_ready[i]);
         if (h->ev_free[i]) cudaEventDestroy(h->ev_free[i]);
         if (h->ev_pin[i]) cudaEventDestroy(h->ev_pin[i]);
@@ -526,6 +522,20 @@ static int check_wf(lgdsp_handle* h, const void* wf, int64_t n_events, int64_t l
     return LGDSP_OK;
 }
 
+// Grows a device buffer of the handle to at least `bytes`; the contents are not kept.  Work on either stream may still use
+// the old buffer, so both are synchronised before it is freed.
+template <class T>
+static int grow(lgdsp_handle* h, T** p, size_t* cap, size_t bytes)
+{
+    if (bytes <= *cap) return LGDSP_OK;
+    CK(cudaStreamSynchronize(h->stream));
+    CK(cudaStreamSynchronize(h->s_copy));
+    cudaFree(*p); *p = nullptr; *cap = 0;
+    CK(cudaMalloc(p, bytes));
+    *cap = bytes;
+    return LGDSP_OK;
+}
+
 // One dsp_icpc pass over a device batch, in stream order behind h->stream.  Fused path: one launch of icpc_kernel.  Split
 // path: the batch is cut into sub-batches whose prefix sums (65.6 KB per event) fit the L2; sub-batches alternate between
 // side streams (forked from / joined to h->stream with events) so that the tail of one kernel overlaps the next sub-batch.
@@ -698,32 +708,6 @@ int lgdsp_icpc_run_ext_device(lgdsp_handle* h, const lgdsp_icpc_params* p, const
     return icpc_run_device_impl(h, p, d_wf, sample_bytes, d_baseline, n_events, ld_samples, d_out_rows);
 }
 
-static int ensure_staging(lgdsp_handle* h, size_t in_bytes, size_t rows_bytes)
-{
-    if (in_bytes > h->in_cap) {
-        for (int i = 0; i < 2; ++i) { cudaFree(h->d_in[i]); h->d_in[i] = nullptr; }
-        h->in_cap = 0;
-        for (int i = 0; i < 2; ++i) CK(cudaMalloc(&h->d_in[i], in_bytes));
-        h->in_cap = in_bytes;
-    }
-    if (rows_bytes > h->rows_cap) {
-        cudaFree(h->d_rows); h->d_rows = nullptr; h->rows_cap = 0;
-        CK(cudaMalloc(&h->d_rows, rows_bytes));
-        h->rows_cap = rows_bytes;
-    }
-    return LGDSP_OK;
-}
-
-static int ensure_aux(lgdsp_handle* h, size_t bytes)
-{
-    if (bytes > h->aux_cap) {
-        cudaFree(h->d_aux); h->d_aux = nullptr; h->aux_cap = 0;
-        CK(cudaMalloc(&h->d_aux, bytes));
-        h->aux_cap = bytes;
-    }
-    return LGDSP_OK;
-}
-
 // ---------------------------------------------------------------------------------------------------
 // Host <-> device traffic of the chunked host paths.  Caller memory that is already page-locked (cudaHostAlloc /
 // cudaHostRegister / torch pin_memory) is copied directly; PAGEABLE caller memory (a Julia `flatview(wvfs.signal)`, a numpy
@@ -766,7 +750,7 @@ struct HostIO {
     lgdsp_handle* h;
     int b = 0;                 // double-buffer index of the current chunk
     size_t in_used = 0, out_used = 0;
-    struct Pending { void* dst; const void* src; size_t bytes; };
+    struct Pending { void* dst; size_t dpitch; const void* src; size_t width, rows; };
     std::vector<Pending> pending[2];   // pinned -> caller copies that wait for ev_out[b]
     bool used_pin[2] = {false, false}, used_out[2] = {false, false};
 
@@ -794,7 +778,7 @@ struct HostIO {
     int flush(int bb)
     {
         if (used_out[bb]) { CK(cudaEventSynchronize(h->ev_out[bb])); used_out[bb] = false; }
-        for (const Pending& q : pending[bb]) memcpy(q.dst, q.src, q.bytes);
+        for (const Pending& q : pending[bb]) pack_rows(q.dst, q.dpitch, q.src, q.width, q.width, q.rows, h->copy_threads);
         pending[bb].clear();
         return LGDSP_OK;
     }
@@ -833,16 +817,21 @@ struct HostIO {
         CK(cudaStreamWaitEvent(h->stream, h->ev_ready[b], 0));
         return LGDSP_OK;
     }
-    // device -> caller, in stream order behind the kernels of this chunk
-    int d2h(void* dst, const void* d_src, size_t bytes, bool dst_pinned)
+    // dense device rows of `width` bytes -> caller rows `dpitch` bytes apart, in stream order behind the kernels of this chunk
+    int d2h(void* dst, size_t dpitch, const void* d_src, size_t width, size_t rows, bool dst_pinned)
     {
-        if (bytes == 0) return LGDSP_OK;
-        if (dst_pinned) { CK(cudaMemcpyAsync(dst, d_src, bytes, cudaMemcpyDeviceToHost, h->stream)); return LGDSP_OK; }
+        if (width == 0 || rows == 0) return LGDSP_OK;
+        if (dst_pinned) {
+            if (dpitch == width) CK(cudaMemcpyAsync(dst, d_src, width * rows, cudaMemcpyDeviceToHost, h->stream));
+            else CK(cudaMemcpy2DAsync(dst, dpitch, d_src, width, width, rows, cudaMemcpyDeviceToHost, h->stream));
+            return LGDSP_OK;
+        }
+        const size_t bytes = width * rows;
         if (out_used + bytes > h->out_cap) return fail(h, LGDSP_ERR_CUDA, "internal: pinned output staging too small");
         char* stage = static_cast<char*>(h->h_out[b]) + out_used;
         out_used = up256(out_used + bytes);
         CK(cudaMemcpyAsync(stage, d_src, bytes, cudaMemcpyDeviceToHost, h->stream));
-        pending[b].push_back({dst, stage, bytes});
+        pending[b].push_back({dst, dpitch, stage, width, rows});
         used_out[b] = true;
         return LGDSP_OK;
     }
@@ -861,53 +850,28 @@ struct HostIO {
     }
 };
 
-static int ensure_bytes(lgdsp_handle* h, void** p, size_t* cap, size_t bytes)
-{
-    if (bytes > *cap) {
-        CK(cudaStreamSynchronize(h->stream));
-        CK(cudaStreamSynchronize(h->s_copy));
-        cudaFree(*p); *p = nullptr; *cap = 0;
-        CK(cudaMalloc(p, bytes));
-        *cap = bytes;
-    }
-    return LGDSP_OK;
-}
-
 // One encoded stream set of a chunk -> decoded device rows: upload of the byte range and of the offsets slice (copy stream),
-// decode kernel (compute stream, behind inputs_ready).  `slot` = 0 / 1: the two waveforms of dsp_icpc_compressed.
+// decode kernel (compute stream, behind inputs_ready).  `slot` = 0 / 1: the input index (dsp_icpc_compressed has two).
 struct EncodedInput {
     int codec, sample_bytes, n_samples, shift;
     const uint8_t* enc;
     const int64_t* offsets;
     bool enc_pinned, off_pinned;
 };
-static int encoded_reserve(lgdsp_handle* h, const EncodedInput& in, int slot, int64_t chunk, int64_t n_events)
+// device buffers of one encoded input; adds what its uploads take of the pinned input staging to *stage_in
+static int encoded_reserve(lgdsp_handle* h, const EncodedInput& in, int slot, int64_t chunk, int64_t n_events, size_t* stage_in)
 {
-    size_t max_bytes = 0;
-    for (int64_t e0 = 0; e0 < n_events; e0 += chunk) {
-        const int64_t e1 = e0 + chunk < n_events ? e0 + chunk : n_events;
-        const size_t nb = (size_t)(in.offsets[e1] - in.offsets[e0]);
-        max_bytes = nb > max_bytes ? nb : max_bytes;
+    size_t max_bytes = 0;   // the longest byte range of one chunk
+    for (int64_t e0 = 0; e0 < n_events; e0 += chunk)
+        max_bytes = std::max(max_bytes, (size_t)(in.offsets[std::min(e0 + chunk, n_events)] - in.offsets[e0]));
+    if (!in.enc_pinned || !in.off_pinned) *stage_in += max_bytes + (size_t)(chunk + 1) * sizeof(int64_t) + 512;
+    int rc = LGDSP_OK;
+    for (int b = 0; b < 2 && !rc; ++b) {
+        rc = grow(h, &h->d_enc[b][slot], &h->enc_cap[b][slot], max_bytes + 16);
+        if (!rc) rc = grow(h, &h->d_off[b][slot], &h->off_cap[b][slot], (size_t)(chunk + 1) * sizeof(long long));
     }
-    for (int bb = 0; bb < 2; ++bb) {
-        size_t cap = h->enc_cap[slot];
-        int rc = ensure_bytes(h, reinterpret_cast<void**>(&h->d_enc[bb][slot]), &cap, max_bytes + 16);
-        if (rc) return rc;
-        if (bb == 1) h->enc_cap[slot] = cap;
-    }
-    if ((size_t)(chunk + 1) * sizeof(long long) > h->off_cap) {
-        CK(cudaStreamSynchronize(h->stream));
-        CK(cudaStreamSynchronize(h->s_copy));
-        for (int bb = 0; bb < 2; ++bb)
-            for (int k = 0; k < 2; ++k) {
-                cudaFree(h->d_off[bb][k]); h->d_off[bb][k] = nullptr;
-                CK(cudaMalloc(&h->d_off[bb][k], (size_t)(chunk + 1) * sizeof(long long)));
-            }
-        h->off_cap = (size_t)(chunk + 1) * sizeof(long long);
-    }
-    int rc = ensure_bytes(h, &h->d_dec[slot], &h->dec_cap[slot], (size_t)chunk * in.n_samples * in.sample_bytes);
-    if (rc) return rc;
-    return ensure_bytes(h, reinterpret_cast<void**>(&h->d_dstat), &h->dstat_cap, 2 * sizeof(int));
+    if (!rc) rc = grow(h, &h->d_dec[slot], &h->dec_cap[slot], (size_t)chunk * in.n_samples * in.sample_bytes);
+    return rc ? rc : grow(h, &h->d_dstat, &h->dstat_cap, 2 * sizeof(int));
 }
 // d_dstat = {number of malformed streams, smallest event index among them} of the running call
 static int decode_err_reset(lgdsp_handle* h)
@@ -923,16 +887,6 @@ static int decode_err_check(lgdsp_handle* h)
     CK(cudaMemcpy(st, h->d_dstat, sizeof(st), cudaMemcpyDeviceToHost));
     if (st[0]) return fail(h, LGDSP_ERR_INVALID_ARG, "%d malformed encoded waveform(s), first at event %d", st[0], st[1]);
     return LGDSP_OK;
-}
-static size_t encoded_stage_bytes(const EncodedInput& in, int64_t chunk, int64_t n_events)
-{
-    size_t m = 0;
-    for (int64_t e0 = 0; e0 < n_events; e0 += chunk) {
-        const int64_t e1 = e0 + chunk < n_events ? e0 + chunk : n_events;
-        const size_t nb = (size_t)(in.offsets[e1] - in.offsets[e0]) + (size_t)(e1 - e0 + 1) * sizeof(int64_t) + 512;
-        m = nb > m ? nb : m;
-    }
-    return m;
 }
 static int encoded_upload(lgdsp_handle* h, HostIO& io, const EncodedInput& in, int slot, int64_t e0, int64_t ne)
 {
@@ -966,11 +920,95 @@ static int check_encoded(lgdsp_handle* h, int codec, const void* enc, const int6
         if (offsets[e + 1] < offsets[e]) return fail(h, LGDSP_ERR_INVALID_ARG, "offsets must be non-decreasing (event %lld)", (long long)e);
     return LGDSP_OK;
 }
-// host buffers in, host rows out: chunked, H2D of chunk k+1 overlaps the kernels of chunk k.  `encin` != NULL: the input
-// is an encoded waveform set (decode_data on the device), else raw samples `wf`.
+// One per-event array of caller memory that a host entry point moves: `width` bytes per event, `pitch` bytes from one event to
+// the next in caller memory, dense rows on the device (the TMA and the 128-bit loads of the kernels rely on that).
+// host == NULL: an optional array that is not given; its device pointer is NULL.
+struct HostArray {
+    const void* host;
+    size_t pitch, width;
+    bool pinned;
+    const EncodedInput* enc;   // input given as encoded streams (decode_data on the device in front of the launch)
+    int from_input;            // output whose device rows are those of this input (no device buffer of its own), else -1
+};
+static HostArray host_array(const void* p, size_t pitch, size_t width)
+{
+    return HostArray{p, pitch, width, p && is_pinned(p), nullptr, -1};
+}
+static HostArray wf_array(const void* wf, size_t pitch, size_t width, const EncodedInput* enc)
+{
+    return enc ? HostArray{nullptr, 0, 0, false, enc, -1} : host_array(wf, pitch, width);
+}
+
+// The chunk loop of every host entry point.  The inputs of chunk c go up on the copy stream while the compute stream runs
+// chunk c-1; the compute stream waits for them, decodes encoded inputs, runs launch(ne, d) and copies the outputs back.
+// d[k] holds the device rows of input k, then of output k - in.size(), in double-buffered slots of the handle.
+typedef std::function<int(int64_t ne, void* const* d)> ChunkLaunch;
+static int run_chunked(lgdsp_handle* h, int64_t n_events, int64_t chunk, const std::vector<HostArray>& in,
+                       const std::vector<HostArray>& out, const ChunkLaunch& launch)
+{
+    chunk = std::min(chunk, n_events);
+    const size_t ni = in.size(), na = ni + out.size();
+    if (na > LGDSP_HOST_ARRAYS) return fail(h, LGDSP_ERR_CUDA, "internal: %zu host arrays", na);
+    HostIO io(h);
+    size_t stage_in = 0, stage_out = 0;
+    bool encoded = false;
+    int rc = LGDSP_OK;
+    for (size_t k = 0; k < na && !rc; ++k) {
+        const HostArray& a = k < ni ? in[k] : out[k - ni];
+        if (a.enc) {
+            encoded = true;
+            rc = encoded_reserve(h, *a.enc, (int)k, chunk, n_events, &stage_in);
+        } else if (a.host) {
+            if (!a.pinned) (k < ni ? stage_in : stage_out) += (size_t)chunk * a.width + 256;
+            for (int b = 0; b < 2 && !rc && a.from_input < 0; ++b) rc = grow(h, &h->d_slot[b][k], &h->slot_cap[b][k], (size_t)chunk * a.width);
+        }
+    }
+    if (!rc) rc = io.reserve(stage_in, stage_out);
+    if (!rc && encoded) rc = decode_err_reset(h);
+    if (rc) return rc;
+    void* d[LGDSP_HOST_ARRAYS];
+    int c = 0;
+    for (int64_t e0 = 0; e0 < n_events; e0 += chunk, ++c) {
+        const int64_t ne = std::min(chunk, n_events - e0);
+        rc = io.begin_chunk(c);
+        if (rc) return rc;
+        const int b = io.b;
+        if (c >= 2) CK(cudaStreamWaitEvent(h->s_copy, h->ev_free[b], 0));   // the device buffers of chunk c-2 are consumed
+        for (size_t k = 0; k < na; ++k) {
+            const HostArray& a = k < ni ? in[k] : out[k - ni];
+            d[k] = a.enc ? h->d_dec[k] : a.from_input >= 0 ? d[a.from_input] : a.host ? h->d_slot[b][k] : nullptr;
+            if (k >= ni) continue;
+            if (a.enc) rc = encoded_upload(h, io, *a.enc, (int)k, e0, ne);
+            else if (a.host) rc = io.h2d(d[k], static_cast<const char*>(a.host) + (size_t)e0 * a.pitch, a.pitch, a.width, (size_t)ne, a.pinned);
+            if (rc) return rc;
+        }
+        rc = io.inputs_ready();
+        if (rc) return rc;
+        // (d_dec is single-buffered: what reads it -- the launch, or the D2H of decode_data -- is in stream order in front of
+        // the next chunk's decode kernel)
+        for (size_t k = 0; k < ni && !rc; ++k)
+            if (in[k].enc) rc = encoded_decode(h, io, *in[k].enc, (int)k, e0, ne);
+        if (!rc) rc = launch(ne, d);
+        if (rc) return rc;
+        CK(cudaEventRecord(h->ev_free[b], h->stream));
+        for (size_t k = ni; k < na && !rc; ++k) {
+            const HostArray& a = out[k - ni];
+            if (a.host) rc = io.d2h(const_cast<char*>(static_cast<const char*>(a.host)) + (size_t)e0 * a.pitch, a.pitch, d[k], a.width,
+                                    (size_t)ne, a.pinned);
+        }
+        if (!rc) rc = io.end_chunk();
+        if (rc) return rc;
+    }
+    rc = io.finish();
+    if (rc) return rc;
+    return encoded ? decode_err_check(h) : LGDSP_OK;
+}
+
+// host buffers in, host rows out.  `encin` != NULL: the input is an encoded waveform set (decode_data on the device), else
+// raw samples `wf`.
 static int icpc_run_host_impl(lgdsp_handle* h, const lgdsp_icpc_params* p, const void* wf, int sample_bytes,
                               const double* baseline, int64_t n_events, int64_t ld_samples, double* out_rows,
-                              const EncodedInput* encin = nullptr)
+                              EncodedInput* encin = nullptr)
 {
     if (!h) return LGDSP_ERR_INVALID_ARG;
     CK(cudaSetDevice(h->device));
@@ -979,6 +1017,7 @@ static int icpc_run_host_impl(lgdsp_handle* h, const lgdsp_icpc_params* p, const
     const int n = h->icpc.n;
     int rc;
     if (encin) {
+        encin->n_samples = n;
         if (n_events < 0) return fail(h, LGDSP_ERR_INVALID_ARG, "n_events < 0");
         if (sample_bytes == 4 && n > LGDSP_MAX_SAMPLES / 2) return fail(h, LGDSP_ERR_UNSUPPORTED, "32-bit samples: n_samples = %d > %d", n, LGDSP_MAX_SAMPLES / 2);
         rc = check_encoded(h, encin->codec, encin->enc, encin->offsets, n_events, sample_bytes);
@@ -988,70 +1027,16 @@ static int icpc_run_host_impl(lgdsp_handle* h, const lgdsp_icpc_params* p, const
     if (rc) return rc;
     if (n_events == 0) return LGDSP_OK;
     if (!out_rows) return fail(h, LGDSP_ERR_INVALID_ARG, "output pointer is NULL");
-    const size_t sb = (size_t)sample_bytes;
-    const bool in_pinned = encin ? false : is_pinned(wf);
+    const HostArray wf_in = wf_array(wf, (size_t)ld_samples * sample_bytes, (size_t)n * sample_bytes, encin);
     // raw samples straight from page-locked memory are bound by the host link: smaller chunks shorten the un-overlapped first
     // copy / last kernel (3.25 vs 3.13 M wf/s); staged and encoded input prefers the larger chunk (2.27 vs 1.76 M wf/s pageable)
-    const int64_t want = (in_pinned && h->host_chunk_direct < h->host_chunk) ? h->host_chunk_direct : h->host_chunk;
-    const int64_t chunk = n_events < want ? n_events : want;
-    const bool out_pinned = is_pinned(out_rows);
-    const bool bl_pinned = baseline ? is_pinned(baseline) : true;
-    HostIO io(h);
-    size_t stage_in = 0;
-    if (encin) stage_in = (encin->enc_pinned && encin->off_pinned) ? 0 : encoded_stage_bytes(*encin, chunk, n_events);
-    else if (!in_pinned) stage_in = (size_t)chunk * n * sb + 256;
-    if (baseline && !bl_pinned) stage_in += (size_t)chunk * sizeof(double) + 256;
-    rc = io.reserve(stage_in, out_pinned ? 0 : (size_t)chunk * LGDSP_NCOL * sizeof(double) + 256);
-    if (rc) return rc;
-    rc = ensure_staging(h, encin ? 16 : (size_t)chunk * n * sb, (size_t)2 * chunk * LGDSP_NCOL * sizeof(double));
-    if (rc) return rc;
-    if (encin) {
-        rc = encoded_reserve(h, *encin, 0, chunk, n_events);
-        if (rc) return rc;
-        rc = decode_err_reset(h);
-        if (rc) return rc;
-    }
-    if (baseline) {
-        rc = ensure_aux(h, (size_t)2 * chunk * sizeof(double));
-        if (rc) return rc;
-    }
-    const unsigned char* src = static_cast<const unsigned char*>(wf);
-    int c = 0;
-    for (int64_t e0 = 0; e0 < n_events; e0 += chunk, ++c) {
-        const int64_t ne = (n_events - e0) < chunk ? (n_events - e0) : chunk;
-        rc = io.begin_chunk(c);
-        if (rc) return rc;
-        const int b = io.b;
-        if (c >= 2) CK(cudaStreamWaitEvent(h->s_copy, h->ev_free[b], 0));   // the device buffers of chunk c-2 are consumed
-        if (encin) rc = encoded_upload(h, io, *encin, 0, e0, ne);
-        else rc = io.h2d(h->d_in[b], src + (size_t)e0 * ld_samples * sb, (size_t)ld_samples * sb, (size_t)n * sb, (size_t)ne, in_pinned);
-        if (rc) return rc;
-        double* d_bl = nullptr;
-        if (baseline) {
-            d_bl = h->d_aux + (size_t)b * chunk;
-            rc = io.h2d(d_bl, baseline + e0, (size_t)ne * sizeof(double), (size_t)ne * sizeof(double), 1, bl_pinned);
-            if (rc) return rc;
-        }
-        rc = io.inputs_ready();
-        if (rc) return rc;
-        const void* d_wf = h->d_in[b];
-        if (encin) {
-            rc = encoded_decode(h, io, *encin, 0, e0, ne);
-            if (rc) return rc;
-            d_wf = h->d_dec[0];
-        }
-        double* d_rows = h->d_rows + (size_t)b * chunk * LGDSP_NCOL;
-        rc = icpc_dispatch(h, h->icpc, d_wf, sample_bytes, ne, n, d_bl, 1, 1.0, d_rows);
-        if (rc) return rc;
-        CK(cudaEventRecord(h->ev_free[b], h->stream));
-        rc = io.d2h(out_rows + e0 * LGDSP_NCOL, d_rows, (size_t)ne * LGDSP_NCOL * sizeof(double), out_pinned);
-        if (rc) return rc;
-        rc = io.end_chunk();
-        if (rc) return rc;
-    }
-    rc = io.finish();
-    if (rc) return rc;
-    return encin ? decode_err_check(h) : LGDSP_OK;
+    const int64_t chunk = (wf_in.pinned && h->host_chunk_direct < h->host_chunk) ? h->host_chunk_direct : h->host_chunk;
+    const size_t row = LGDSP_NCOL * sizeof(double);
+    return run_chunked(h, n_events, chunk, {wf_in, host_array(baseline, sizeof(double), sizeof(double))}, {host_array(out_rows, row, row)},
+                       [&](int64_t ne, void* const* d) {
+                           return icpc_dispatch(h, h->icpc, d[0], sample_bytes, ne, n, static_cast<const double*>(d[1]), 1, 1.0,
+                                                static_cast<double*>(d[2]));
+                       });
 }
 
 int lgdsp_icpc_run(lgdsp_handle* h, const lgdsp_icpc_params* p, const uint16_t* wf, int64_t n_events,
@@ -1119,69 +1104,30 @@ int lgdsp_decode_data(lgdsp_handle* h, int32_t codec, const uint8_t* enc, const 
     if (n_events == 0) return LGDSP_OK;
     if (!wf) return fail(h, LGDSP_ERR_INVALID_ARG, "output pointer is NULL");
     EncodedInput in{codec, sample_bytes, n_samples, shift, enc, offsets, is_pinned(enc), is_pinned(offsets)};
-    const int64_t chunk = n_events < 8192 ? n_events : 8192;
-    const bool out_pinned = is_pinned(wf);
-    const size_t row = (size_t)n_samples * sample_bytes;
-    HostIO io(h);
-    rc = io.reserve((in.enc_pinned && in.off_pinned) ? 0 : encoded_stage_bytes(in, chunk, n_events), out_pinned ? 0 : (size_t)chunk * row + 256);
-    if (rc) return rc;
-    rc = encoded_reserve(h, in, 0, chunk, n_events);
-    if (rc) return rc;
-    rc = decode_err_reset(h);
-    if (rc) return rc;
-    int c = 0;
-    for (int64_t e0 = 0; e0 < n_events; e0 += chunk, ++c) {
-        const int64_t ne = (n_events - e0) < chunk ? (n_events - e0) : chunk;
-        rc = io.begin_chunk(c);
-        if (rc) return rc;
-        if (c >= 2) CK(cudaStreamWaitEvent(h->s_copy, h->ev_free[io.b], 0));
-        rc = encoded_upload(h, io, in, 0, e0, ne);
-        if (rc) return rc;
-        rc = io.inputs_ready();
-        if (rc) return rc;
-        rc = encoded_decode(h, io, in, 0, e0, ne);
-        if (rc) return rc;
-        CK(cudaEventRecord(h->ev_free[io.b], h->stream));
-        // (d_dec is single-buffered: the D2H below is in stream order in front of the next chunk's decode kernel)
-        if (ld_samples == n_samples) {
-            rc = io.d2h(static_cast<char*>(wf) + (size_t)e0 * row, h->d_dec[0], (size_t)ne * row, out_pinned);
-        } else {
-            for (int64_t e = 0; e < ne && !rc; ++e)
-                rc = io.d2h(static_cast<char*>(wf) + (size_t)(e0 + e) * ld_samples * sample_bytes, static_cast<char*>(h->d_dec[0]) + (size_t)e * row,
-                            row, out_pinned);
-        }
-        if (rc) return rc;
-        rc = io.end_chunk();
-        if (rc) return rc;
-    }
-    rc = io.finish();
-    if (rc) return rc;
-    return decode_err_check(h);
+    // the output is the decoded rows themselves: nothing to launch
+    HostArray rows = host_array(wf, (size_t)ld_samples * sample_bytes, (size_t)n_samples * sample_bytes);
+    rows.from_input = 0;
+    return run_chunked(h, n_events, 8192, {wf_array(nullptr, 0, 0, &in)}, {rows}, [](int64_t, void* const*) { return (int)LGDSP_OK; });
 }
 
 // dsp_icpc on ENCODED waveforms: the host link carries the codec's bytes, decode_data runs on the device in front of the chain
 int lgdsp_icpc_run_encoded(lgdsp_handle* h, const lgdsp_icpc_params* p, int32_t codec, const uint8_t* enc, const int64_t* offsets,
                            int32_t shift, int32_t sample_bytes, const double* baseline, int64_t n_events, double* out_rows)
 {
-    if (!h) return LGDSP_ERR_INVALID_ARG;
-    CK(cudaSetDevice(h->device));
-    if (p) { int rc = icpc_prepare(h, p); if (rc) return rc; }
-    if (!h->have_icpc) return fail(h, LGDSP_ERR_INVALID_ARG, "no parameters set");
-    EncodedInput in{codec, sample_bytes, h->icpc.n, shift, enc, offsets, enc ? is_pinned(enc) : false, offsets ? is_pinned(offsets) : false};
-    return icpc_run_host_impl(h, nullptr, nullptr, sample_bytes, baseline, n_events, h->icpc.n, out_rows, &in);
+    EncodedInput in{codec, sample_bytes, 0, shift, enc, offsets, enc ? is_pinned(enc) : false, offsets ? is_pinned(offsets) : false};
+    return icpc_run_host_impl(h, p, nullptr, sample_bytes, baseline, n_events, 0, out_rows, &in);
 }
 
-// signalstats on n_windows windows of every waveform (optionally shifted by -shift[e]): out double[n_events][n_windows][5]
-int lgdsp_window_stats_run_device(lgdsp_handle* h, const void* d_wf, int32_t sample_bytes, int64_t n_events, int32_t n_samples,
-                                  int64_t ld_samples, double t_first_ns, double dt_ns, const double* d_shift,
-                                  const int32_t* windows, int32_t n_windows, double* d_out)
+// the checks lgdsp_window_stats_run and _run_device share (nothing to do when n_events or n_windows is 0)
+static int window_stats_check(lgdsp_handle* h, const void* wf, int sample_bytes, int64_t n_events, int n_samples, int64_t ld_samples,
+                              double t_first_ns, double dt_ns, const int32_t* windows, int n_windows, const double* out)
 {
     if (!h) return LGDSP_ERR_INVALID_ARG;
     CK(cudaSetDevice(h->device));
     if (sample_bytes != 2 && sample_bytes != 4) return fail(h, LGDSP_ERR_UNSUPPORTED, "sample_bytes = %d", sample_bytes);
     if (n_events < 0 || n_windows < 0 || n_windows > LGDSP_MAX_STAT_WINDOWS) return fail(h, LGDSP_ERR_INVALID_ARG, "bad n_events / n_windows");
     if (n_events == 0 || n_windows == 0) return LGDSP_OK;
-    if (!d_wf || !windows || !d_out) return fail(h, LGDSP_ERR_INVALID_ARG, "NULL pointer");
+    if (!wf || !windows || !out) return fail(h, LGDSP_ERR_INVALID_ARG, "NULL pointer");
     if (n_samples < 1 || ld_samples < n_samples) return fail(h, LGDSP_ERR_INVALID_ARG, "bad n_samples / ld_samples");
     if (!(dt_ns > 0) || !std::isfinite(t_first_ns)) return fail(h, LGDSP_ERR_INVALID_ARG, "bad time axis");
     for (int w = 0; w < n_windows; ++w) {
@@ -1189,7 +1135,16 @@ int lgdsp_window_stats_run_device(lgdsp_handle* h, const void* d_wf, int32_t sam
         // @assert firstindex(X) <= first(idxs) <= last(idxs) <= lastindex(X)   /root/reference/src/tailstats.jl:23-25
         if (!(0 <= a && a <= b && b <= n_samples - 1)) return fail(h, LGDSP_ERR_INVALID_ARG, "window %d (%d:%d) outside the waveform", w, a, b);
     }
-    if (!h->d_win) CK(cudaMalloc(&h->d_win, sizeof(int) * 2 * LGDSP_MAX_STAT_WINDOWS));
+    return LGDSP_OK;
+}
+
+// signalstats on n_windows windows of every waveform (optionally shifted by -shift[e]): out double[n_events][n_windows][5]
+int lgdsp_window_stats_run_device(lgdsp_handle* h, const void* d_wf, int32_t sample_bytes, int64_t n_events, int32_t n_samples,
+                                  int64_t ld_samples, double t_first_ns, double dt_ns, const double* d_shift,
+                                  const int32_t* windows, int32_t n_windows, double* d_out)
+{
+    int rc = window_stats_check(h, d_wf, sample_bytes, n_events, n_samples, ld_samples, t_first_ns, dt_ns, windows, n_windows, d_out);
+    if (rc || n_events == 0 || n_windows == 0) return rc;
     CK(cudaMemcpyAsync(h->d_win, windows, sizeof(int) * 2 * (size_t)n_windows, cudaMemcpyHostToDevice, h->stream));
     CK(cudaEventRecord(h->ev0, h->stream));
     window_stats_launch(d_wf, sample_bytes, n_events, ld_samples, t_first_ns, dt_ns, d_shift, 1, 0xFFFFFFFFu, h->d_win, n_windows, d_out, h->stream);
@@ -1206,32 +1161,19 @@ int lgdsp_window_stats_run(lgdsp_handle* h, const void* wf, int32_t sample_bytes
                            int64_t ld_samples, double t_first_ns, double dt_ns, const double* shift,
                            const int32_t* windows, int32_t n_windows, double* out)
 {
-    if (!h) return LGDSP_ERR_INVALID_ARG;
-    CK(cudaSetDevice(h->device));
-    if (sample_bytes != 2 && sample_bytes != 4) return fail(h, LGDSP_ERR_UNSUPPORTED, "sample_bytes = %d", sample_bytes);
-    if (n_events < 0 || n_windows < 0 || n_windows > LGDSP_MAX_STAT_WINDOWS) return fail(h, LGDSP_ERR_INVALID_ARG, "bad n_events / n_windows");
-    if (n_events == 0 || n_windows == 0) return LGDSP_OK;
-    if (!wf || !out) return fail(h, LGDSP_ERR_INVALID_ARG, "NULL pointer");
-    if (n_samples < 1 || ld_samples < n_samples) return fail(h, LGDSP_ERR_INVALID_ARG, "bad n_samples / ld_samples");
-    const size_t sb = (size_t)sample_bytes;
-    const int64_t chunk = n_events < 8192 ? n_events : 8192;
-    const size_t out_per = (size_t)n_windows * 5;
-    int rc = ensure_staging(h, (size_t)chunk * n_samples * sb, (size_t)chunk * out_per * sizeof(double));
-    if (rc) return rc;
-    if (shift) { rc = ensure_aux(h, (size_t)chunk * sizeof(double)); if (rc) return rc; }
-    const unsigned char* src = static_cast<const unsigned char*>(wf);
-    for (int64_t e0 = 0; e0 < n_events; e0 += chunk) {
-        const int64_t ne = (n_events - e0) < chunk ? (n_events - e0) : chunk;
-        CK(cudaMemcpy2DAsync(h->d_in[0], (size_t)n_samples * sb, src + (size_t)e0 * ld_samples * sb, (size_t)ld_samples * sb,
-                             (size_t)n_samples * sb, (size_t)ne, cudaMemcpyHostToDevice, h->stream));
-        if (shift) CK(cudaMemcpyAsync(h->d_aux, shift + e0, (size_t)ne * sizeof(double), cudaMemcpyHostToDevice, h->stream));
-        rc = lgdsp_window_stats_run_device(h, h->d_in[0], sample_bytes, ne, n_samples, n_samples, t_first_ns, dt_ns,
-                                           shift ? h->d_aux : nullptr, windows, n_windows, h->d_rows);
-        if (rc) return rc;
-        CK(cudaMemcpyAsync(out + (size_t)e0 * out_per, h->d_rows, (size_t)ne * out_per * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
-        CK(cudaStreamSynchronize(h->stream));
-    }
-    return LGDSP_OK;
+    int rc = window_stats_check(h, wf, sample_bytes, n_events, n_samples, ld_samples, t_first_ns, dt_ns, windows, n_windows, out);
+    if (rc || n_events == 0 || n_windows == 0) return rc;
+    // (run_chunked synchronises the stream before it returns: the window list is consumed by then)
+    CK(cudaMemcpyAsync(h->d_win, windows, sizeof(int) * 2 * (size_t)n_windows, cudaMemcpyHostToDevice, h->stream));
+    const size_t sb = (size_t)sample_bytes, out_per = (size_t)n_windows * 5 * sizeof(double);
+    return run_chunked(h, n_events, 8192, {host_array(wf, (size_t)ld_samples * sb, (size_t)n_samples * sb), host_array(shift, sizeof(double), sizeof(double))},
+                       {host_array(out, out_per, out_per)}, [&](int64_t ne, void* const* d) {
+                           window_stats_launch(d[0], sample_bytes, ne, n_samples, t_first_ns, dt_ns, static_cast<const double*>(d[1]), 1,
+                                               0xFFFFFFFFu, h->d_win, n_windows, static_cast<double*>(d[2]), h->stream);
+                           CK(cudaGetLastError());
+                           h->launches += 1;
+                           return (int)LGDSP_OK;
+                       });
 }
 
 // ---- dsp_icpc_compressed: presummed + windowed waveform per event (/root/reference/src/dsp_icpc.jl:293-499) ----
@@ -1250,7 +1192,6 @@ static int compressed_prepare(lgdsp_handle* h, const lgdsp_icpc_params* p_pre, c
         const int a = aux[2 * w], b = aux[2 * w + 1];
         if (!(0 <= a && a <= b && b <= n - 1)) return fail(h, LGDSP_ERR_INVALID_ARG, "auxiliary window %d (%d:%d) outside the presummed waveform", w, a, b);
     }
-    if (!h->d_win) CK(cudaMalloc(&h->d_win, sizeof(int) * 2 * LGDSP_MAX_STAT_WINDOWS));
     // window order of the statistics output: auxbl1, auxbl2, bl_window (raw), auxpz1, auxpz2 (baseline-subtracted)
     const int win[10] = {aux[0], aux[1], aux[2], aux[3], h->icpc.bl_from, h->icpc.bl_until, aux[4], aux[5], aux[6], aux[7]};
     CK(cudaMemcpyAsync(h->d_win, win, sizeof(win), cudaMemcpyHostToDevice, h->stream));
@@ -1303,7 +1244,7 @@ int lgdsp_icpc_compressed_run_device(lgdsp_handle* h, const lgdsp_icpc_params* p
 // host buffers: raw samples (wf_* != NULL) or encoded waveform sets (enc_* != NULL) per waveform kind
 static int compressed_run_host_impl(lgdsp_handle* h, const lgdsp_icpc_params* p_pre, const lgdsp_icpc_params* p_wdw, const void* wf_pre,
                                     int pre_sample_bytes, int64_t ld_pre, const void* wf_wdw, int wdw_sample_bytes, int64_t ld_wdw,
-                                    const EncodedInput* enc_pre, const EncodedInput* enc_wdw, double presum_rate,
+                                    EncodedInput* enc_pre, EncodedInput* enc_wdw, double presum_rate,
                                     const int32_t* aux_windows, int64_t n_events, double* rows_pre, double* rows_wdw, double* stats)
 {
     if (!h) return LGDSP_ERR_INVALID_ARG;
@@ -1311,85 +1252,27 @@ static int compressed_run_host_impl(lgdsp_handle* h, const lgdsp_icpc_params* p_
     int rc = compressed_prepare(h, p_pre, p_wdw, pre_sample_bytes, wdw_sample_bytes, presum_rate, aux_windows);
     if (rc) return rc;
     const int np = h->icpc.n, nw = h->icpc_w.n;
-    EncodedInput ep{}, ew{};
-    if (enc_pre) { ep = *enc_pre; ep.n_samples = np; rc = check_encoded(h, ep.codec, ep.enc, ep.offsets, n_events, pre_sample_bytes); }
+    if (enc_pre) { enc_pre->n_samples = np; rc = check_encoded(h, enc_pre->codec, enc_pre->enc, enc_pre->offsets, n_events, pre_sample_bytes); }
     else rc = check_wf(h, wf_pre, n_events, ld_pre, np, false, pre_sample_bytes);
     if (rc) return rc;
-    if (enc_wdw) { ew = *enc_wdw; ew.n_samples = nw; rc = check_encoded(h, ew.codec, ew.enc, ew.offsets, n_events, wdw_sample_bytes); }
+    if (enc_wdw) { enc_wdw->n_samples = nw; rc = check_encoded(h, enc_wdw->codec, enc_wdw->enc, enc_wdw->offsets, n_events, wdw_sample_bytes); }
     else rc = check_wf(h, wf_wdw, n_events, ld_wdw, nw, false, wdw_sample_bytes);
     if (rc) return rc;
     if (n_events < 0) return fail(h, LGDSP_ERR_INVALID_ARG, "n_events < 0");
     if (n_events == 0) return LGDSP_OK;
     if (!rows_pre || !rows_wdw || !stats) return fail(h, LGDSP_ERR_INVALID_ARG, "output pointer is NULL");
-    const int64_t chunk = n_events < h->host_chunk ? n_events : h->host_chunk;
     const size_t sbp = (size_t)pre_sample_bytes, sbw = (size_t)wdw_sample_bytes;
-    const size_t need[2] = {enc_pre ? 16 : (size_t)chunk * np * sbp, enc_wdw ? 16 : (size_t)chunk * nw * sbw};
-    for (int k = 0; k < 2; ++k)
-        if (need[k] > h->cin_cap[k]) {
-            CK(cudaStreamSynchronize(h->stream));
-            CK(cudaStreamSynchronize(h->s_copy));
-            for (int b = 0; b < 2; ++b) { cudaFree(h->d_cin[b][k]); h->d_cin[b][k] = nullptr; }
-            h->cin_cap[k] = 0;
-            for (int b = 0; b < 2; ++b) CK(cudaMalloc(&h->d_cin[b][k], need[k]));
-            h->cin_cap[k] = need[k];
-        }
-    const size_t per_event = 2 * LGDSP_NCOL + 5 * LGDSP_NSTAT;
-    if ((size_t)2 * chunk * per_event * sizeof(double) > h->crows_cap) {
-        CK(cudaStreamSynchronize(h->stream));
-        cudaFree(h->d_crows); h->d_crows = nullptr; h->crows_cap = 0;
-        CK(cudaMalloc(&h->d_crows, (size_t)2 * chunk * per_event * sizeof(double)));
-        h->crows_cap = (size_t)2 * chunk * per_event * sizeof(double);
-    }
-    const bool pin_pre = enc_pre ? (ep.enc_pinned && ep.off_pinned) : is_pinned(wf_pre);
-    const bool pin_wdw = enc_wdw ? (ew.enc_pinned && ew.off_pinned) : is_pinned(wf_wdw);
-    const bool pin_out = is_pinned(rows_pre) && is_pinned(rows_wdw) && is_pinned(stats);
-    HostIO io(h);
-    size_t stage_in = 0;
-    if (!pin_pre) stage_in += (enc_pre ? encoded_stage_bytes(ep, chunk, n_events) : (size_t)chunk * np * sbp) + 512;
-    if (!pin_wdw) stage_in += (enc_wdw ? encoded_stage_bytes(ew, chunk, n_events) : (size_t)chunk * nw * sbw) + 512;
-    rc = io.reserve(stage_in, pin_out ? 0 : (size_t)chunk * per_event * sizeof(double) + 1024);
-    if (rc) return rc;
-    if (enc_pre) { rc = encoded_reserve(h, ep, 0, chunk, n_events); if (rc) return rc; }
-    if (enc_wdw) { rc = encoded_reserve(h, ew, 1, chunk, n_events); if (rc) return rc; }
-    if (enc_pre || enc_wdw) { rc = decode_err_reset(h); if (rc) return rc; }
-    const unsigned char* sp = static_cast<const unsigned char*>(wf_pre);
-    const unsigned char* sw = static_cast<const unsigned char*>(wf_wdw);
-    int c = 0;
-    for (int64_t e0 = 0; e0 < n_events; e0 += chunk, ++c) {
-        const int64_t ne = (n_events - e0) < chunk ? (n_events - e0) : chunk;
-        rc = io.begin_chunk(c);
-        if (rc) return rc;
-        const int b = io.b;
-        if (c >= 2) CK(cudaStreamWaitEvent(h->s_copy, h->ev_free[b], 0));
-        if (enc_pre) rc = encoded_upload(h, io, ep, 0, e0, ne);
-        else rc = io.h2d(h->d_cin[b][0], sp + (size_t)e0 * ld_pre * sbp, (size_t)ld_pre * sbp, (size_t)np * sbp, (size_t)ne, pin_pre);
-        if (rc) return rc;
-        if (enc_wdw) rc = encoded_upload(h, io, ew, 1, e0, ne);
-        else rc = io.h2d(h->d_cin[b][1], sw + (size_t)e0 * ld_wdw * sbw, (size_t)ld_wdw * sbw, (size_t)nw * sbw, (size_t)ne, pin_wdw);
-        if (rc) return rc;
-        rc = io.inputs_ready();
-        if (rc) return rc;
-        const void* d_pre = h->d_cin[b][0];
-        const void* d_wdw = h->d_cin[b][1];
-        if (enc_pre) { rc = encoded_decode(h, io, ep, 0, e0, ne); if (rc) return rc; d_pre = h->d_dec[0]; }
-        if (enc_wdw) { rc = encoded_decode(h, io, ew, 1, e0, ne); if (rc) return rc; d_wdw = h->d_dec[1]; }
-        double* d_rp = h->d_crows + (size_t)b * chunk * per_event;
-        double* d_rw = d_rp + (size_t)chunk * LGDSP_NCOL;
-        double* d_st = d_rw + (size_t)chunk * LGDSP_NCOL;
-        rc = compressed_launch(h, d_pre, pre_sample_bytes, np, d_wdw, wdw_sample_bytes, nw, presum_rate, ne, d_rp, d_rw, d_st);
-        if (rc) return rc;
-        CK(cudaGetLastError());
-        CK(cudaEventRecord(h->ev_free[b], h->stream));
-        rc = io.d2h(rows_pre + e0 * LGDSP_NCOL, d_rp, (size_t)ne * LGDSP_NCOL * sizeof(double), pin_out);
-        if (!rc) rc = io.d2h(rows_wdw + e0 * LGDSP_NCOL, d_rw, (size_t)ne * LGDSP_NCOL * sizeof(double), pin_out);
-        if (!rc) rc = io.d2h(stats + e0 * 5 * LGDSP_NSTAT, d_st, (size_t)ne * 5 * LGDSP_NSTAT * sizeof(double), pin_out);
-        if (rc) return rc;
-        rc = io.end_chunk();
-        if (rc) return rc;
-    }
-    rc = io.finish();
-    if (rc) return rc;
-    return (enc_pre || enc_wdw) ? decode_err_check(h) : LGDSP_OK;
+    const size_t row = LGDSP_NCOL * sizeof(double), st = 5 * LGDSP_NSTAT * sizeof(double);
+    return run_chunked(h, n_events, h->host_chunk,
+                       {wf_array(wf_pre, (size_t)ld_pre * sbp, (size_t)np * sbp, enc_pre), wf_array(wf_wdw, (size_t)ld_wdw * sbw, (size_t)nw * sbw, enc_wdw)},
+                       {host_array(rows_pre, row, row), host_array(rows_wdw, row, row), host_array(stats, st, st)},
+                       [&](int64_t ne, void* const* d) {
+                           int rc = compressed_launch(h, d[0], pre_sample_bytes, np, d[1], wdw_sample_bytes, nw, presum_rate, ne,
+                                                      static_cast<double*>(d[2]), static_cast<double*>(d[3]), static_cast<double*>(d[4]));
+                           if (rc) return rc;
+                           CK(cudaGetLastError());
+                           return (int)LGDSP_OK;
+                       });
 }
 
 int lgdsp_icpc_compressed_run(lgdsp_handle* h, const lgdsp_icpc_params* p_pre, const lgdsp_icpc_params* p_wdw, const void* wf_pre,
@@ -1510,16 +1393,9 @@ static int sweep_prepare(lgdsp_handle* h, const lgdsp_sweep_params* p, const lgd
             return fail(h, LGDSP_ERR_INVALID_ARG, "variant %d: unknown kind %d", v, in.kind);
         }
     }
-    if (nvar > h->vars_cap) {
-        cudaFree(h->d_vars); h->d_vars = nullptr; h->vars_cap = 0;
-        CK(cudaMalloc(&h->d_vars, sizeof(SweepVar) * nvar));
-        h->vars_cap = nvar;
-    }
-    if (taps.size() > h->taps_cap) {
-        cudaFree(h->d_taps); h->d_taps = nullptr; h->taps_cap = 0;
-        CK(cudaMalloc(&h->d_taps, sizeof(double) * taps.size()));
-        h->taps_cap = taps.size();
-    }
+    int rc = grow(h, &h->d_vars, &h->vars_cap, sizeof(SweepVar) * nvar);
+    if (!rc) rc = grow(h, &h->d_taps, &h->taps_cap, sizeof(double) * taps.size());
+    if (rc) return rc;
     for (int v = 0; v < nvar; ++v)
         if (sv[v].kind != 0) sv[v].g = h->d_taps + tap_off[v];
     if (!taps.empty()) CK(cudaMemcpyAsync(h->d_taps, taps.data(), sizeof(double) * taps.size(), cudaMemcpyHostToDevice, h->stream));
@@ -1634,53 +1510,18 @@ static int sweep_run_host_impl(lgdsp_handle* h, const lgdsp_sweep_params* p, con
     if (n_events == 0) return LGDSP_OK;
     if (!out) return fail(h, LGDSP_ERR_INVALID_ARG, "output pointer is NULL");
     const size_t sb = (size_t)sample_bytes;
-    const int64_t chunk = n_events < 8192 ? n_events : 8192;
-    rc = ensure_staging(h, (size_t)chunk * n * sb, 0);
-    if (rc) return rc;
-    if (baseline) {
-        rc = ensure_aux(h, (size_t)2 * chunk * sizeof(double));
-        if (rc) return rc;
-    }
-    const size_t esz = D.out_f64 ? sizeof(double) : sizeof(float);
-    const size_t ob = (size_t)2 * chunk * (n_variants * esz + 4 * sizeof(double));
-    if (ob > h->sweep_out_cap) {
-        cudaFree(h->d_sweep_out); h->d_sweep_out = nullptr; h->sweep_out_cap = 0;
-        CK(cudaMalloc(&h->d_sweep_out, ob));
-        h->sweep_out_cap = ob;
-    }
+    const size_t ow = (size_t)n_variants * (D.out_f64 ? sizeof(double) : sizeof(float)), aw = 4 * sizeof(double);
     const long long cap = (long long)h->sm_count * h->sweep_bps;
-    char* base = reinterpret_cast<char*>(h->d_sweep_out);
-    const unsigned char* src = static_cast<const unsigned char*>(wf);
-    const size_t out_bytes = (size_t)chunk * n_variants * esz;   // per buffer; the aux buffers follow the two output buffers
-    int c = 0;
-    for (int64_t e0 = 0; e0 < n_events; e0 += chunk, ++c) {
-        const int b = c & 1;
-        const int64_t ne = (n_events - e0) < chunk ? (n_events - e0) : chunk;
-        if (c >= 2) CK(cudaStreamWaitEvent(h->s_copy, h->ev_free[b], 0));
-        CK(cudaMemcpy2DAsync(h->d_in[b], (size_t)n * sb, src + (size_t)e0 * ld_samples * sb, (size_t)ld_samples * sb, (size_t)n * sb,
-                             (size_t)ne, cudaMemcpyHostToDevice, h->s_copy));
-        double* d_bl = nullptr;
-        if (baseline) {
-            d_bl = h->d_aux + (size_t)b * chunk;
-            CK(cudaMemcpyAsync(d_bl, baseline + e0, (size_t)ne * sizeof(double), cudaMemcpyHostToDevice, h->s_copy));
-        }
-        CK(cudaEventRecord(h->ev_ready[b], h->s_copy));
-        CK(cudaStreamWaitEvent(h->stream, h->ev_ready[b], 0));
-        void* d_o = base + (size_t)b * out_bytes;
-        double* d_a = aux ? reinterpret_cast<double*>(base + 2 * out_bytes) + (size_t)b * chunk * 4 : nullptr;
-        const int grid = (int)(ne < cap ? ne : cap);
-        if (sweep_launch(D, p->sig_dni.A, h->d_in[b], sample_bytes, ne, n, d_bl, d_o, d_a, grid, h->sm_count, h->stream) < 0)
-            return fail(h, LGDSP_ERR_UNSUPPORTED, "LGDSP_SWEEP_PATH=warp: this variant set / sample type runs on the one-CTA-per-waveform kernel");
-        CK(cudaGetLastError());
-        h->launches += 1;
-        CK(cudaEventRecord(h->ev_free[b], h->stream));
-        CK(cudaMemcpyAsync(reinterpret_cast<char*>(out) + (size_t)e0 * n_variants * esz, d_o, (size_t)ne * n_variants * esz,
-                           cudaMemcpyDeviceToHost, h->stream));
-        if (aux) CK(cudaMemcpyAsync(aux + e0 * 4, d_a, (size_t)ne * 4 * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
-    }
-    CK(cudaStreamSynchronize(h->s_copy));
-    CK(cudaStreamSynchronize(h->stream));
-    return LGDSP_OK;
+    return run_chunked(h, n_events, 8192, {host_array(wf, (size_t)ld_samples * sb, (size_t)n * sb), host_array(baseline, sizeof(double), sizeof(double))},
+                       {host_array(out, ow, ow), host_array(aux, aw, aw)}, [&](int64_t ne, void* const* d) {
+                           const int grid = (int)(ne < cap ? ne : cap);
+                           if (sweep_launch(D, p->sig_dni.A, d[0], sample_bytes, ne, n, static_cast<const double*>(d[1]), d[2],
+                                            static_cast<double*>(d[3]), grid, h->sm_count, h->stream) < 0)
+                               return fail(h, LGDSP_ERR_UNSUPPORTED, "LGDSP_SWEEP_PATH=warp: this variant set / sample type runs on the one-CTA-per-waveform kernel");
+                           CK(cudaGetLastError());
+                           h->launches += 1;
+                           return (int)LGDSP_OK;
+                       });
 }
 
 int lgdsp_sweep_run_device(lgdsp_handle* h, const lgdsp_sweep_params* p, const uint16_t* d_wf, int64_t n_events,
@@ -1788,19 +1629,28 @@ static int sipm_prepare(lgdsp_handle* h, const lgdsp_sipm_params* p, SipmDev& D,
     return LGDSP_OK;
 }
 
-int lgdsp_sipm_run_device(lgdsp_handle* h, const lgdsp_sipm_params* p, const void* d_wf, int64_t n_events, int64_t ld_samples,
-                          double* d_rows, double* d_trig)
+// sipm_prepare plus the checks lgdsp_sipm_run and _run_device share (nothing to do when n_events is 0)
+static int sipm_check(lgdsp_handle* h, const lgdsp_sipm_params* p, const void* wf, int64_t n_events, int64_t ld_samples,
+                      const double* rows, const double* trig, SipmDev& D, int& bps)
 {
     if (!h) return LGDSP_ERR_INVALID_ARG;
     CK(cudaSetDevice(h->device));
-    SipmDev D;
-    int bps = 0;
     int rc = sipm_prepare(h, p, D, bps);
     if (rc) return rc;
     if (n_events < 0) return fail(h, LGDSP_ERR_INVALID_ARG, "n_events < 0");
     if (n_events == 0) return LGDSP_OK;
-    if (!d_wf || !d_rows || !d_trig) return fail(h, LGDSP_ERR_INVALID_ARG, "NULL pointer");
+    if (!wf || !rows || !trig) return fail(h, LGDSP_ERR_INVALID_ARG, "NULL pointer");
     if (ld_samples < D.n) return fail(h, LGDSP_ERR_INVALID_ARG, "ld_samples (%lld) < n_samples (%d)", (long long)ld_samples, D.n);
+    return LGDSP_OK;
+}
+
+int lgdsp_sipm_run_device(lgdsp_handle* h, const lgdsp_sipm_params* p, const void* d_wf, int64_t n_events, int64_t ld_samples,
+                          double* d_rows, double* d_trig)
+{
+    SipmDev D;
+    int bps = 0;
+    int rc = sipm_check(h, p, d_wf, n_events, ld_samples, d_rows, d_trig, D, bps);
+    if (rc || n_events == 0) return rc;
     const long long cap = (long long)h->sm_count * bps;
     const int grid = (int)(n_events < cap ? n_events : cap);
     CK(cudaEventRecord(h->ev0, h->stream));
@@ -1815,47 +1665,21 @@ int lgdsp_sipm_run_device(lgdsp_handle* h, const lgdsp_sipm_params* p, const voi
 int lgdsp_sipm_run(lgdsp_handle* h, const lgdsp_sipm_params* p, const void* wf, int64_t n_events, int64_t ld_samples, double* rows,
                    double* trig)
 {
-    if (!h) return LGDSP_ERR_INVALID_ARG;
-    CK(cudaSetDevice(h->device));
     SipmDev D;
     int bps = 0;
-    int rc = sipm_prepare(h, p, D, bps);
-    if (rc) return rc;
-    if (n_events < 0) return fail(h, LGDSP_ERR_INVALID_ARG, "n_events < 0");
-    if (n_events == 0) return LGDSP_OK;
-    if (!wf || !rows || !trig) return fail(h, LGDSP_ERR_INVALID_ARG, "NULL pointer");
-    if (ld_samples < D.n) return fail(h, LGDSP_ERR_INVALID_ARG, "ld_samples (%lld) < n_samples (%d)", (long long)ld_samples, D.n);
+    int rc = sipm_check(h, p, wf, n_events, ld_samples, rows, trig, D, bps);
+    if (rc || n_events == 0) return rc;
     const size_t sb = (size_t)D.kind;   // bytes per sample
-    const size_t per_trig = (size_t)LGDSP_SIPM_NLIST * LGDSP_SIPM_NFIELD * D.cap;
-    // double-buffered: the H2D copy of chunk k+1 (copy stream) overlaps the kernel and the D2H copies of chunk k
-    const int64_t chunk = n_events < 8192 ? n_events : 8192;
-    const size_t out_per = LGDSP_SIPM_NCOL + per_trig;
-    rc = ensure_staging(h, (size_t)chunk * D.n * sb, (size_t)2 * chunk * out_per * sizeof(double));
-    if (rc) return rc;
+    const size_t rw = LGDSP_SIPM_NCOL * sizeof(double), tw = (size_t)LGDSP_SIPM_NLIST * LGDSP_SIPM_NFIELD * D.cap * sizeof(double);
     const long long gcap = (long long)h->sm_count * bps;
-    const unsigned char* src = static_cast<const unsigned char*>(wf);
-    int c = 0;
-    for (int64_t e0 = 0; e0 < n_events; e0 += chunk, ++c) {
-        const int b = c & 1;
-        const int64_t ne = (n_events - e0) < chunk ? (n_events - e0) : chunk;
-        if (c >= 2) CK(cudaStreamWaitEvent(h->s_copy, h->ev_free[b], 0));
-        CK(cudaMemcpy2DAsync(h->d_in[b], (size_t)D.n * sb, src + (size_t)e0 * ld_samples * sb, (size_t)ld_samples * sb, (size_t)D.n * sb,
-                             (size_t)ne, cudaMemcpyHostToDevice, h->s_copy));
-        CK(cudaEventRecord(h->ev_ready[b], h->s_copy));
-        CK(cudaStreamWaitEvent(h->stream, h->ev_ready[b], 0));
-        double* d_rows = h->d_rows + (size_t)b * chunk * out_per;
-        double* d_trig = d_rows + (size_t)chunk * LGDSP_SIPM_NCOL;
-        const int grid = (int)(ne < gcap ? ne : gcap);
-        sipm_launch(D, h->d_in[b], ne, D.n, d_rows, d_trig, grid, h->stream);
-        CK(cudaGetLastError());
-        h->launches += 1;
-        CK(cudaEventRecord(h->ev_free[b], h->stream));
-        CK(cudaMemcpyAsync(rows + e0 * LGDSP_SIPM_NCOL, d_rows, (size_t)ne * LGDSP_SIPM_NCOL * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
-        CK(cudaMemcpyAsync(trig + (size_t)e0 * per_trig, d_trig, (size_t)ne * per_trig * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
-    }
-    CK(cudaStreamSynchronize(h->s_copy));
-    CK(cudaStreamSynchronize(h->stream));
-    return LGDSP_OK;
+    return run_chunked(h, n_events, 8192, {host_array(wf, (size_t)ld_samples * sb, (size_t)D.n * sb)}, {host_array(rows, rw, rw), host_array(trig, tw, tw)},
+                       [&](int64_t ne, void* const* d) {
+                           const int grid = (int)(ne < gcap ? ne : gcap);
+                           sipm_launch(D, d[0], ne, D.n, static_cast<double*>(d[1]), static_cast<double*>(d[2]), grid, h->stream);
+                           CK(cudaGetLastError());
+                           h->launches += 1;
+                           return (int)LGDSP_OK;
+                       });
 }
 
 int lgdsp_sipm_list_pointers_device(lgdsp_handle* h, const double* d_rows, int64_t n_events, int32_t list, int32_t max_triggers,
@@ -1898,15 +1722,18 @@ static int prim_run(lgdsp_handle* h, int mode, const double* y, int n, double a,
     CK(cudaSetDevice(h->device));
     if (n < 0 || n > 65536) return fail(h, LGDSP_ERR_UNSUPPORTED, "n = %d: single-trace primitives take 0 .. 65536 samples", n);
     if (n > 0 && !y) return fail(h, LGDSP_ERR_INVALID_ARG, "trace pointer is NULL");
-    int rc = ensure_staging(h, (size_t)(n > 0 ? n : 1) * sizeof(double), (size_t)(n_out + 2) * sizeof(double));
+    // d_prim: the trace, then n_out results and the count
+    const size_t n_in = n > 0 ? (size_t)n : 1;
+    int rc = grow(h, &h->d_prim, &h->prim_cap, (n_in + n_out + 2) * sizeof(double));
     if (rc) return rc;
-    if (n > 0) CK(cudaMemcpyAsync(h->d_in[0], y, (size_t)n * sizeof(double), cudaMemcpyHostToDevice, h->stream));
-    int* d_cnt = reinterpret_cast<int*>(h->d_rows + n_out);
+    double* d_out = h->d_prim + n_in;
+    int* d_cnt = reinterpret_cast<int*>(d_out + n_out);
+    if (n > 0) CK(cudaMemcpyAsync(h->d_prim, y, (size_t)n * sizeof(double), cudaMemcpyHostToDevice, h->stream));
     CK(cudaMemsetAsync(d_cnt, 0, sizeof(int), h->stream));
-    sipm_prim_launch(mode, reinterpret_cast<const double*>(h->d_in[0]), n, a, b, t0, dt, min_n, max_n, cap, h->d_rows, d_cnt, h->stream);
+    sipm_prim_launch(mode, h->d_prim, n, a, b, t0, dt, min_n, max_n, cap, d_out, d_cnt, h->stream);
     CK(cudaGetLastError());
     h->launches += 1;
-    CK(cudaMemcpyAsync(out_host, h->d_rows, (size_t)n_out * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaMemcpyAsync(out_host, d_out, (size_t)n_out * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
     int cnt = 0;
     CK(cudaMemcpyAsync(&cnt, d_cnt, sizeof(int), cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
@@ -1961,18 +1788,27 @@ static int mi_prepare(lgdsp_handle* h, const lgdsp_multi_intersect_params* p, Mi
     return LGDSP_OK;
 }
 
-int lgdsp_multi_intersect_run_device(lgdsp_handle* h, const lgdsp_multi_intersect_params* p, const double* d_y, int64_t n_events,
-                                     int64_t ld_samples, double* d_x, int32_t* d_flags)
+// mi_prepare plus the checks lgdsp_multi_intersect_run and _run_device share (nothing to do when n_events is 0)
+static int mi_check(lgdsp_handle* h, const lgdsp_multi_intersect_params* p, const double* y, int64_t n_events, int64_t ld_samples,
+                    const double* x, const int32_t* flags, MiDev& D)
 {
     if (!h) return LGDSP_ERR_INVALID_ARG;
     CK(cudaSetDevice(h->device));
-    MiDev D;
     int rc = mi_prepare(h, p, D);
     if (rc) return rc;
     if (n_events < 0) return fail(h, LGDSP_ERR_INVALID_ARG, "n_events < 0");
     if (n_events == 0) return LGDSP_OK;
-    if (!d_y || !d_x || !d_flags) return fail(h, LGDSP_ERR_INVALID_ARG, "NULL pointer");
+    if (!y || !x || !flags) return fail(h, LGDSP_ERR_INVALID_ARG, "NULL pointer");
     if (ld_samples < D.len) return fail(h, LGDSP_ERR_INVALID_ARG, "ld_samples < n_samples");
+    return LGDSP_OK;
+}
+
+int lgdsp_multi_intersect_run_device(lgdsp_handle* h, const lgdsp_multi_intersect_params* p, const double* d_y, int64_t n_events,
+                                     int64_t ld_samples, double* d_x, int32_t* d_flags)
+{
+    MiDev D;
+    int rc = mi_check(h, p, d_y, n_events, ld_samples, d_x, d_flags, D);
+    if (rc || n_events == 0) return rc;
     CK(cudaEventRecord(h->ev0, h->stream));
     multi_intersect_launch(D, d_y, n_events, ld_samples, d_x, d_flags, h->stream);
     CK(cudaGetLastError());
@@ -1985,33 +1821,18 @@ int lgdsp_multi_intersect_run_device(lgdsp_handle* h, const lgdsp_multi_intersec
 int lgdsp_multi_intersect_run(lgdsp_handle* h, const lgdsp_multi_intersect_params* p, const double* y, int64_t n_events,
                               int64_t ld_samples, double* x, int32_t* flags)
 {
-    if (!h) return LGDSP_ERR_INVALID_ARG;
-    CK(cudaSetDevice(h->device));
     MiDev D;
-    int rc = mi_prepare(h, p, D);
-    if (rc) return rc;
-    if (n_events < 0) return fail(h, LGDSP_ERR_INVALID_ARG, "n_events < 0");
-    if (n_events == 0) return LGDSP_OK;
-    if (!y || !x || !flags) return fail(h, LGDSP_ERR_INVALID_ARG, "NULL pointer");
-    if (ld_samples < D.len) return fail(h, LGDSP_ERR_INVALID_ARG, "ld_samples < n_samples");
-    const int64_t chunk = n_events < 4096 ? n_events : 4096;
-    const size_t out_per = (size_t)D.n_thr * sizeof(double) + sizeof(int32_t);
-    rc = ensure_staging(h, (size_t)chunk * D.len * sizeof(double), (size_t)chunk * out_per + 16);
-    if (rc) return rc;
-    double* d_x = h->d_rows;
-    int* d_f = reinterpret_cast<int*>(h->d_rows + (size_t)chunk * D.n_thr);
-    for (int64_t e0 = 0; e0 < n_events; e0 += chunk) {
-        const int64_t ne = (n_events - e0) < chunk ? (n_events - e0) : chunk;
-        CK(cudaMemcpy2DAsync(h->d_in[0], (size_t)D.len * sizeof(double), y + e0 * ld_samples, (size_t)ld_samples * sizeof(double),
-                             (size_t)D.len * sizeof(double), (size_t)ne, cudaMemcpyHostToDevice, h->stream));
-        multi_intersect_launch(D, reinterpret_cast<const double*>(h->d_in[0]), ne, D.len, d_x, d_f, h->stream);
-        CK(cudaGetLastError());
-        h->launches += 1;
-        CK(cudaMemcpyAsync(x + e0 * D.n_thr, d_x, (size_t)ne * D.n_thr * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
-        CK(cudaMemcpyAsync(flags + e0, d_f, (size_t)ne * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
-        CK(cudaStreamSynchronize(h->stream));
-    }
-    return LGDSP_OK;
+    int rc = mi_check(h, p, y, n_events, ld_samples, x, flags, D);
+    if (rc || n_events == 0) return rc;
+    const size_t xw = (size_t)D.n_thr * sizeof(double);
+    return run_chunked(h, n_events, 4096, {host_array(y, (size_t)ld_samples * sizeof(double), (size_t)D.len * sizeof(double))},
+                       {host_array(x, xw, xw), host_array(flags, sizeof(int32_t), sizeof(int32_t))}, [&](int64_t ne, void* const* d) {
+                           multi_intersect_launch(D, static_cast<const double*>(d[0]), ne, D.len, static_cast<double*>(d[1]),
+                                                  static_cast<int*>(d[2]), h->stream);
+                           CK(cudaGetLastError());
+                           h->launches += 1;
+                           return (int)LGDSP_OK;
+                       });
 }
 
 // ---------------------------------------------------------------------------------------------------
