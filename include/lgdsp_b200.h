@@ -530,14 +530,6 @@ int lgdsp_icpc_profile_device(lgdsp_handle* h, const uint16_t* d_wf, int64_t n_e
  * handle's stream (valid after lgdsp_synchronize) ---- */
 double lgdsp_last_kernel_ms(const lgdsp_handle* h);
 
-/* ---- debug: barrier-to-barrier cycle counters of the fused kernel (summed over CTAs) of the last
- * lgdsp_icpc_run_device call: out8[0] TMA wait, out8[1..6] phases P1, P2, P3, P4a, P4b, P5 (lgdsp_icpc.cu).
- * enable != 0 turns the counters on for subsequent calls (small overhead), 0 turns them off. ---- */
-int lgdsp_debug_phase_cycles(lgdsp_handle* h, int enable, double* out8);
-/* finer (section, warp) cycle sums, out256[section*8 + warp]; all zero unless the library was built with
- * -DLGDSP_PROFILE_SECTIONS (python legenddsp.jl_b200/build.py --profile) */
-int lgdsp_debug_section_cycles(lgdsp_handle* h, double* out256);
-
 #ifdef __cplusplus
 }
 #endif

@@ -89,8 +89,6 @@ def load_library():
                                              vp, vp]
     L.lgdsp_synth_generate_device.argtypes = [vp, C.POINTER(_abi.SynthParams), i64, i64, i64, vp]
     L.lgdsp_synth_generate_host.argtypes = [C.POINTER(_abi.SynthParams), i64, i64, i64, vp]
-    L.lgdsp_debug_phase_cycles.argtypes = [vp, C.c_int, _dp]
-    L.lgdsp_debug_section_cycles.argtypes = [vp, _dp]
     _lib = L
     return L
 
@@ -106,7 +104,7 @@ EXPORTED_SYMBOLS = (
     "lgdsp_sipm_list_pointers_device", "lgdsp_sipm_list_gather_device", "lgdsp_thresholdstats", "lgdsp_intersect_maximum", "lgdsp_multi_intersect_run", "lgdsp_multi_intersect_run_device", "lgdsp_icpc_compressed_run", "lgdsp_icpc_compressed_run_device",
     "lgdsp_trap_sweep_run", "lgdsp_trap_sweep_run_device", "lgdsp_sweep_run", "lgdsp_sweep_run_device",
     "lgdsp_sweep_run_ext", "lgdsp_sweep_run_ext_device",
-    "lgdsp_synth_generate_device", "lgdsp_synth_generate_host", "lgdsp_last_kernel_ms", "lgdsp_debug_phase_cycles", "lgdsp_debug_section_cycles",
+    "lgdsp_synth_generate_device", "lgdsp_synth_generate_host", "lgdsp_last_kernel_ms",
 )
 
 
@@ -164,19 +162,6 @@ class Handle:
 
     def last_kernel_ms(self):
         return float(self._lib.lgdsp_last_kernel_ms(self._h))
-
-    def phase_cycles(self, enable=True):
-        """debug: (cycles of the last device run per phase, summed over CTAs: TMA wait, P1, P2, P3, P4a, P4b, P5, -);
-        `enable` switches the counters on/off for the following runs"""
-        out = (C.c_double * 8)()
-        self._check(self._lib.lgdsp_debug_phase_cycles(self._h, 1 if enable else 0, out))
-        return list(out)
-
-    def section_cycles(self):
-        """debug (profile build only): cycles per (section, warp) of the last device run as a 32 x 8 nested list"""
-        out = (C.c_double * 256)()
-        self._check(self._lib.lgdsp_debug_section_cycles(self._h, out))
-        return [[out[s * 8 + w] for w in range(8)] for s in range(32)]
 
     # ---- dsp_icpc ----
     def icpc_set_params(self, params):

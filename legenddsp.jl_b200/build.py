@@ -21,14 +21,12 @@ def needs_build():
     return any(os.path.getmtime(d) > t for d in deps)
 
 
-def build_library(force=False, verbose=False, profile=False):
-    """profile=True adds -DLGDSP_PROFILE_SECTIONS (per-section cycle counters, tools/phase_cycles.py); not for benchmarks"""
+def build_library(force=False, verbose=False):
     if not force and not needs_build():
         return OUT
     nvcc = shutil.which("nvcc") or "/usr/local/cuda/bin/nvcc"
-    extra = os.environ.get("LGDSP_NVCC_EXTRA", "").split()   # experiment knobs (-D...), never set for a release build
-    cmd = ([nvcc] + NVCC_FLAGS + extra + (["-Xptxas", "-v"] if verbose else []) + (["-DLGDSP_PROFILE_SECTIONS"] if profile else [])
-           + ["-o", OUT] + list(SOURCES))
+    extra = os.environ.get("LGDSP_NVCC_EXTRA", "").split()   # extra flags of experiment builds, never set for a release build
+    cmd = ([nvcc] + NVCC_FLAGS + extra + (["-Xptxas", "-v"] if verbose else []) + ["-o", OUT] + list(SOURCES))
     r = subprocess.run(cmd, cwd=CSRC, capture_output=True, text=True)
     if r.returncode != 0:
         sys.stderr.write(r.stdout + r.stderr)
@@ -39,4 +37,4 @@ def build_library(force=False, verbose=False, profile=False):
 
 
 if __name__ == "__main__":
-    print(build_library(force="--force" in sys.argv or "--profile" in sys.argv, verbose=True, profile="--profile" in sys.argv))
+    print(build_library(force="--force" in sys.argv, verbose=True))

@@ -29,9 +29,6 @@ struct lgdsp_handle {
     double* d_cusp_g = nullptr;    // [LGDSP_MAX_FIR+1]
     double* d_zac_g = nullptr;     // [LGDSP_MAX_FIR+1]
     double* d_sweep_dniA = nullptr;
-    unsigned long long* d_phase = nullptr;   // [grid][8] phase cycle counters (debug)
-    int phase_grid = 0;
-    bool phase_on = false;
     SweepVar* d_vars = nullptr;
     size_t vars_cap = 0;
     double* d_taps = nullptr;      // differenced FIR / SG taps of the sweep variants
@@ -86,7 +83,6 @@ struct lgdsp_handle {
     cudaStream_t s_split[LGDSP_SPLIT_MAX_STREAMS] = {};
     cudaStream_t s_cz[LGDSP_SPLIT_MAX_STREAMS] = {};   // CUSP/ZAC kernel next to the extract kernel
     cudaEvent_t ev_pre[LGDSP_SPLIT_MAX_STREAMS] = {}, ev_cz[LGDSP_SPLIT_MAX_STREAMS] = {};
-    int split_par = 1;             // 1: CUSP/ZAC kernel on its own stream
     cudaEvent_t ev_fork = nullptr, ev_join[LGDSP_SPLIT_MAX_STREAMS] = {nullptr, nullptr, nullptr, nullptr};
 };
 
@@ -192,13 +188,6 @@ int lgdsp_create(int device, void* stream, lgdsp_handle** out)
     if (const char* env = getenv("LGDSP_ICPC_PATH")) h->icpc_path = (strcmp(env, "fused") == 0) ? 0 : 1;
     if (const char* env = getenv("LGDSP_SPLIT_BATCH")) h->split_batch = atoll(env);
     if (const char* env = getenv("LGDSP_SPLIT_STREAMS")) h->split_streams = atoi(env);
-    if (const char* env = getenv("LGDSP_SPLIT_PAR")) h->split_par = atoi(env) != 0;
-    if (const char* env = getenv("LGDSP_SPLIT_BPS")) {   // experiment knob: resident blocks per SM of {prefix, extract, cuspzac}, e.g. "2,3,1"
-        int v[3] = {0, 0, 0};
-        if (sscanf(env, "%d,%d,%d", &v[0], &v[1], &v[2]) == 3)
-            for (int k = 0; k < 3; ++k)
-                if (v[k] >= 1 && v[k] < h->split_bps[k]) h->split_bps[k] = v[k];
-    }
     if (h->split_streams < 1) h->split_streams = 1;
     if (h->split_streams > LGDSP_SPLIT_MAX_STREAMS) h->split_streams = LGDSP_SPLIT_MAX_STREAMS;
     *out = h;
@@ -219,7 +208,6 @@ void lgdsp_destroy(lgdsp_handle* h)
     }
     if (h->ev_fork) cudaEventDestroy(h->ev_fork);
     cudaFree(h->d_tt); cudaFree(h->d_saux); cudaFree(h->d_scz);
-    cudaFree(h->d_phase);
     cudaFree(h->d_dniA); cudaFree(h->d_cusp_g); cudaFree(h->d_zac_g); cudaFree(h->d_sweep_dniA); cudaFree(h->d_vars); cudaFree(h->d_taps);
     cudaFree(h->d_win); cudaFree(h->d_prim);
     cudaFree(h->d_dniA_w); cudaFree(h->d_cusp_g_w); cudaFree(h->d_zac_g_w);
@@ -542,7 +530,7 @@ static int grow(lgdsp_handle* h, T** p, size_t* cap, size_t bytes)
 static int icpc_dispatch(lgdsp_handle* h, const IcpcDev& D, const void* d_wf, int sample_bytes, int64_t ne, int64_t ld,
                          const double* d_bl, int64_t bl_stride, double bl_div, double* d_rows)
 {
-    if (h->icpc_path == 0 || D.phase_cycles != nullptr) {
+    if (h->icpc_path == 0) {
         const long long cap = (long long)h->sm_count * h->icpc_bps;
         const int grid = (int)(ne < cap ? ne : cap);
         icpc_launch(D, d_wf, sample_bytes, ne, ld, d_bl, bl_stride, bl_div, d_rows, grid, h->stream);
@@ -581,7 +569,7 @@ static int icpc_dispatch(lgdsp_handle* h, const IcpcDev& D, const void* d_wf, in
                                 h->d_saux + (size_t)si * (size_t)B * (size_t)icpc_split_aux_doubles(),
                                 h->d_scz + (size_t)si * (size_t)B * (size_t)icpc_split_cz_doubles(),
                                 h->split_bps, h->sm_count, st,
-                                h->split_par ? h->s_cz[si] : nullptr, h->ev_pre[si], h->ev_cz[si], nullptr);
+                                h->s_cz[si], h->ev_pre[si], h->ev_cz[si], nullptr);
         CK(cudaGetLastError());
         h->launches += cz ? (D.direct ? 3 : 4) : 2;
     }
@@ -625,18 +613,8 @@ static int icpc_run_device_impl(lgdsp_handle* h, const lgdsp_icpc_params* p, con
     if (rc) return rc;
     if (n_events == 0) return LGDSP_OK;  // empty input -> empty table
     if (!d_out_rows) return fail(h, LGDSP_ERR_INVALID_ARG, "output pointer is NULL");
-    const long long cap = (long long)h->sm_count * h->icpc_bps;
-    const int grid = (int)(n_events < cap ? n_events : cap);
-    IcpcDev D = h->icpc;
-    D.phase_cycles = nullptr;
-    if (h->phase_on) {
-        if (!h->d_phase) CK(cudaMalloc(&h->d_phase, sizeof(unsigned long long) * (8 * (size_t)cap + 32 * 8)));
-        CK(cudaMemsetAsync(h->d_phase, 0, sizeof(unsigned long long) * (8 * (size_t)cap + 32 * 8), h->stream));
-        D.phase_cycles = h->d_phase;
-        h->phase_grid = grid;
-    }
     CK(cudaEventRecord(h->ev0, h->stream));
-    rc = icpc_dispatch(h, D, d_wf, sample_bytes, n_events, ld_samples, d_baseline, 1, 1.0, d_out_rows);
+    rc = icpc_dispatch(h, h->icpc, d_wf, sample_bytes, n_events, ld_samples, d_baseline, 1, 1.0, d_out_rows);
     if (rc) return rc;
     CK(cudaEventRecord(h->ev1, h->stream));
     h->timed = true;
@@ -657,8 +635,7 @@ int lgdsp_icpc_profile_device(lgdsp_handle* h, const uint16_t* d_wf, int64_t n_e
     const int64_t keepB = h->split_batch;
     const int keepS = h->split_streams;
     h->split_batch = n_events; h->split_streams = 1;
-    IcpcDev D = h->icpc;
-    D.phase_cycles = nullptr;
+    const IcpcDev& D = h->icpc;
     rc = icpc_dispatch(h, D, d_wf, 2, n_events, ld_samples, nullptr, 1, 1.0, d_out_rows);   // sizes the scratch, warms up
     h->split_batch = keepB; h->split_streams = keepS;
     if (rc) return rc;
@@ -1298,40 +1275,6 @@ int lgdsp_icpc_compressed_run_encoded(lgdsp_handle* h, const lgdsp_icpc_params* 
                     off_wdw ? is_pinned(off_wdw) : false};
     return compressed_run_host_impl(h, p_pre, p_wdw, nullptr, pre_sample_bytes, 0, nullptr, wdw_sample_bytes, 0, &ep, &ew, presum_rate,
                                     aux_windows, n_events, rows_pre, rows_wdw, stats);
-}
-
-// debug: per-phase cycle counters of the last lgdsp_icpc_run_device call (sum over CTAs; index 0: TMA wait,
-// 1..6: P1, P2, P3, P4a, P4b, P5, see lgdsp_icpc.cu).  enable != 0 switches the counters on for later calls.
-int lgdsp_debug_phase_cycles(lgdsp_handle* h, int enable, double* out8)
-{
-    if (!h) return LGDSP_ERR_INVALID_ARG;
-    CK(cudaSetDevice(h->device));
-    if (out8) {
-        for (int i = 0; i < 8; ++i) out8[i] = 0.0;
-        if (h->d_phase && h->phase_grid > 0) {
-            CK(cudaStreamSynchronize(h->stream));
-            std::vector<unsigned long long> v((size_t)h->phase_grid * 8);
-            CK(cudaMemcpy(v.data(), h->d_phase, v.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
-            for (int b = 0; b < h->phase_grid; ++b)
-                for (int i = 0; i < 8; ++i) out8[i] += (double)v[(size_t)b * 8 + i];
-        }
-    }
-    h->phase_on = enable != 0;
-    return LGDSP_OK;
-}
-
-// debug (library built with -DLGDSP_PROFILE_SECTIONS only): cycles per (section, warp) of the last run, out[32*8]
-int lgdsp_debug_section_cycles(lgdsp_handle* h, double* out256)
-{
-    if (!h || !out256) return LGDSP_ERR_INVALID_ARG;
-    CK(cudaSetDevice(h->device));
-    for (int i = 0; i < 256; ++i) out256[i] = 0.0;
-    if (!h->d_phase || h->phase_grid <= 0) return LGDSP_OK;
-    CK(cudaStreamSynchronize(h->stream));
-    unsigned long long v[256];
-    CK(cudaMemcpy(v, h->d_phase + (size_t)h->phase_grid * 8, sizeof(v), cudaMemcpyDeviceToHost));
-    for (int i = 0; i < 256; ++i) out256[i] = (double)v[i];
-    return LGDSP_OK;
 }
 
 // ---------------------------------------------------------------------------------------------------

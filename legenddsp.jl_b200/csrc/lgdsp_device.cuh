@@ -77,7 +77,6 @@ struct IcpcDev {
     const double* dni_A;    // [2][LGDSP_MAX_DNI*4]: int_dni, sig_dni fit matrices
     const double* cusp_g;   // differenced CUSP taps on TT, cusp_L+1 values
     const double* zac_g;    // differenced ZAC taps on TT, zac_L+1 values
-    unsigned long long* phase_cycles;   // optional [grid][8] per-phase cycle counters (NULL: off), see lgdsp_debug_phase_cycles
 };
 
 

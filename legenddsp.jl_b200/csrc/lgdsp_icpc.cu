@@ -523,11 +523,7 @@ __device__ __forceinline__ double* cz_tab(double* tabA, double* tabB, int idx)
 // CONTIG: tables 8..15 follow tables 0..7 in memory (the split pipeline's layout): no per-access choice of the half
 template <int PAR_OFF, bool CONTIG = false>
 __device__ __noinline__ void cz_scan(int ps, const double* TT, int n, int tid, double* tabA, double* tabB, double* red,
-                        double* pp0
-#ifdef LGDSP_PROFILE_SECTIONS
-                        , unsigned long long* sect_cnt, unsigned long long* sect_last
-#endif
-                        )
+                        double* pp0)
 {
     // SMEM copy of the descriptor, addressed through the dynamic shared memory base so that the loads are LDS
     // (a reference to the kernel parameter or a generic pointer would force generic loads)
@@ -612,13 +608,6 @@ __device__ __noinline__ void cz_scan(int ps, const double* TT, int n, int tid, d
     }
     if (lane == 31) { red[wid] = vpm; red[8 + wid] = vd1; red[16 + wid] = vd2; }
     if (lane == 0) red[24 + wid] = vpp;
-#ifdef LGDSP_PROFILE_SECTIONS
-    if (sect_cnt != nullptr && lane == 0) {   // section 25: cz_scan up to its barrier
-        const unsigned long long now_ = (unsigned long long)clock64();
-        atomicAdd(sect_cnt, now_ - *sect_last);
-        *sect_last = now_;
-    }
-#endif
     __syncthreads();
     double gpm = 0, gd1 = 0, gd2 = 0, gpp = 0;   // carries of the neighbouring warps
     for (int w = 0; w < wid; ++w) { gpm = fma(Z.rho_warp, gpm, red[w]); gd1 += red[8 + w]; gd2 += red[16 + w]; }
@@ -813,10 +802,7 @@ __device__ __forceinline__ void cz_out_each(const CzDev& Z, const double* TT, in
 // the trace ends take the same values as in cz_out_each (for interior chunks the clamp is void), and every float64
 // operation keeps its operands and order.  All 32 lanes must call it (warp-synchronous); lanes without a candidate
 // (has == false, chunk 0) help to stage and never call f.  nact: candidates of the warp (lanes 0..nact-1).
-#ifndef LGDSP_CZ_STAGE
-#define LGDSP_CZ_STAGE 4
-#endif
-constexpr int CZ_STAGE = LGDSP_CZ_STAGE;   // steps per staged piece (a power of two dividing CH - 1 = 32)
+constexpr int CZ_STAGE = 4;   // steps per staged piece (a power of two dividing CH - 1 = 32)
 static_assert(CZ_STAGE >= 1 && CZ_STAGE <= 32 && (CZ_STAGE & (CZ_STAGE - 1)) == 0 && (CH - 1) % CZ_STAGE == 0, "stage piece");
 constexpr int CZ_SLAB = 2 * 4 * CZ_STAGE * 32;   // doubles of one warp's slab
 template <typename F>
@@ -1062,31 +1048,12 @@ icpc_kernel(const __grid_constant__ IcpcDev P, const SAMPLE* __restrict__ wf, lo
     const bool cz_structured = cz_on && !P.direct;
     const int npass = cz_structured ? (P.cz_shared ? 1 : 2) : 0;
 
-    // optional phase timing (debug): thread 0 accumulates barrier-to-barrier cycles
-    unsigned long long* pc_acc = reinterpret_cast<unsigned long long*>(scr + 20);   // [9]: 8 counters + last clock (SMEM)
-    const bool pc_on = (P.phase_cycles != nullptr) && tid == 0;
-#define LGDSP_PHASE(i) do { if (pc_on) { const unsigned long long now_ = (unsigned long long)clock64(); pc_acc[i] += now_ - pc_acc[8]; pc_acc[8] = now_; } } while (0)
-    if (pc_on) {
-        for (int i = 0; i < 8; ++i) pc_acc[i] = 0ull;
-        pc_acc[8] = (unsigned long long)clock64();
-    }
-#ifdef LGDSP_PROFILE_SECTIONS
-    // per-(section, warp) cycle sums (debug build only): lane 0 of every warp, global atomics behind the phase counters
-    unsigned long long sect_last = (unsigned long long)clock64();
-#define SECT(i) do { if (P.phase_cycles != nullptr && lane == 0) { const unsigned long long now_ = (unsigned long long)clock64(); \
-        atomicAdd(&P.phase_cycles[(size_t)gridDim.x * 8 + (i) * 8 + wid], now_ - sect_last); sect_last = now_; } } while (0)
-#else
-#define SECT(i) do { } while (0)
-#endif
-
     for (; e < n_events; e += gridDim.x) {
         // ==========================================================================================
         // P1: raw samples
         // ==========================================================================================
         mbar_wait(bar, phase);
         phase ^= 1;
-        LGDSP_PHASE(0);   // wait for the TMA load
-        SECT(31);
         const SAMPLE* xp = xs + i0;
         uint32_t csum = 0, cq = 0, cmn = 0xFFFFFFFFu, cmx = 0;
 #pragma unroll 1
@@ -1097,7 +1064,6 @@ icpc_kernel(const __grid_constant__ IcpcDev P, const SAMPLE* __restrict__ wf, lo
             cmn = min(cmn, x);
             cmx = max(cmx, x);
         }
-        SECT(0);
         // baseline regression sums (exact integers), samples of the window strided over ALL threads (the window covers the
         // first chunks only: summed chunk-wise, three warps would do the whole job while the others wait at B1)
         {
@@ -1160,10 +1126,7 @@ icpc_kernel(const __grid_constant__ IcpcDev P, const SAMPLE* __restrict__ wf, lo
 #pragma unroll
         for (int q = 0; q < NMASK; ++q) masks[q * NWORDS + tid] = 0u;
         if (tid == 0) { ibuf[IB_QN] = 0; ibuf[IB_CZN] = 0; }
-        SECT(1);
         __syncthreads();   // ---- B1 ----
-        LGDSP_PHASE(1);
-        SECT(2);
 
         // exclusive prefixes of this thread's chunk
         uint32_t P_excl;
@@ -1239,7 +1202,6 @@ icpc_kernel(const __grid_constant__ IcpcDev P, const SAMPLE* __restrict__ wf, lo
 #pragma unroll
         for (int k = 0; k < 5; ++k) thr[k] = e_max * P.tx_frac[k];
 
-        SECT(3);
         // ==========================================================================================
         // P2: prefix sums of the pole-zero waveform; t10..t99 masks; tail log-regression
         // ==========================================================================================
@@ -1271,7 +1233,6 @@ icpc_kernel(const __grid_constant__ IcpcDev P, const SAMPLE* __restrict__ wf, lo
                 for (; k < cvalid; ++k) body(k);
                 if (tid == 0) TT[0] = 0.0;
             }
-            SECT(4);
             // Conservative bounds of y = w + km1*cumsum(w) on the chunk from the integer min/max of the raw samples:
             // cumsum(w)[i0+k] lies between S0 + (k+1)*wmin and S0 + (k+1)*wmax.
             const double wmin = (double)cmn - m, wmax = (double)cmx - m;
@@ -1329,7 +1290,6 @@ icpc_kernel(const __grid_constant__ IcpcDev P, const SAMPLE* __restrict__ wf, lo
             const double ya = wmax_d(cvalid > 0 ? fmax(fabs(ylo), fabs(yhi)) : 0.0);
             red_put(red, R_YMAX, wid, lane, ya);
         }
-        SECT(5);
         // tailstats: log-regression on the PRE-PZ waveform (src/tailstats.jl:22-72), samples strided over the block
         {
             double tl_S = 0, tl_SS = 0, tl_SX = 0;
@@ -1378,10 +1338,7 @@ icpc_kernel(const __grid_constant__ IcpcDev P, const SAMPLE* __restrict__ wf, lo
                 red[R_TLSX * NWARP + wid] = tl_SX; red[R_TLBAD * NWARP + wid] = anybad ? 1.0 : 0.0;
             }
         }
-        SECT(6);
         __syncthreads();   // ---- B2: TT and the t10..t99 masks are complete; xs is dead ----
-        LGDSP_PHASE(2);
-        SECT(7);
 
         // xs is free now: prefetch the next event (TMA, async proxy) -- unless the structured CUSP/ZAC pass borrows
         // xs for its prefix tables; then the prefetch is issued when the tables are dead
@@ -1422,7 +1379,6 @@ icpc_kernel(const __grid_constant__ IcpcDev P, const SAMPLE* __restrict__ wf, lo
                 ibuf[IB_PKFROM + lane] = pf;
             }
         }
-        SECT(8);
         // PZ tail statistics (signalstats on the tail window, src/dsp_icpc.jl:123)
         {
             double pz_S = 0, pz_SS = 0, pz_SX = 0;
@@ -1439,7 +1395,6 @@ icpc_kernel(const __grid_constant__ IcpcDev P, const SAMPLE* __restrict__ wf, lo
                 red[R_PZS * NWARP + wid] = pz_S; red[R_PZSS * NWARP + wid] = pz_SS; red[R_PZSX * NWARP + wid] = pz_SX;
             }
         }
-        SECT(9);
         // trapezoids whose minimum is needed as well: full traces
         if (G & LGDSP_GROUP_TRAPS) {
             double o4[4];
@@ -1450,7 +1405,6 @@ icpc_kernel(const __grid_constant__ IcpcDev P, const SAMPLE* __restrict__ wf, lo
                 red[R_E313 * NWARP + wid] = c; red[R_E313N * NWARP + wid] = d;
             }
         }
-        SECT(10);
         // coarse grid (outputs 33*tid and 33*(tid+1)) of the other trapezoids
         double c0a = 0, c0b = 0, cia = 0, cib = 0, c5a = -CUDART_INF, c5b = -CUDART_INF, cea = -CUDART_INF, ceb = -CUDART_INF;
         {
@@ -1473,7 +1427,6 @@ icpc_kernel(const __grid_constant__ IcpcDev P, const SAMPLE* __restrict__ wf, lo
                 red_put(red, R_CET, wid, lane, we);
             }
         }
-        SECT(11);
         // currents: sg[0] over the whole trace (chunked, sliding window in registers): trace maximum, windowed first
         // argmax, baseline-window sums; the chunk maximum is kept for the mask pass
         double sgcmax = -CUDART_INF;
@@ -1485,7 +1438,6 @@ icpc_kernel(const __grid_constant__ IcpcDev P, const SAMPLE* __restrict__ wf, lo
             double sg_S = 0, sg_SS = 0;
             // (a) whole trace, one chunk per thread: only the chunk maximum (uniform cost for every thread)
             if (want_intr) sg_chunk(TT, P.sg[0], i0, min(CH, nsg - i0), [&](int k, double s) { sgcmax = s > sgcmax ? s : sgcmax; });
-            SECT(12);
             // (b) windowed quantities, strided over the block (same operation order as the chunk pass: identical values):
             //     first argmax of sg[0..2] and of the plain derivative inside the current window, baseline-window sums of sg[0]
 #pragma unroll 1
@@ -1547,7 +1499,6 @@ icpc_kernel(const __grid_constant__ IcpcDev P, const SAMPLE* __restrict__ wf, lo
                     if (d > cmax[3]) { cmax[3] = d; carg[3] = j; }
                 }
             }
-            SECT(13);
             const double wsm = wmax_d(sgcmax);
             sg_S = wsum_d(sg_S); sg_SS = wsum_d(sg_SS);
 #pragma unroll
@@ -1561,18 +1512,9 @@ icpc_kernel(const __grid_constant__ IcpcDev P, const SAMPLE* __restrict__ wf, lo
                 }
             }
         }
-        SECT(14);
         // CUSP/ZAC prefix tables (first descriptor)
-#ifdef LGDSP_PROFILE_SECTIONS
-        if (cz_structured) cz_scan<SM_PAR>(npass == 2 ? 1 : 0, TT, n, tid, tabA, tabB, red + R_CZSCR * NWARP, scr + SC_PP0,
-                                   P.phase_cycles ? &P.phase_cycles[(size_t)gridDim.x * 8 + 25 * 8 + wid] : nullptr, &sect_last);
-#else
         if (cz_structured) cz_scan<SM_PAR>(npass == 2 ? 1 : 0, TT, n, tid, tabA, tabB, red + R_CZSCR * NWARP, scr + SC_PP0);
-#endif
-        SECT(15);
         __syncthreads();   // ---- B3 ----
-        LGDSP_PHASE(3);
-        SECT(16);
 
         // ==========================================================================================
         // P4a: decisions that need block-wide values; fine evaluation of the flagged intervals
@@ -1588,7 +1530,6 @@ icpc_kernel(const __grid_constant__ IcpcDev P, const SAMPLE* __restrict__ wf, lo
         // the 44 trap(rt,ft) outputs of the e_trap pick-off window
         if ((G & LGDSP_GROUP_TRAPS) && tid < P.sig_dni.n_w) stash[tid] = trap_at(TT, P.etrap, pk_from[0] + tid);
 
-        SECT(17);
         // ---- thresholds of the sg[0] masks (t50_current at half the trace maximum; pile-up at n sigma of the baseline
         //      window, sigma exactly as signalstats computes it) ----
         double pile_thr = 0.0, cur_thr = 0.0;
@@ -1690,7 +1631,6 @@ icpc_kernel(const __grid_constant__ IcpcDev P, const SAMPLE* __restrict__ wf, lo
             }
             flags = (f0 ? 1u : 0u) | (fi ? 2u : 0u) | (f5 ? 4u : 0u) | (fe ? 8u : 0u);
         }
-        SECT(18);
 
         // ---- masks on the sg[0] trace (t50_current, in-trace pile-up on the REVERSED trace): only chunks whose
         //      maximum reaches the smaller threshold can contribute a bit ----
@@ -1729,7 +1669,6 @@ icpc_kernel(const __grid_constant__ IcpcDev P, const SAMPLE* __restrict__ wf, lo
                 else ovf |= 1u << type;
             }
         }
-        SECT(19);
 
         // ---- CUSP / ZAC ----
         double czmax[2] = {-CUDART_INF, -CUDART_INF};
@@ -1971,11 +1910,7 @@ icpc_kernel(const __grid_constant__ IcpcDev P, const SAMPLE* __restrict__ wf, lo
             if (rescan) {
                 __syncthreads();   // the previous pass is done with the tables, the coarse values and the output buffer
                 if (tid == 0) ibuf[IB_CZN] = 0;
-#ifdef LGDSP_PROFILE_SECTIONS
-                cz_scan<SM_PAR>(ps, TT, n, tid, tabA, tabB, red + R_CZSCR * NWARP, scr + SC_PP0, nullptr, &sect_last);
-#else
                 cz_scan<SM_PAR>(ps, TT, n, tid, tabA, tabB, red + R_CZSCR * NWARP, scr + SC_PP0);
-#endif
                 __syncthreads();
             }
             CzState st;
@@ -1996,10 +1931,7 @@ icpc_kernel(const __grid_constant__ IcpcDev P, const SAMPLE* __restrict__ wf, lo
                 red_put(red, R_CZC0, wid, lane, wc);
                 red_put(red, R_CZC1, wid, lane, wz);
             }
-            SECT(20);
             __syncthreads();   // ---- B4: tables are dead, coarse values and the work queue are complete ----
-            LGDSP_PHASE(4);
-            SECT(21);
             if (czp && last_pass) prefetch_next();   // every thread has read its table entries: xs may be overwritten
             // candidate chunks: Lipschitz bound on (33 tid, 33 tid + 33) against the best coarse value; chunks that
             // hold part of a pick-off window are always evaluated
@@ -2040,14 +1972,12 @@ icpc_kernel(const __grid_constant__ IcpcDev P, const SAMPLE* __restrict__ wf, lo
                 base = __shfl_sync(FULL, base, 0);
                 if (cand) slot = base + __popc(bc & ((1u << lane) - 1u));
             }
-            SECT(22);
             // the queued intervals, spread over all warps (before the long recurrences of the candidate warps)
             if (!queue_done) {
                 run_queue();
                 queue_done = true;
             }
             if (last_pass) __syncthreads();   // ---- Bq: masks and trapezoid partials are complete ----
-            SECT(29);
             // rounds: recurrences of up to CZCAP candidate chunks write their outputs to SMEM, then the whole block
             // takes maxima / first argmaxima / pick-off windows from there
             double* czbuf = tabB;
@@ -2057,11 +1987,8 @@ icpc_kernel(const __grid_constant__ IcpcDev P, const SAMPLE* __restrict__ wf, lo
                     ibuf[IB_CZT + slot - r0] = tid;
                     cz_out(Z, TT, n, tid, st, czbuf + (size_t)(slot - r0) * (CH * 2));
                 }
-                SECT(23);
                 if (last_pass && r0 == 0) scalar_jobs();   // overlaps the recurrences of the candidate warps
-                SECT(27);
                 __syncthreads();   // ---- B5 ----
-                SECT(30);
                 const int ncz = czp ? ibuf[IB_CZN] : 0;
                 const int nslot = min(ncz - r0, CZCAP);
                 const int nw = P.sig_dni.n_w;
@@ -2096,11 +2023,7 @@ icpc_kernel(const __grid_constant__ IcpcDev P, const SAMPLE* __restrict__ wf, lo
                 red[R_CZMAX1 * NWARP + wid] = czmax[1]; red[R_CZARG1 * NWARP + wid] = (double)czarg[1];
             }
         }
-        SECT(24);
-        SECT(25);
         __syncthreads();   // ---- B6 ----
-        LGDSP_PHASE(5);
-        SECT(26);
 
         if (wid == 3 || wid == 4) {
             if (cz_on) {
@@ -2118,19 +2041,10 @@ icpc_kernel(const __grid_constant__ IcpcDev P, const SAMPLE* __restrict__ wf, lo
                 }
             }
         }
-        SECT(28);
         __syncthreads();   // ---- B8 ----
-        LGDSP_PHASE(6);
-        SECT(28);
         if (tid < LGDSP_NCOL) rows[e * LGDSP_NCOL + tid] = wrapped ? CUDART_NAN : row[tid];
         // (the next iteration's first barrier orders the reuse of row/stash/masks/scr/red)
     }
-    if (pc_on) {
-#pragma unroll
-        for (int i = 0; i < 8; ++i) P.phase_cycles[blockIdx.x * 8 + i] = pc_acc[i];
-    }
-#undef LGDSP_PHASE
-#undef SECT
 }
 
 // ==================================================================================================
@@ -2465,22 +2379,17 @@ int sweep_warp_max_window() { return SWW_MAX_STEPS * SWW_STEP; }
 int sweep_launch(const SweepDev& P, const double* dni_A_host, const void* d_wf, int sample_bytes, long long n_events, long long ld,
                  const double* d_bl_ext, void* d_out, double* d_aux, int grid, int sm_count, cudaStream_t stream)
 {
-    // LGDSP_SWEEP_PATH=cta forces the one-CTA-per-waveform kernel (A/B tests); LGDSP_SWEEP_WPE=2: two warps per waveform (default 1)
+    // LGDSP_SWEEP_PATH=cta forces the one-CTA-per-waveform kernel (A/B tests)
     const char* env = getenv("LGDSP_SWEEP_PATH");
     if (P.warp_ok && sample_bytes == 2 && dni_A_host && !(env && strcmp(env, "cta") == 0)) {
-        const char* ew = getenv("LGDSP_SWEEP_WPE");
-        const int wpe = (ew && ew[0] == '2') ? 2 : 1;   // measured: 2 warps per waveform 37.0 M wf/s, 1 warp 40.2 M (instruction fetch)
-        const SwwGeom g = wpe == 1 ? sww_geometry_t<1>(P.win_steps) : sww_geometry_t<2>(P.win_steps);
-        if (g.ctas_per_sm > 0) {
+        const int ctas_per_sm = sww_geometry(P.win_steps);
+        if (ctas_per_sm > 0) {
             SweepDni D;
             memcpy(D.A, dni_A_host, sizeof(D.A));
-            const long long cap = (long long)sm_count * g.ctas_per_sm;
+            const long long cap = (long long)sm_count * ctas_per_sm;
             const int wgrid = (int)(n_events < cap ? n_events : cap);
             const size_t smem = (size_t)sww_warp_bytes(P.win_steps);
-            if (wpe == 1)
-                sweep_warp_kernel<1><<<wgrid, 32, smem, stream>>>(P, D, static_cast<const uint16_t*>(d_wf), n_events, ld, d_bl_ext, d_out, d_aux);
-            else
-                sweep_warp_kernel<2><<<wgrid, 64, smem, stream>>>(P, D, static_cast<const uint16_t*>(d_wf), n_events, ld, d_bl_ext, d_out, d_aux);
+            sweep_warp_kernel<<<wgrid, 32, smem, stream>>>(P, D, static_cast<const uint16_t*>(d_wf), n_events, ld, d_bl_ext, d_out, d_aux);
             return 1;
         }
     }

@@ -1051,10 +1051,7 @@ constexpr int CZ_HDR = 16;                    // doubles per (event, pass) heade
 enum { CZH_N = 0, CZH_MAXC, CZH_ARGC, CZH_MAXZ, CZH_ARGZ, CZH_PKP0, CZH_PKF0, CZH_PKP1, CZH_PKF1,
        CZH_CNT };                                    // (pass 0 only) arrival counter of the finish kernel's warps, zeroed here
 constexpr int CZP_LEN = CZ_HDR + CZ_MAXC * CZ_REC;   // doubles per (event, pass)
-#ifndef LGDSP_K4_NBLK
-#define LGDSP_K4_NBLK 4
-#endif
-constexpr int K4_NBLK = LGDSP_K4_NBLK;               // warps of the finish kernel that may share one event
+constexpr int K4_NBLK = 4;                           // warps of the finish kernel that may share one event
 constexpr int CZ_SCR = K4_NBLK * 4 + 2 * LGDSP_MAX_DNI;   // their exchange area: partial (max, argmax) x 2 + the two pick-off windows
 constexpr int CZG_LEN = 2 * CZP_LEN + CZ_SCR;        // doubles per event slot
 

@@ -26,31 +26,22 @@
 //              A variant whose window leaves [lo, lo + W) -- clamped pick-offs of events with t50 at the trace ends -- waits
 //              for a second window built where it needs it (rare; the loop ends because every variant fits W on its own).
 //
-// No block barrier, no atomics (sweep_warp_kernel<1>, the default: one warp = one CTA).  sweep_warp_kernel<2> splits every phase
-// over a team of two warps (same shared memory per waveform, twice the resident warps, ~8 barriers of 64 threads): measured
-// slower (37.0 vs 40.4 M wf/s, instruction fetch), kept behind LGDSP_SWEEP_WPE=2.  Outputs are bit-identical to sweep_kernel's
-// (same arithmetic on the same exact integers), which stays the path of FIR / Savitzky-Golay variants, 32-bit samples and
-// variant sets whose reach exceeds the window capacity.
+// No block barrier, no atomics: one warp is one CTA.  Residency is limited by the float64 window in shared memory, not by the
+// thread count.  A team of two warps per waveform (every phase split, ~8 barriers of 64 threads per waveform, twice the resident
+// warps) was measured slower, 37.0 vs 40.4 M wf/s (instruction fetch: 16 % more instructions for the redundant scalar work), and
+// was removed.  Outputs are bit-identical to sweep_kernel's (same arithmetic on the same exact integers), which stays the path of
+// FIR / Savitzky-Golay variants, 32-bit samples and variant sets whose reach exceeds the window capacity.
 
-#ifndef SWW_UNR
-#define SWW_UNR 11   // outputs per iteration of the pick-off window loop (measured: 2 / 4 / 11 / 44 -> 37.3 / 38.9 / 39.9 / 33.6 M wf/s)
-#endif
-#ifndef SWW_U1A
-#define SWW_U1A 1
-#endif
-#ifndef SWW_U1B
-#define SWW_U1B 1
-#endif
-constexpr int kU1A = SWW_U1A, kU1B = SWW_U1B;   // unroll factors of the group loops (pragma arguments are not macro-expanded)
 constexpr int SWW_STEP = 288;        // samples per window-build step (9 per lane)
 constexpr int SWW_MIN_STEPS = 4;     // the window area also holds pass 1's group table (8 KB)
 constexpr int SWW_MAX_STEPS = 10;
 constexpr int SWW_EXT_BYTES = 4096;  // float2 per 16-sample group
 __host__ __device__ constexpr int sww_win_bytes(int steps) { return (steps * SWW_STEP + 8) * 8; }
-// per waveform: window | mask | cP[20] | cPP[18] | locPP[16] | xch[8] | stepP[16] | xchi[4]   (11 CTAs per SM at 8 window steps)
+// per waveform: window | mask | cP[20] | cPP[18] | 272 spare bytes   (11 CTAs per SM at 8 window steps).  The spare bytes keep
+// the CTAs per SM that every window size was measured with: without them a 9-step window would fit 10 CTAs per SM instead of 9.
 __host__ __device__ constexpr int sww_warp_bytes(int steps)
 {
-    return sww_win_bytes(steps) + NWORDS * 4 + 20 * 4 + 18 * 8 + 16 * 8 + 8 * 8 + 16 * 4 + 4 * 4;
+    return sww_win_bytes(steps) + NWORDS * 4 + 20 * 4 + 18 * 8 + 272;
 }
 
 struct SweepDni {
@@ -173,9 +164,9 @@ __device__ __forceinline__ void sww_dni_sums(const SweepDni& D, const double* p0
     const double* p3 = p0 + t.L;
     c0 = 0; c1 = 0; c2 = 0; c3 = 0;
     if (NW > 0) {
-        // blocks of 4 outputs: the loop body (about 60 instructions) stays inside the instruction cache of a scheduler; a
-        // complete unroll (44 x 12 instructions) ran fetch-bound
-        constexpr int UNR = SWW_UNR;
+        // blocks of 11 outputs: the loop body stays inside the instruction cache of a scheduler; a complete unroll (44 x 12
+        // instructions) ran fetch-bound (measured: blocks of 2 / 4 / 11 / 44 -> 37.3 / 38.9 / 39.9 / 33.6 M wf/s)
+        constexpr int UNR = 11;
         static_assert(NW % UNR == 0, "window length must be a multiple of the unroll factor");
 #pragma unroll 1
         for (int ib = 0; ib < NW; ib += UNR) {
@@ -202,55 +193,27 @@ __device__ __forceinline__ void sww_dni_sums(const SweepDni& D, const double* p0
     }
 }
 
-// WPE warps (a CTA) own one waveform: WPE = 1 needs no block barrier at all; WPE = 2 halves every phase and doubles the warps an
-// SM holds (the float64 window, not the thread count, limits residency) for ~8 CTA-wide barriers of 64 threads per waveform.
-template <int WPE>
-__device__ __forceinline__ void sww_team_sync()
-{
-    if (WPE == 1) __syncwarp();
-    else __syncthreads();
-}
-// maximum over the team of a warp-uniform value (slot: a distinct exchange slot per use inside one waveform)
-template <int WPE>
-__device__ __forceinline__ double sww_team_max(double v, double* xch, int slot, int we, int lane)
-{
-    if (WPE == 1) return v;
-    if (lane == 0) xch[slot * WPE + we] = v;
-    __syncthreads();
-    double r = xch[slot * WPE];
-#pragma unroll
-    for (int w = 1; w < WPE; ++w) r = xch[slot * WPE + w] > r ? xch[slot * WPE + w] : r;
-    return r;
-}
-
-template <int WPE>
-__global__ void __launch_bounds__(32 * WPE, 11)
+__global__ void __launch_bounds__(32, 11)
 sweep_warp_kernel(const __grid_constant__ SweepDev P, const __grid_constant__ SweepDni D, const uint16_t* __restrict__ wf,
                   long long n_events, long long ld, const double* __restrict__ bl_ext, void* __restrict__ out,
                   double* __restrict__ aux)
 {
     extern __shared__ __align__(128) unsigned char smem[];
-    const int lane = threadIdx.x & 31, we = threadIdx.x >> 5;
+    const int lane = threadIdx.x & 31;
     const int steps = P.win_steps;
     const int W = steps * SWW_STEP;
     unsigned char* base = smem;
     double* win = reinterpret_cast<double*>(base);
     float2* ext = reinterpret_cast<float2*>(base);
-    // P at the group start: absolute (WPE == 1) / relative to its 512-sample step, whose carry is known after the team's barrier
     uint32_t* pst = reinterpret_cast<uint32_t*>(base + SWW_EXT_BYTES);
     uint32_t* xmm = pst + MAXN / 16;
     uint32_t* mask = reinterpret_cast<uint32_t*>(base + sww_win_bytes(steps));
     uint32_t* cP = mask + NWORDS;
     double* cPP = reinterpret_cast<double*>(cP + 20);
-    double* locPP = cPP + 18;                                           // [16] sum over a step of (P(i) - P(step start))
-    double* xch = locPP + 16;                                           // [2][WPE <= 4] team exchange slots
-    uint32_t* stepP = reinterpret_cast<uint32_t*>(xch + 8);            // [16] sum of the samples of a step
-    int* xchi = reinterpret_cast<int*>(stepP + 16);                     // [4]
 
-    const int n = P.n, n_it = (n + 511) >> 9;
+    const int n = P.n;
     const double t_first = P.t_first, dt = P.dt, km1 = P.km1;
     const int n_w = P.sig_dni.n_w, mdeg = P.sig_dni.m;
-    auto pbase = [&](int it) -> uint32_t { return WPE == 1 ? 0u : cP[it]; };
 
     for (long long e = blockIdx.x; e < n_events; e += gridDim.x) {
         const uint16_t* __restrict__ x = wf + e * ld;
@@ -261,19 +224,19 @@ sweep_warp_kernel(const __grid_constant__ SweepDev P, const __grid_constant__ Sw
         const int n_s = need_t50 ? n : min(n, (P.stream_n + 15) & ~15);   // samples of the integer pass (multiple of 8: n is)
         const int n_it_s = (n_s + 511) >> 9;
         if (threadIdx.x == 0 && e + gridDim.x < n_events) tma_prefetch_l2(wf + (e + gridDim.x) * ld, (uint32_t)n_s * 2u);
-        // ---- pass 1 (integers only): the steps it = we, we + WPE, ...; prefix sums inside the step, group table, step sums ----
+        // ---- pass 1 (integers only): steps of 512 samples; prefix sums, group table, P and PP at the step boundaries ----
         {
-            uint32_t carryP = 0;             // (WPE == 1: the steps follow each other, the carries run along)
+            uint32_t carryP = 0;
             unsigned long long carryPP = 0;
-            uint4 ra[3], rb[3];   // raw samples of this warp's next three steps
+            uint4 ra[3], rb[3];   // raw samples of the next three steps
 #pragma unroll
-            for (int q = 0; q < 3; ++q) sww_ld16_raw(x, (we + q * WPE) * 512 + 16 * lane, n_s, ra[q], rb[q]);
+            for (int q = 0; q < 3; ++q) sww_ld16_raw(x, q * 512 + 16 * lane, n_s, ra[q], rb[q]);
 #pragma unroll 1
-            for (int it = we; it < n_it_s; it += WPE) {
+            for (int it = 0; it < n_it_s; ++it) {
                 uint32_t v[16];
                 sww_unpack16(ra[0], rb[0], v);
                 ra[0] = ra[1]; rb[0] = rb[1]; ra[1] = ra[2]; rb[1] = rb[2];
-                sww_ld16_raw(x, (it + 3 * WPE) * 512 + 16 * lane, n_s, ra[2], rb[2]);    // three steps ahead
+                sww_ld16_raw(x, (it + 3) * 512 + 16 * lane, n_s, ra[2], rb[2]);    // three steps ahead
                 uint32_t s[16];
                 s[0] = v[0];
 #pragma unroll
@@ -300,35 +263,16 @@ sweep_warp_kernel(const __grid_constant__ SweepDev P, const __grid_constant__ Sw
                 for (int k = 0; k < 16; k += 4) tl += (s[k] + s[k + 1]) + (s[k + 2] + s[k + 3]);
                 const uint32_t sum_t = __reduce_add_sync(FULL, tl);
                 const uint32_t sum_ex = __reduce_add_sync(FULL, (uint32_t)(31 - lane) * s[15]);
-                if (WPE == 1) {
-                    if (lane == 0) { cP[it] = carryP; cPP[it] = (double)carryPP; }
-                    if (need_t50 && i0 < n) pst[it * 32 + lane] = carryP + incl - s[15];
-                    carryPP += 512ull * carryP + 16ull * sum_ex + sum_t;
-                    carryP += __shfl_sync(FULL, incl, 31);
-                } else {
-                    if (lane == 31) {
-                        stepP[it] = incl;
-                        locPP[it] = (double)(16ull * sum_ex + sum_t);
-                    }
-                    if (need_t50 && i0 < n) pst[it * 32 + lane] = incl - s[15];
-                }
+                // P and PP = cumsum(P) at every 512-sample boundary (exact integers; PP < 2^43 in float64)
+                if (lane == 0) { cP[it] = carryP; cPP[it] = (double)carryPP; }
+                if (need_t50 && i0 < n) pst[it * 32 + lane] = carryP + incl - s[15];
+                carryPP += 512ull * carryP + 16ull * sum_ex + sum_t;
+                carryP += __shfl_sync(FULL, incl, 31);
                 if (need_t50 && i0 < n) xmm[it * 32 + lane] = (xmax << 16) | xmin;
             }
-            if (WPE == 1 && lane == 0) { cP[n_it_s] = carryP; cPP[n_it_s] = (double)carryPP; }
+            if (lane == 0) { cP[n_it_s] = carryP; cPP[n_it_s] = (double)carryPP; }
         }
-        sww_team_sync<WPE>();
-        // P and PP = cumsum(P) at every 512-sample boundary (exact integers; PP < 2^43 in float64)
-        if (WPE > 1 && we == 0 && lane <= n_it_s) {
-            uint32_t cp = 0;
-            double cpp = 0.0;
-            for (int i = 0; i < lane; ++i) {
-                cpp += fma(512.0, u2d(cp), locPP[i]);
-                cp += stepP[i];
-            }
-            cP[lane] = cp;
-            cPP[lane] = cpp;
-        }
-        sww_team_sync<WPE>();
+        __syncwarp();
 
         // ---- baseline window from the prefix sums: sum x = P(b+1) - P(a), sum i*x = b*P(b+1) - a*P(a) - (PP(b) - PP(a)) ----
         double blSd, blSXd = 0.0;
@@ -359,12 +303,13 @@ sweep_warp_kernel(const __grid_constant__ SweepDev P, const __grid_constant__ Sw
             float best_ub = -CUDART_INF_F;
             int best_it = -1;
             const int my_groups = (n - 16 * lane + 511) >> 9;   // groups of this lane's column (<= 0: none)
-#pragma unroll (kU1A)
-            for (int it = we; it < my_groups; it += WPE) {
+            // (the group loops of pass 1a / 1b unrolled by 2 or 4: 38.0-38.4 M wf/s, code size)
+#pragma unroll 1
+            for (int it = 0; it < my_groups; ++it) {
                 const int i0 = it * 512 + 16 * lane;
                 const uint32_t xm = xmm[it * 32 + lane];
                 const double dmax = u2d(xm >> 16) - m, dmin = u2d(xm & 0xffffu) - m;
-                const double Sd0 = fma(-(double)i0, m, u2d(pst[it * 32 + lane] + pbase(it)));
+                const double Sd0 = fma(-(double)i0, m, u2d(pst[it * 32 + lane]));
                 const double Sd_hi = fma(16.0, dmax > 0.0 ? dmax : 0.0, Sd0), Sd_lo = fma(16.0, dmin < 0.0 ? dmin : 0.0, Sd0);
                 const double k_hi = km1 >= 0.0 ? Sd_hi : Sd_lo, k_lo = km1 >= 0.0 ? Sd_lo : Sd_hi;
                 const double ub = fma(km1, k_hi, dmax) + G;
@@ -377,37 +322,37 @@ sweep_warp_kernel(const __grid_constant__ SweepDev P, const __grid_constant__ Sw
             }
             // every lane evaluates the group with its largest upper bound exactly: a lower bound close to the maximum ...
             double ymax = -CUDART_INF;
-            if (best_it >= 0) ymax = sww_group_max(x, best_it * 512 + 16 * lane, n, pst[best_it * 32 + lane] + pbase(best_it), m, km1);
-            const double LB = sww_team_max<WPE>(fmax(warp_max(ymax), warp_max(lbmax)), xch, 0, we, lane);
+            if (best_it >= 0) ymax = sww_group_max(x, best_it * 512 + 16 * lane, n, pst[best_it * 32 + lane], m, km1);
+            const double LB = fmax(warp_max(ymax), warp_max(lbmax));
             // ... and only groups whose upper bound reaches it can hold a larger sample
 #pragma unroll 1
-            for (int it = we; it < my_groups; it += WPE) {
+            for (int it = 0; it < my_groups; ++it) {
                 const int i0 = it * 512 + 16 * lane;
                 if ((double)ext[it * 32 + lane].x >= LB && it != best_it) {
-                    const double gm = sww_group_max(x, i0, n, pst[it * 32 + lane] + pbase(it), m, km1);
+                    const double gm = sww_group_max(x, i0, n, pst[it * 32 + lane], m, km1);
                     ymax = gm > ymax ? gm : ymax;
                 }
             }
-            ymax = sww_team_max<WPE>(warp_max(ymax), xch, 1, we, lane);
+            ymax = warp_max(ymax);
             thr = ymax * 0.5;
 
             // ---- pass 1b: threshold mask of y >= thr, first run of >= tx_min_n samples ----
-#pragma unroll (kU1B)
-            for (int it = we; it < NWORDS / 16; it += WPE) {
+#pragma unroll 1
+            for (int it = 0; it < NWORDS / 16; ++it) {
                 uint32_t b = 0;
                 const int i0 = it * 512 + 16 * lane;
                 if (i0 < n) {
                     const float2 ex = ext[it * 32 + lane];
                     if ((double)ex.x >= thr) {
                         if ((double)ex.y >= thr) b = (i0 + 8 < n) ? 0xffffu : 0xffu;
-                        else b = sww_group_bits(x, i0, n, pst[it * 32 + lane] + pbase(it), m, km1, thr);
+                        else b = sww_group_bits(x, i0, n, pst[it * 32 + lane], m, km1, thr);
                     }
                 }
                 b <<= 16 * (lane & 1);
                 b |= __shfl_xor_sync(FULL, b, 1);
                 if ((lane & 1) == 0) mask[it * 16 + (lane >> 1)] = b;
             }
-            sww_team_sync<WPE>();
+            __syncwarp();
             int mult;
             resolve_runs(mask, P.tx_min_n, lane, pos, mult);
 
@@ -421,42 +366,37 @@ sweep_warp_kernel(const __grid_constant__ SweepDev P, const __grid_constant__ Sw
         unsigned done = 0;
         double t50_us = 0.0;
         bool first = true;
-        constexpr int VSTRIDE = 32 * WPE;                  // variants per round of the team
-        const int vlane = we * 32 + lane;
         // (the first round's variant parameters travel while the window is built)
-        const TrapDev t_first_round = P.vars[min(vlane, P.nvar - 1)].t;
-        const double pick_first_round = P.vars[min(vlane, P.nvar - 1)].pick_ns;
-        const int mode_first_round = P.vars[min(vlane, P.nvar - 1)].mode;
+        const TrapDev t_first_round = P.vars[min(lane, P.nvar - 1)].t;
+        const double pick_first_round = P.vars[min(lane, P.nvar - 1)].pick_ns;
+        const int mode_first_round = P.vars[min(lane, P.nvar - 1)].mode;
         int rounds = 0;
-        const int steps_w = (steps + WPE - 1) / WPE;       // window steps per warp: warp `we` builds [we*steps_w, (we+1)*steps_w)
 #pragma unroll 1
         while (true) {
-            sww_team_sync<WPE>();   // every read of the group table / the previous window is over
-            const int j_from = we * steps_w, j_until = min(steps, j_from + steps_w);
-            if (j_from < j_until) {
-                // prefix sums at this warp's first sample
-                const int start = lo + SWW_STEP * j_from;
+            __syncwarp();   // every read of the group table / the previous window is over
+            if (steps > 0) {   // (always true: the launch needs SWW_MIN_STEPS; the guard keeps the measured code generation)
+                // prefix sums at the window's first sample
                 uint32_t cp;
                 double cpp;
-                sww_prefix_at(x, n, cP, cPP, min(start, n), lane, cp, cpp);
-                if (we == 0 && lane == 0) {
+                sww_prefix_at(x, n, cP, cPP, min(lo, n), lane, cp, cpp);
+                if (lane == 0) {
                     const double lod = (double)lo;
                     const double tri = 0.5 * lod * (lod + 1.0);
                     win[0] = fma(km1, fma(-tri, m, cpp), fma(-lod, m, u2d(cp)));
                 }
                 uint32_t q[9];
                 {
-                    const int i0 = start + 9 * lane;
+                    const int i0 = lo + 9 * lane;
 #pragma unroll
                     for (int k = 0; k < 9; ++k) q[k] = (i0 + k < n) ? (uint32_t)__ldg(x + i0 + k) : 0u;
                 }
 #pragma unroll 1
-                for (int j = j_from; j < j_until; ++j) {
+                for (int j = 0; j < steps; ++j) {
                     uint32_t v[9];
 #pragma unroll
                     for (int k = 0; k < 9; ++k) v[k] = q[k];
                     const int i0 = lo + SWW_STEP * j + 9 * lane;
-                    if (j + 1 < j_until) {
+                    if (j + 1 < steps) {
 #pragma unroll
                         for (int k = 0; k < 9; ++k) q[k] = (i0 + SWW_STEP + k < n) ? (uint32_t)__ldg(x + i0 + SWW_STEP + k) : 0u;
                     }
@@ -502,7 +442,7 @@ sweep_warp_kernel(const __grid_constant__ SweepDev P, const __grid_constant__ Sw
                     cp += __shfl_sync(FULL, incl, 31);
                 }
             }
-            sww_team_sync<WPE>();
+            __syncwarp();
             const double* TTw = win - lo;   // TTw[i] = TT[i] for lo <= i <= lo + W
             if (first) {
                 first = false;
@@ -517,9 +457,9 @@ sweep_warp_kernel(const __grid_constant__ SweepDev P, const __grid_constant__ Sw
                 }
             }
             int minfrom = 0x7fffffff;
-            // Warp-uniform loop over rounds of 32*WPE variants: every lane runs the arithmetic (a lane without work reads the start of
+            // Warp-uniform loop over rounds of 32 variants: every lane runs the arithmetic (a lane without work reads the start of
             // the window), so the inner loop sits in convergent code and the fit matrix is read through the uniform datapath
-            const int n_rounds = (P.nvar + VSTRIDE - 1) / VSTRIDE;
+            const int n_rounds = (P.nvar + 31) / 32;
             int rnd;
             // this lane's variant of the next round is loaded one round ahead (the table comes from L2 / L1)
             TrapDev tn = t_first_round;
@@ -527,12 +467,12 @@ sweep_warp_kernel(const __grid_constant__ SweepDev P, const __grid_constant__ Sw
             int moden = mode_first_round;
 #pragma unroll 1
             for (rnd = 0; rnd < n_rounds; ++rnd) {
-                const int v = rnd * VSTRIDE + vlane;
+                const int v = rnd * 32 + lane;
                 const TrapDev tv = tn;
                 const double pick = pickn;
                 const int mode = moden;
                 {
-                    const SweepVar& nx = P.vars[min(v + VSTRIDE, P.nvar - 1)];
+                    const SweepVar& nx = P.vars[min(v + 32, P.nvar - 1)];
                     tn = nx.t; pickn = nx.pick_ns; moden = nx.mode;
                 }
                 bool eval = false;
@@ -567,18 +507,11 @@ sweep_warp_kernel(const __grid_constant__ SweepDev P, const __grid_constant__ Sw
                 }
             }
             minfrom = __reduce_min_sync(FULL, minfrom);
-            if (WPE > 1) {   // the decision to build another window belongs to the team
-                if (lane == 0) xchi[we] = minfrom;
-                __syncthreads();
-#pragma unroll
-                for (int w = 0; w < WPE; ++w) minfrom = min(minfrom, xchi[w]);
-                __syncthreads();
-            }
             if (minfrom == 0x7fffffff) break;
             if (++rounds > 2 * 1024 / 32 + 2) {
                 // cannot happen (every variant fits a window that starts at its own `from`); never spin on the device
                 rnd = 0;
-                for (int v = vlane; v < P.nvar; v += VSTRIDE, ++rnd) {
+                for (int v = lane; v < P.nvar; v += 32, ++rnd) {
                     if ((done >> rnd) & 1u) continue;
                     if (P.out_f64) reinterpret_cast<double*>(out)[e * (long long)P.nvar + v] = CUDART_NAN;
                     else reinterpret_cast<float*>(out)[e * (long long)P.nvar + v] = CUDART_NAN_F;
@@ -587,36 +520,29 @@ sweep_warp_kernel(const __grid_constant__ SweepDev P, const __grid_constant__ Sw
             }
             lo = max(0, min(minfrom, lo_max));
         }
-        sww_team_sync<WPE>();   // the window area becomes the next event's group table
+        __syncwarp();   // the window area becomes the next event's group table
     }
 }
 
-// launch geometry for a window of `steps` steps: warps per waveform (CTA) and CTAs per SM
-struct SwwGeom {
-    int warps_per_cta = 0, ctas_per_sm = 0;
-};
-template <int WPE>
-inline SwwGeom sww_geometry_t(int steps)
+// launch geometry for a window of `steps` steps: CTAs (one waveform each) per SM, 0 if the kernel cannot run
+inline int sww_geometry(int steps)
 {
-    static SwwGeom cache[SWW_MAX_STEPS + 1];
+    static int cache[SWW_MAX_STEPS + 1];
     static bool attr_set = false;
-    if (steps < SWW_MIN_STEPS || steps > SWW_MAX_STEPS) return SwwGeom{};
-    if (cache[steps].warps_per_cta) return cache[steps];
+    if (steps < SWW_MIN_STEPS || steps > SWW_MAX_STEPS) return 0;
+    if (cache[steps]) return cache[steps];
     if (!attr_set) {
         int dev = 0, optin = 0;
         cudaGetDevice(&dev);
         cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
-        if (cudaFuncSetAttribute(sweep_warp_kernel<WPE>, cudaFuncAttributeMaxDynamicSharedMemorySize, optin) != cudaSuccess) return SwwGeom{};
+        if (cudaFuncSetAttribute(sweep_warp_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, optin) != cudaSuccess) return 0;
         attr_set = true;
     }
-    SwwGeom g;
     int nb = 0;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, sweep_warp_kernel<WPE>, WPE * 32, (size_t)sww_warp_bytes(steps)) != cudaSuccess) {
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, sweep_warp_kernel, 32, (size_t)sww_warp_bytes(steps)) != cudaSuccess) {
         cudaGetLastError();
-        return SwwGeom{};
+        return 0;
     }
-    g.warps_per_cta = WPE;
-    g.ctas_per_sm = nb;
-    if (nb > 0) cache[steps] = g;
-    return g;
+    cache[steps] = nb;
+    return nb;
 }

@@ -35,26 +35,6 @@ LEAN_COLUMNS = ("blmean", "t0", "t50", "e_trap", "e_10410", "e_max", "e_min", "n
 PZ_TRAP_COLUMNS = ("blmean", "t0", "t50", "e_trap", "e_10410")                               # O.pz_trap's five
 
 
-class _env:
-    """set (or remove, value None) one environment variable for the duration of a block"""
-
-    def __init__(self, name, value):
-        self.name, self.value = name, value
-
-    def __enter__(self):
-        self.old = os.environ.get(self.name)
-        if self.value is None:
-            os.environ.pop(self.name, None)
-        else:
-            os.environ[self.name] = self.value
-
-    def __exit__(self, *a):
-        if self.old is None:
-            os.environ.pop(self.name, None)
-        else:
-            os.environ[self.name] = self.old
-
-
 def _t_first(L, rng, cfg):
     """a non-zero time of the first sample, up to +-20 us and up to 0.4 of the baseline window's end (the in-trace pile-up
     window starts at leftendpoint(bl_window) + first(time), src/dsp_routines.jl:75: it has to stay on the trace), on a multiple
@@ -265,22 +245,15 @@ def _warp_runs(L, handle, S64, S32, wf, W, cfg, tau, var, tvar):
         wide[:, :n] = wf
         strided = np.zeros((ne, len(var)))
         handle.gsweep_run_host(S64, wide.ctypes.data, ne, n + 24, var.array, strided.ctypes.data)
-        with _env("LGDSP_SWEEP_WPE", "2"):
-            team = _run_general(W, cfg, tau, var, f64=True, handle=handle)
-            a_t, aux_t = _run_general(W, cfg, tau, var, f64=True, want_aux=True, handle=handle)
-        with _env("LGDSP_SWEEP_WPE", "1"):
-            one = _run_general(W, cfg, tau, var, f64=True, handle=handle)
     with sweep_path("cta"):
         a_c, aux_c = _run_general(W, cfg, tau, var, f64=True, want_aux=True, handle=handle)
         c32 = _run_general(W, cfg, tau, var, f64=False, handle=handle)
     default = _run_general(W, cfg, tau, var, f64=True, handle=handle)
-    for name, v in (("warp + aux", a_w), ("strided", strided), ("2 warps", team), ("2 warps + aux", a_t), ("1 warp", one),
-                    ("cta", a_c), ("default dispatch", default)):
+    for name, v in (("warp + aux", a_w), ("strided", strided), ("cta", a_c), ("default dispatch", default)):
         assert np.array_equal(v, base, equal_nan=True), (name, np.nanmax(np.abs(v - base)))
     b32 = base.astype(np.float32)
     for name, v in (("f32", f32), ("lgdsp_trap_sweep_run", t32), ("cta f32", c32)):
         assert np.array_equal(v, b32, equal_nan=True), name
-    assert np.array_equal(aux_t, aux_w, equal_nan=True)
     return base, aux_w, aux_c
 
 

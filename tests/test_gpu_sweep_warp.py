@@ -52,19 +52,7 @@ def _grid(L):
     return rts, fts
 
 
-@pytest.fixture(params=["1", "2"])
-def wpe(request):
-    """warps per waveform of the warp path (LGDSP_SWEEP_WPE; 1 is the default, 2 the measured-and-slower team variant)"""
-    old = os.environ.get("LGDSP_SWEEP_WPE")
-    os.environ["LGDSP_SWEEP_WPE"] = request.param
-    yield request.param
-    if old is None:
-        os.environ.pop("LGDSP_SWEEP_WPE", None)
-    else:
-        os.environ["LGDSP_SWEEP_WPE"] = old
-
-
-def test_warp_path_equals_cta_path_and_oracle_on_the_grid(L, O, handle, wpe):
+def test_warp_path_equals_cta_path_and_oracle_on_the_grid(L, O, handle):
     cfg, tau = L.example_config(), L.us(500.0)
     wf = np.concatenate([L.synth.generate_host(700, first_event=4242), L.synth.generate_host(40, mode=1), _pathological(8192)])
     W = L.RDWaveforms(wf)
@@ -84,7 +72,7 @@ def test_warp_path_equals_cta_path_and_oracle_on_the_grid(L, O, handle, wpe):
 
 
 @pytest.mark.parametrize("n_samples", [264, 1024, 4104, 6000, 8192])
-def test_warp_path_ragged_lengths(L, O, handle, n_samples, wpe):
+def test_warp_path_ragged_lengths(L, O, handle, n_samples):
     cfg, tau = L.example_config(), L.us(500.0)
     full = L.synth.generate_host(96, first_event=77)
     a0 = max(0, 3400 - n_samples // 2) // 8 * 8

@@ -26,18 +26,3 @@ for rep in range(2):
     t_st = h.last_kernel_ms()
 print(f"{n} events: presummed pass {t_pre:.3f} ms ({n / t_pre / 1e3:.2f} M ev/s), windowed pass {t_wdw:.3f} ms ({n / t_wdw / 1e3:.2f} M ev/s), "
       f"window stats {t_st:.3f} ms")
-h.phase_cycles(True)
-for name, P, d, sb, ld, b in (("presummed", Pp, d_pre, 4, 1024, None), ("windowed", Pw, d_wdw, 2, 1400, bl)):
-    h.icpc_run_ext_device(P, d.data_ptr(), sb, b.data_ptr() if b is not None else None, n, ld, rows.data_ptr()); h.synchronize()
-    c = h.phase_cycles(True)
-    print(name, "cycles/event per CTA:", " ".join(f"{nm}={v / n:.0f}" for nm, v in zip(["tma", "P1", "P2", "P3", "P4a", "P4b", "P5"], c)))
-    sec = h.section_cycles()
-    if sec and any(any(r) for r in sec):
-        names = {31: "tma wait", 0: "P1 loop", 1: "P1 red+scan", 2: "B1 wait", 3: "fold/sat/blstats", 4: "P2 TT loop", 5: "t10..t99 masks",
-                 6: "tail log", 7: "B2 wait", 8: "resolve t10..", 9: "pz tail stats", 10: "full traps", 11: "coarse traps",
-                 12: "sg0 chunk pass", 13: "sg1/2+deriv", 14: "sg reductions", 15: "cz_scan", 16: "B3 wait", 17: "t50/pk/stash",
-                 18: "trap items", 19: "sg masks", 20: "cz_init+coarse", 21: "B4 wait", 22: "cz cand", 23: "cz_run", 24: "final partials",
-                 25: "cz_scan to barrier", 26: "B6 wait", 27: "scalar jobs", 28: "cz jobs/B8 wait", 29: "queue items", 30: "B5 wait"}
-        for i in [31] + list(range(31)):
-            r = [v / n for v in sec[i]]
-            print(f"  {i:2d} {names.get(i, ''):18s} {max(r):8.0f} {sum(r) / 8:8.0f} | " + " ".join(f"{v:6.0f}" for v in r))
