@@ -223,6 +223,7 @@ enum lgdsp_sipm_col {
 #define LGDSP_SIPM_NFIELD 4
 #define LGDSP_SAMPLE_U16 2
 #define LGDSP_SAMPLE_F32 4
+#define LGDSP_SAMPLE_F64 8
 
 typedef struct lgdsp_sipm_params {
     uint32_t struct_size;      /* sizeof(lgdsp_sipm_params), checked */
@@ -493,12 +494,66 @@ int lgdsp_sipm_list_pointers_device(lgdsp_handle* h, const double* d_rows, int64
 int lgdsp_sipm_list_gather_device(lgdsp_handle* h, const double* d_trig, int64_t n_events, int32_t list, int32_t max_triggers,
                                   const int64_t* d_elem_ptr, double* d_flat, int64_t flat_stride);
 /* the in-tree primitives of the chain on single traces of doubles (host buffers; one trace per call, for tests and
- * small jobs): thresholdstats / thresholdstats_mad (src/thresholdstats.jl:19-41, 61-71) and IntersectMaximum
- * (src/intersect_maximum.jl:24-119; x/x_high/x_tot/max: double[max_triggers], returns the count in *n_found) */
+ * small jobs; n = 0 .. 65536): thresholdstats / thresholdstats_mad (src/thresholdstats.jl:19-41, 61-71) and IntersectMaximum
+ * (src/intersect_maximum.jl:24-119; x/x_high/x_tot/max: double[max_triggers], returns the count in *n_found).  Both are
+ * n_events = 1 calls of lgdsp_wfstats_run. */
 int lgdsp_thresholdstats(lgdsp_handle* h, const double* y, int32_t n, double min, double max, int32_t mad, double* out);
 int lgdsp_intersect_maximum(lgdsp_handle* h, const double* y, int32_t n, double t_first_ns, double dt_ns, double threshold,
                             int32_t min_n, int32_t max_n, int32_t max_triggers, double* x, double* x_high, double* x_tot,
                             double* max, int32_t* n_found);
+
+/* ---- per-waveform primitives on whole waveform arrays: the broadcasts f.(wvfs, ...) of the in-tree primitives ----
+ * One pass over each waveform computes every primitive selected in `what`; every window is a 0-based inclusive sample range
+ * and must lie inside [0, n_samples-1] for a selected primitive (the reference's @assert, src/tailstats.jl:23-25).
+ * Times (tmin, tmax, tail_tau, the IntersectMaximum x / x_high / x_tot) are in ns on the axis X[i] = t_first + i*dt. */
+#define LGDSP_WFSTAT_SATURATION         0x01u   /* saturation(wvf, low, high[, start, stop])   src/saturation.jl:12-65; U16 only */
+#define LGDSP_WFSTAT_EXTREMESTATS       0x02u   /* extremestats(wvf[, start, stop])           src/extremestats.jl:14-40 */
+#define LGDSP_WFSTAT_TAILSTATS          0x04u   /* tailstats(wvf, start, stop)                src/tailstats.jl:13-72 */
+#define LGDSP_WFSTAT_WVF_MAXIMUM        0x08u   /* get_wvf_maximum(wvf, start, stop)          src/interpolation.jl:21-46 */
+#define LGDSP_WFSTAT_THRESHOLDSTATS     0x10u   /* thresholdstats(wvf, min, max)              src/thresholdstats.jl:19-41 */
+#define LGDSP_WFSTAT_THRESHOLDSTATS_MAD 0x20u   /* thresholdstats_mad(wvf, min, max)          src/thresholdstats.jl:61-71 */
+#define LGDSP_WFSTAT_INTERSECT_MAXIMUM  0x40u   /* IntersectMaximum(mintot, maxtot)(wvf, thr) src/intersect_maximum.jl:24-119 */
+#define LGDSP_WFSTAT_ALL                0x7Fu
+/* output rows: double rows[n_events][LGDSP_WFSTAT_NCOL]; columns of unselected primitives are 0.  The saturation counts and
+ * the multiplicity are exact small integers; the multiplicity is the TRUE number of triggers (a value > max_triggers means
+ * the lists were cut and the call should be repeated with a larger capacity). */
+enum lgdsp_wfstat_col {
+    LGDSP_WFSTAT_sat_low = 0, LGDSP_WFSTAT_sat_high, LGDSP_WFSTAT_sat_max_cons_low, LGDSP_WFSTAT_sat_max_cons_high,
+    LGDSP_WFSTAT_min, LGDSP_WFSTAT_max, LGDSP_WFSTAT_tmin, LGDSP_WFSTAT_tmax,
+    LGDSP_WFSTAT_tail_mean, LGDSP_WFSTAT_tail_sigma, LGDSP_WFSTAT_tail_tau,
+    LGDSP_WFSTAT_wvf_max, LGDSP_WFSTAT_thr_sigma, LGDSP_WFSTAT_thr_mad, LGDSP_WFSTAT_multiplicity,
+    LGDSP_WFSTAT_NCOL /* = 15 */
+};
+#define LGDSP_WFSTAT_MAX_SAMPLES 65536
+#define LGDSP_WFSTAT_MAX_TRIGGERS 65536
+
+typedef struct lgdsp_wfstats_params {
+    uint32_t struct_size;      /* sizeof(lgdsp_wfstats_params), checked */
+    uint32_t version;          /* LGDSP_PARAMS_VERSION */
+    int32_t n_samples;         /* 0 .. LGDSP_WFSTAT_MAX_SAMPLES */
+    int32_t sample_kind;       /* LGDSP_SAMPLE_U16 / _F32 / _F64, converted exactly to double */
+    uint32_t what;             /* LGDSP_WFSTAT_* mask, at least one bit */
+    int32_t reserved0;
+    double t_first_ns, dt_ns;
+    int32_t sat_from, sat_until;     /* saturation window */
+    int32_t ext_from, ext_until;     /* extremestats window */
+    int32_t tail_from, tail_until;   /* tailstats window */
+    int32_t max_from, max_until;     /* get_wvf_maximum window */
+    int64_t sat_low, sat_high;       /* saturation levels, compared with the raw integer samples */
+    double thr_min, thr_max;         /* bounds of thresholdstats / thresholdstats_mad (+-Inf: open) */
+    int32_t im_min_n, im_max_n;      /* IntersectMaximum: max(1, round(mintot/dt)), max(1, round(maxtot/dt)) */
+    int32_t max_triggers;            /* capacity of every trigger list, 1 .. LGDSP_WFSTAT_MAX_TRIGGERS */
+    int32_t reserved1;
+} lgdsp_wfstats_params;
+/* wf: n_events waveforms of `sample_kind` samples, row stride ld_samples (in samples); thresholds: double[n_events], the
+ * IntersectMaximum threshold of every event (read only when it is selected, may be NULL otherwise); rows: see above;
+ * lists: double[n_events][4][max_triggers] = x, x_high, x_tot, max of the triggers, zero-filled behind the last one (written
+ * only when IntersectMaximum is selected, may be NULL otherwise).  Host buffers (chunked copies, blocks until the results are
+ * in rows / lists) / device buffers (asynchronous on the handle's stream). */
+int lgdsp_wfstats_run(lgdsp_handle* h, const lgdsp_wfstats_params* p, const void* wf, const double* thresholds, int64_t n_events,
+                      int64_t ld_samples, double* rows, double* lists);
+int lgdsp_wfstats_run_device(lgdsp_handle* h, const lgdsp_wfstats_params* p, const void* d_wf, const double* d_thresholds,
+                             int64_t n_events, int64_t ld_samples, double* d_rows, double* d_lists);
 
 /* MultiIntersect on a batch of traces of doubles: y[e*ld_samples + i]; x: double[n_events][n_thresholds] (ns);
  * flags: int32[n_events], 1 where the reference's boundary assertion (:85-88) fails (that event's x are NaN) */

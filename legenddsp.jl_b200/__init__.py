@@ -6,6 +6,8 @@ Public surface (mirrors the reference's names, /root/reference/src/LegendDSP.jl:
     dsp_trap/cusp/zac_rt_optimization, dsp_trap/cusp/zac_ft_optimization, dsp_sg_optimization
                                                    src/dsp_filter_optimization.jl:102-441
     dsp_puls, dsp_decay_times                      src/dsp_puls.jl:29, src/dsp_decaytime.jl:11
+    extremestats, saturation, tailstats, get_wvf_maximum, thresholdstats(_mad), IntersectMaximum
+                                                   the per-waveform primitives, broadcast over waveform arrays
 
 All compute happens in the in-tree CUDA library (csrc/ -> liblgdsp_b200.so) behind the C ABI of
 include/lgdsp_b200.h.  Importing this package does not need a GPU; calling a compute function does.
@@ -26,6 +28,7 @@ from .dsp_filter_optimization import (dsp_trap_rt_optimization, dsp_trap_ft_opti
 from .dsp_sipm import (dsp_sipm, dsp_sipm_compressed, sipm_rows, sipm_to_table, resolve_sipm_params, example_sipm_config, SIPM_TABLE,
                        VectorOfVectors, IntersectMaximum, MultiIntersect, thresholdstats, thresholdstats_mad)
 from .dsp_puls import dsp_puls, dsp_puls_compressed, dsp_decay_times, resolve_puls_params, PULS_COLUMNS
+from .stats import extremestats, saturation, tailstats, get_wvf_maximum
 from .codec import EncodedWaveforms, encode_waveforms, decode_data, RADWARE_SIGCOMPRESS, ULEB128_ZIGZAG_DIFF
 from . import synth, sharding, codec
 
@@ -41,6 +44,7 @@ __all__ = [
     "dsp_puls_compressed", "dsp_sipm_compressed", "dsp_sg_optimization_compressed",
     "dsp_sipm", "sipm_rows", "sipm_to_table", "resolve_sipm_params", "example_sipm_config", "SIPM_TABLE", "VectorOfVectors",
     "IntersectMaximum", "MultiIntersect", "thresholdstats", "thresholdstats_mad",
+    "extremestats", "saturation", "tailstats", "get_wvf_maximum",
     "EncodedWaveforms", "encode_waveforms", "decode_data", "RADWARE_SIGCOMPRESS", "ULEB128_ZIGZAG_DIFF", "codec",
     "synth", "sharding", "COLUMNS", "COL", "INT_COLUMNS", "NCOL", "UNITS",
 ]

@@ -153,7 +153,7 @@ SIPM_COL = {name: i for i, name in enumerate(SIPM_COLUMNS)}
 SIPM_NCOL = len(SIPM_COLUMNS)
 SIPM_NLIST, SIPM_NFIELD = 4, 4
 SIPM_MAX_TRIGGERS = 1024
-SAMPLE_U16, SAMPLE_F32 = 2, 4
+SAMPLE_U16, SAMPLE_F32, SAMPLE_F64 = 2, 4, 8
 
 
 class SipmParams(C.Structure):
@@ -191,3 +191,34 @@ class MultiIntersectParams(C.Structure):
 class SynthParams(C.Structure):
     _fields_ = [("seed", C.c_uint64), ("n_samples", C.c_int32), ("mode", C.c_int32),
                 ("noise_sigma", C.c_double), ("tau_samples", C.c_double)]
+
+
+# ---- per-waveform primitives on waveform arrays (include/lgdsp_b200.h: LGDSP_WFSTAT_*, lgdsp_wfstats_params) ----
+WFSTAT_SATURATION = 0x01
+WFSTAT_EXTREMESTATS = 0x02
+WFSTAT_TAILSTATS = 0x04
+WFSTAT_WVF_MAXIMUM = 0x08
+WFSTAT_THRESHOLDSTATS = 0x10
+WFSTAT_THRESHOLDSTATS_MAD = 0x20
+WFSTAT_INTERSECT_MAXIMUM = 0x40
+WFSTAT_ALL = 0x7F
+WFSTAT_COLUMNS = ("sat_low", "sat_high", "sat_max_cons_low", "sat_max_cons_high", "min", "max", "tmin", "tmax",
+                  "tail_mean", "tail_sigma", "tail_tau", "wvf_max", "thr_sigma", "thr_mad", "multiplicity")
+WFSTAT_COL = {name: i for i, name in enumerate(WFSTAT_COLUMNS)}
+WFSTAT_NCOL = len(WFSTAT_COLUMNS)
+WFSTAT_MAX_SAMPLES = 65536
+WFSTAT_MAX_TRIGGERS = 65536
+
+
+class WfstatsParams(C.Structure):
+    _fields_ = [
+        ("struct_size", C.c_uint32), ("version", C.c_uint32),
+        ("n_samples", C.c_int32), ("sample_kind", C.c_int32),
+        ("what", C.c_uint32), ("reserved0", C.c_int32),
+        ("t_first_ns", C.c_double), ("dt_ns", C.c_double),
+        ("sat_from", C.c_int32), ("sat_until", C.c_int32), ("ext_from", C.c_int32), ("ext_until", C.c_int32),
+        ("tail_from", C.c_int32), ("tail_until", C.c_int32), ("max_from", C.c_int32), ("max_until", C.c_int32),
+        ("sat_low", C.c_int64), ("sat_high", C.c_int64),
+        ("thr_min", C.c_double), ("thr_max", C.c_double),
+        ("im_min_n", C.c_int32), ("im_max_n", C.c_int32), ("max_triggers", C.c_int32), ("reserved1", C.c_int32),
+    ]

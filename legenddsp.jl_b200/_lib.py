@@ -77,6 +77,8 @@ def load_library():
     L.lgdsp_thresholdstats.argtypes = [vp, vp, i32, C.c_double, C.c_double, i32, _dp]
     L.lgdsp_intersect_maximum.argtypes = [vp, vp, i32, C.c_double, C.c_double, C.c_double, i32, i32, i32, vp, vp, vp, vp,
                                           C.POINTER(i32)]
+    L.lgdsp_wfstats_run.argtypes = [vp, C.POINTER(_abi.WfstatsParams), vp, vp, i64, i64, vp, vp]
+    L.lgdsp_wfstats_run_device.argtypes = [vp, C.POINTER(_abi.WfstatsParams), vp, vp, i64, i64, vp, vp]
     L.lgdsp_multi_intersect_run.argtypes = [vp, C.POINTER(_abi.MultiIntersectParams), vp, i64, i64, vp, vp]
     L.lgdsp_multi_intersect_run_device.argtypes = [vp, C.POINTER(_abi.MultiIntersectParams), vp, i64, i64, vp, vp]
     L.lgdsp_trap_sweep_run.argtypes = [vp, C.POINTER(_abi.SweepParams), vp, i64, i64, C.POINTER(_abi.TrapVariant), i32, vp]
@@ -101,7 +103,7 @@ EXPORTED_SYMBOLS = (
     "lgdsp_host_unregister", "lgdsp_icpc_run_ext", "lgdsp_icpc_run_ext_device",
     "lgdsp_codec_max_encoded_bytes", "lgdsp_codec_encode_host", "lgdsp_decode_data", "lgdsp_decode_data_device", "lgdsp_icpc_run_encoded", "lgdsp_icpc_compressed_run_encoded",
     "lgdsp_window_stats_run", "lgdsp_window_stats_run_device", "lgdsp_sipm_run", "lgdsp_sipm_run_device",
-    "lgdsp_sipm_list_pointers_device", "lgdsp_sipm_list_gather_device", "lgdsp_thresholdstats", "lgdsp_intersect_maximum", "lgdsp_multi_intersect_run", "lgdsp_multi_intersect_run_device", "lgdsp_icpc_compressed_run", "lgdsp_icpc_compressed_run_device",
+    "lgdsp_sipm_list_pointers_device", "lgdsp_sipm_list_gather_device", "lgdsp_thresholdstats", "lgdsp_intersect_maximum", "lgdsp_wfstats_run", "lgdsp_wfstats_run_device", "lgdsp_multi_intersect_run", "lgdsp_multi_intersect_run_device", "lgdsp_icpc_compressed_run", "lgdsp_icpc_compressed_run_device",
     "lgdsp_trap_sweep_run", "lgdsp_trap_sweep_run_device", "lgdsp_sweep_run", "lgdsp_sweep_run_device",
     "lgdsp_sweep_run_ext", "lgdsp_sweep_run_ext_device",
     "lgdsp_synth_generate_device", "lgdsp_synth_generate_host", "lgdsp_last_kernel_ms",
@@ -289,6 +291,17 @@ class Handle:
                                                       *[C.c_void_p(o.ctypes.data) for o in out], C.byref(n)))
         m = min(n.value, cap)
         return {"x": out[0][:m], "x_high": out[1][:m], "x_tot": out[2][:m], "max": out[3][:m], "multiplicity": n.value}
+
+    def wfstats_run_host(self, params, wf_ptr, thr_ptr, n_events, ld, rows_ptr, lists_ptr):
+        """the per-waveform primitives selected in params.what on host buffers (lgdsp_wfstats_run)"""
+        self._check(self._lib.lgdsp_wfstats_run(self._h, C.byref(params), C.c_void_p(wf_ptr), C.c_void_p(thr_ptr) if thr_ptr else None,
+                                                int(n_events), int(ld), C.c_void_p(rows_ptr),
+                                                C.c_void_p(lists_ptr) if lists_ptr else None))
+
+    def wfstats_run_device(self, params, d_wf_ptr, d_thr_ptr, n_events, ld, d_rows_ptr, d_lists_ptr):
+        self._check(self._lib.lgdsp_wfstats_run_device(self._h, C.byref(params), C.c_void_p(d_wf_ptr),
+                                                       C.c_void_p(d_thr_ptr) if d_thr_ptr else None, int(n_events), int(ld),
+                                                       C.c_void_p(d_rows_ptr), C.c_void_p(d_lists_ptr) if d_lists_ptr else None))
 
     def multi_intersect_host(self, params, y_ptr, n_events, ld, x_ptr, flags_ptr):
         self._check(self._lib.lgdsp_multi_intersect_run(self._h, C.byref(params), C.c_void_p(y_ptr), int(n_events), int(ld),

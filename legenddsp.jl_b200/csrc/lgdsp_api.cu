@@ -45,8 +45,8 @@ struct lgdsp_handle {
     // device slots of the chunked host paths (run_chunked): [buffer][array], the dense rows of one chunk
     void* d_slot[2][LGDSP_HOST_ARRAYS] = {};
     size_t slot_cap[2][LGDSP_HOST_ARRAYS] = {};
-    double* d_prim = nullptr;  // trace in, results out of the single-trace primitives
-    size_t prim_cap = 0;
+    double* d_work = nullptr;  // converted traces of lgdsp_wfstats_run when they are not staged in shared memory
+    size_t work_cap = 0;
     cudaStream_t s_copy = nullptr;
     cudaEvent_t ev_ready[2] = {nullptr, nullptr}, ev_free[2] = {nullptr, nullptr};
     // pinned staging of the host paths (HostIO below): pageable caller memory goes through these double buffers
@@ -209,7 +209,7 @@ void lgdsp_destroy(lgdsp_handle* h)
     if (h->ev_fork) cudaEventDestroy(h->ev_fork);
     cudaFree(h->d_tt); cudaFree(h->d_saux); cudaFree(h->d_scz);
     cudaFree(h->d_dniA); cudaFree(h->d_cusp_g); cudaFree(h->d_zac_g); cudaFree(h->d_sweep_dniA); cudaFree(h->d_vars); cudaFree(h->d_taps);
-    cudaFree(h->d_win); cudaFree(h->d_prim);
+    cudaFree(h->d_win); cudaFree(h->d_work);
     cudaFree(h->d_dniA_w); cudaFree(h->d_cusp_g_w); cudaFree(h->d_zac_g_w);
     for (int i = 0; i < 2; ++i) {
         for (int k = 0; k < LGDSP_HOST_ARRAYS; ++k) cudaFree(h->d_slot[i][k]);
@@ -1657,37 +1657,156 @@ int lgdsp_sipm_list_gather_device(lgdsp_handle* h, const double* d_trig, int64_t
     return LGDSP_OK;
 }
 
-// single-trace primitives (host buffers)
-static int prim_run(lgdsp_handle* h, int mode, const double* y, int n, double a, double b, double t0, double dt, int min_n, int max_n,
-                    int cap, double* out_host, int n_out, int32_t* n_found)
+// ---------------------------------------------------------------------------------------------------
+// per-waveform primitives on waveform arrays (lgdsp_wfstats_run)
+// ---------------------------------------------------------------------------------------------------
+static int wfstats_prepare(lgdsp_handle* h, const lgdsp_wfstats_params* p, WfstatsDev& D, int& bps)
+{
+    if (!p) return fail(h, LGDSP_ERR_INVALID_ARG, "params is NULL");
+    if (p->struct_size != sizeof(lgdsp_wfstats_params) || p->version != LGDSP_PARAMS_VERSION)
+        return fail(h, LGDSP_ERR_INVALID_ARG, "lgdsp_wfstats_params: size/version mismatch (got %u/%u, want %zu/%u)", p->struct_size,
+                    p->version, sizeof(lgdsp_wfstats_params), LGDSP_PARAMS_VERSION);
+    const unsigned what = p->what;
+    if (what == 0 || (what & ~LGDSP_WFSTAT_ALL)) return fail(h, LGDSP_ERR_INVALID_ARG, "what = 0x%x: a non-empty LGDSP_WFSTAT_* mask", what);
+    const int n = p->n_samples;
+    if (n < 0 || n > LGDSP_WFSTAT_MAX_SAMPLES) return fail(h, LGDSP_ERR_UNSUPPORTED, "n_samples = %d: need 0 .. %d", n, LGDSP_WFSTAT_MAX_SAMPLES);
+    const int kind = p->sample_kind;
+    if (kind != LGDSP_SAMPLE_U16 && kind != LGDSP_SAMPLE_F32 && kind != LGDSP_SAMPLE_F64)
+        return fail(h, LGDSP_ERR_UNSUPPORTED, "sample_kind = %d: LGDSP_SAMPLE_U16, _F32 or _F64", kind);
+    // saturation compares raw ADC samples with integer levels (src/saturation.jl; SURVEY.md App. F)
+    if ((what & LGDSP_WFSTAT_SATURATION) && kind != LGDSP_SAMPLE_U16)
+        return fail(h, LGDSP_ERR_UNSUPPORTED, "saturation takes raw UInt16 samples (LGDSP_SAMPLE_U16)");
+    if (!std::isfinite(p->dt_ns) || !std::isfinite(p->t_first_ns)) return fail(h, LGDSP_ERR_INVALID_ARG, "bad time axis");
+    // @assert firstindex(X) <= first(idxs) <= last(idxs) <= lastindex(X)   src/tailstats.jl:23-25
+    const struct { unsigned bit; int from, until; const char* name; } win[4] = {
+        {LGDSP_WFSTAT_SATURATION, p->sat_from, p->sat_until, "saturation"},
+        {LGDSP_WFSTAT_EXTREMESTATS, p->ext_from, p->ext_until, "extremestats"},
+        {LGDSP_WFSTAT_TAILSTATS, p->tail_from, p->tail_until, "tailstats"},
+        {LGDSP_WFSTAT_WVF_MAXIMUM, p->max_from, p->max_until, "get_wvf_maximum"}};
+    for (const auto& w : win)
+        if ((what & w.bit) && !(0 <= w.from && w.from <= w.until && w.until <= n - 1))
+            return fail(h, LGDSP_ERR_INVALID_ARG, "%s window %d:%d outside the waveform (0:%d)", w.name, w.from, w.until, n - 1);
+    const bool im = (what & LGDSP_WFSTAT_INTERSECT_MAXIMUM) != 0;
+    if (im && (p->im_min_n < 1 || p->im_max_n < 1)) return fail(h, LGDSP_ERR_INVALID_ARG, "im_min_n / im_max_n must be >= 1");
+    if (im && (p->max_triggers < 1 || p->max_triggers > LGDSP_WFSTAT_MAX_TRIGGERS))
+        return fail(h, LGDSP_ERR_INVALID_ARG, "max_triggers outside 1..%d", LGDSP_WFSTAT_MAX_TRIGGERS);
+    D = WfstatsDev{};
+    D.n = n; D.kind = kind; D.what = what; D.cap = im ? p->max_triggers : 0;
+    D.t0 = p->t_first_ns; D.dt = p->dt_ns;
+    D.sat_from = p->sat_from; D.sat_until = p->sat_until; D.ext_from = p->ext_from; D.ext_until = p->ext_until;
+    D.tail_from = p->tail_from; D.tail_until = p->tail_until; D.max_from = p->max_from; D.max_until = p->max_until;
+    D.sat_low = p->sat_low; D.sat_high = p->sat_high;
+    D.thr_min = p->thr_min; D.thr_max = p->thr_max;
+    D.im_min_n = p->im_min_n; D.im_max_n = p->im_max_n;
+    CK(wfstats_configure(D, &bps));
+    if (bps < 1) return fail(h, LGDSP_ERR_CUDA, "wfstats kernel does not fit on an SM");
+    return LGDSP_OK;
+}
+
+// wfstats_prepare plus the checks lgdsp_wfstats_run and _run_device share (nothing to do when n_events is 0)
+static int wfstats_check(lgdsp_handle* h, const lgdsp_wfstats_params* p, const void* wf, const double* thresholds, int64_t n_events,
+                         int64_t ld_samples, const double* rows, const double* lists, WfstatsDev& D, int& bps)
 {
     if (!h) return LGDSP_ERR_INVALID_ARG;
     CK(cudaSetDevice(h->device));
-    if (n < 0 || n > 65536) return fail(h, LGDSP_ERR_UNSUPPORTED, "n = %d: single-trace primitives take 0 .. 65536 samples", n);
-    if (n > 0 && !y) return fail(h, LGDSP_ERR_INVALID_ARG, "trace pointer is NULL");
-    // d_prim: the trace, then n_out results and the count
-    const size_t n_in = n > 0 ? (size_t)n : 1;
-    int rc = grow(h, &h->d_prim, &h->prim_cap, (n_in + n_out + 2) * sizeof(double));
+    int rc = wfstats_prepare(h, p, D, bps);
     if (rc) return rc;
-    double* d_out = h->d_prim + n_in;
-    int* d_cnt = reinterpret_cast<int*>(d_out + n_out);
-    if (n > 0) CK(cudaMemcpyAsync(h->d_prim, y, (size_t)n * sizeof(double), cudaMemcpyHostToDevice, h->stream));
-    CK(cudaMemsetAsync(d_cnt, 0, sizeof(int), h->stream));
-    sipm_prim_launch(mode, h->d_prim, n, a, b, t0, dt, min_n, max_n, cap, d_out, d_cnt, h->stream);
-    CK(cudaGetLastError());
-    h->launches += 1;
-    CK(cudaMemcpyAsync(out_host, d_out, (size_t)n_out * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
-    int cnt = 0;
-    CK(cudaMemcpyAsync(&cnt, d_cnt, sizeof(int), cudaMemcpyDeviceToHost, h->stream));
-    CK(cudaStreamSynchronize(h->stream));
-    if (n_found) *n_found = cnt;
+    const bool im = (D.what & LGDSP_WFSTAT_INTERSECT_MAXIMUM) != 0;
+    if (n_events < 0) return fail(h, LGDSP_ERR_INVALID_ARG, "n_events < 0");
+    if (n_events == 0) return LGDSP_OK;
+    if (ld_samples < D.n) return fail(h, LGDSP_ERR_INVALID_ARG, "ld_samples (%lld) < n_samples (%d)", (long long)ld_samples, D.n);
+    if (im && !thresholds) return fail(h, LGDSP_ERR_INVALID_ARG, "IntersectMaximum needs the per-event thresholds (NULL pointer)");
+    if ((D.n > 0 && !wf) || !rows || (im && !lists)) return fail(h, LGDSP_ERR_INVALID_ARG, "NULL pointer");
     return LGDSP_OK;
+}
+
+// persistent grid; when thresholdstats_mad needs the converted trace in global memory (long non-double traces) the grid is also
+// limited so that those per-CTA copies take at most 256 MiB (at least one CTA per SM)
+static int wfstats_grid(lgdsp_handle* h, const WfstatsDev& D, int bps, int64_t n_events, int& grid)
+{
+    long long g = (long long)h->sm_count * bps;
+    const long long per_cta = wfstats_work_doubles(D);
+    if (per_cta > 0) {
+        g = std::min(g, std::max((long long)h->sm_count, (256ll << 20) / (per_cta * (long long)sizeof(double))));
+        const int rc = grow(h, &h->d_work, &h->work_cap, (size_t)g * per_cta * sizeof(double));
+        if (rc) return rc;
+    }
+    grid = (int)std::min<long long>(g, n_events);
+    return LGDSP_OK;
+}
+
+int lgdsp_wfstats_run_device(lgdsp_handle* h, const lgdsp_wfstats_params* p, const void* d_wf, const double* d_thresholds,
+                             int64_t n_events, int64_t ld_samples, double* d_rows, double* d_lists)
+{
+    WfstatsDev D;
+    int bps = 0, grid = 0;
+    int rc = wfstats_check(h, p, d_wf, d_thresholds, n_events, ld_samples, d_rows, d_lists, D, bps);
+    if (rc || n_events == 0) return rc;
+    rc = wfstats_grid(h, D, bps, n_events, grid);
+    if (rc) return rc;
+    CK(cudaEventRecord(h->ev0, h->stream));
+    wfstats_launch(D, d_wf, d_thresholds, n_events, ld_samples, d_rows, d_lists, h->d_work, grid, h->stream);
+    CK(cudaGetLastError());
+    CK(cudaEventRecord(h->ev1, h->stream));
+    h->timed = true;
+    h->launches += 1;
+    return LGDSP_OK;
+}
+
+int lgdsp_wfstats_run(lgdsp_handle* h, const lgdsp_wfstats_params* p, const void* wf, const double* thresholds, int64_t n_events,
+                      int64_t ld_samples, double* rows, double* lists)
+{
+    WfstatsDev D;
+    int bps = 0, grid = 0;
+    int rc = wfstats_check(h, p, wf, thresholds, n_events, ld_samples, rows, lists, D, bps);
+    if (rc || n_events == 0) return rc;
+    rc = wfstats_grid(h, D, bps, n_events, grid);
+    if (rc) return rc;
+    const bool im = (D.what & LGDSP_WFSTAT_INTERSECT_MAXIMUM) != 0;
+    const size_t sb = (size_t)D.kind;   // bytes per sample
+    const size_t rw = LGDSP_WFSTAT_NCOL * sizeof(double), lw = (size_t)4 * D.cap * sizeof(double);
+    // events per chunk: at most 8192, and few enough that one chunk's device rows (samples, threshold, row, lists) take at most
+    // 64 MiB -- the lists alone are 2 MiB per event at max_triggers = 65536; the double-buffered slots and the pinned staging
+    // of pageable memory stay bounded the same way
+    const size_t per_event = (size_t)D.n * sb + rw + (im ? sizeof(double) + lw : 0);
+    const int64_t chunk = std::max<int64_t>(1, std::min<int64_t>(8192, (int64_t)((64ull << 20) / per_event)));
+    return run_chunked(h, n_events, chunk,
+                       {host_array(D.n > 0 ? wf : nullptr, (size_t)ld_samples * sb, (size_t)D.n * sb),
+                        host_array(im ? thresholds : nullptr, sizeof(double), sizeof(double))},
+                       {host_array(rows, rw, rw), host_array(im ? lists : nullptr, lw, lw)}, [&](int64_t ne, void* const* d) {
+                           wfstats_launch(D, d[0], static_cast<const double*>(d[1]), ne, D.n, static_cast<double*>(d[2]),
+                                          static_cast<double*>(d[3]), h->d_work, (int)std::min<int64_t>(grid, ne), h->stream);
+                           CK(cudaGetLastError());
+                           h->launches += 1;
+                           return (int)LGDSP_OK;
+                       });
+}
+
+// the single-trace primitives: n_events = 1 calls of lgdsp_wfstats_run on a trace of doubles
+static lgdsp_wfstats_params single_trace_params(int32_t n, unsigned what)
+{
+    lgdsp_wfstats_params p;
+    memset(&p, 0, sizeof(p));
+    p.struct_size = sizeof(p);
+    p.version = LGDSP_PARAMS_VERSION;
+    p.n_samples = n;
+    p.sample_kind = LGDSP_SAMPLE_F64;
+    p.what = what;
+    p.dt_ns = 1.0;
+    return p;
 }
 
 int lgdsp_thresholdstats(lgdsp_handle* h, const double* y, int32_t n, double min, double max, int32_t mad, double* out)
 {
     if (!out) return h ? fail(h, LGDSP_ERR_INVALID_ARG, "output pointer is NULL") : LGDSP_ERR_INVALID_ARG;
-    return prim_run(h, mad ? 1 : 0, y, n, min, max, 0.0, 1.0, 1, 1, 1, out, 1, nullptr);
+    lgdsp_wfstats_params p = single_trace_params(n, mad ? LGDSP_WFSTAT_THRESHOLDSTATS_MAD : LGDSP_WFSTAT_THRESHOLDSTATS);
+    p.thr_min = min;
+    p.thr_max = max;
+    double row[LGDSP_WFSTAT_NCOL];
+    const int rc = lgdsp_wfstats_run(h, &p, y, nullptr, 1, n, row, nullptr);
+    if (rc) return rc;
+    *out = row[mad ? LGDSP_WFSTAT_thr_mad : LGDSP_WFSTAT_thr_sigma];
+    return LGDSP_OK;
 }
 
 int lgdsp_intersect_maximum(lgdsp_handle* h, const double* y, int32_t n, double t_first_ns, double dt_ns, double threshold,
@@ -1696,15 +1815,24 @@ int lgdsp_intersect_maximum(lgdsp_handle* h, const double* y, int32_t n, double 
 {
     if (!h) return LGDSP_ERR_INVALID_ARG;
     if (!x || !x_high || !x_tot || !max || !n_found) return fail(h, LGDSP_ERR_INVALID_ARG, "output pointer is NULL");
-    if (min_n < 1 || max_n < 1 || max_triggers < 1 || max_triggers > 65536) return fail(h, LGDSP_ERR_INVALID_ARG, "min_n / max_n / max_triggers out of range");
+    lgdsp_wfstats_params p = single_trace_params(n, LGDSP_WFSTAT_INTERSECT_MAXIMUM);
+    p.t_first_ns = t_first_ns;
+    p.dt_ns = dt_ns;
+    p.im_min_n = min_n;
+    p.im_max_n = max_n;
+    p.max_triggers = max_triggers;
+    if (max_triggers < 1 || max_triggers > LGDSP_WFSTAT_MAX_TRIGGERS)
+        return fail(h, LGDSP_ERR_INVALID_ARG, "max_triggers outside 1..%d", LGDSP_WFSTAT_MAX_TRIGGERS);
     std::vector<double> buf((size_t)4 * max_triggers);
-    int rc = prim_run(h, 2, y, n, threshold, 0.0, t_first_ns, dt_ns, min_n, max_n, max_triggers, buf.data(), 4 * max_triggers, n_found);
+    double row[LGDSP_WFSTAT_NCOL];
+    const int rc = lgdsp_wfstats_run(h, &p, y, &threshold, 1, n, row, buf.data());
     if (rc) return rc;
     const size_t c = (size_t)max_triggers;
     memcpy(x, buf.data(), c * sizeof(double));
     memcpy(x_high, buf.data() + c, c * sizeof(double));
     memcpy(x_tot, buf.data() + 2 * c, c * sizeof(double));
     memcpy(max, buf.data() + 3 * c, c * sizeof(double));
+    *n_found = (int32_t)row[LGDSP_WFSTAT_multiplicity];
     return LGDSP_OK;
 }
 

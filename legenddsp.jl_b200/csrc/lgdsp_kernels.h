@@ -94,9 +94,25 @@ struct SipmDev {
 cudaError_t sipm_configure(int n, int sample_kind, int* max_blocks_per_sm);
 void sipm_launch(const SipmDev& P, const void* d_wf, long long n_events, long long ld, double* d_rows, double* d_trig, int grid,
                  cudaStream_t stream);
-// mode 0: thresholdstats, 1: thresholdstats_mad (a, b = bounds), 2: IntersectMaximum (a = threshold)
-void sipm_prim_launch(int mode, const double* d_y, int n, double a, double b, double t0, double dt, int min_n, int max_n, int cap,
-                      double* d_out, int* d_n_found, cudaStream_t stream);
+
+// ---- per-waveform primitives on waveform arrays (lgdsp_sipm.cu, lgdsp_wfstats_run) ----
+struct WfstatsDev {
+    int n, kind;
+    unsigned what;
+    int cap;
+    double t0, dt;
+    int sat_from, sat_until, ext_from, ext_until, tail_from, tail_until, max_from, max_until;
+    long long sat_low, sat_high;
+    double thr_min, thr_max;
+    int im_min_n, im_max_n;
+};
+// shared memory per CTA, whether the trace is staged there, and CTAs per SM of the kernel for (n, kind, what)
+cudaError_t wfstats_configure(const WfstatsDev& P, int* max_blocks_per_sm);
+// d_work: grid * n doubles, the converted trace of every CTA when it is not staged in shared memory and thresholdstats_mad is
+// selected on non-double samples (wfstats_work_doubles(P) > 0), else unused
+long long wfstats_work_doubles(const WfstatsDev& P);
+void wfstats_launch(const WfstatsDev& P, const void* d_wf, const double* d_thr, long long n_events, long long ld, double* d_rows,
+                    double* d_lists, double* d_work, int grid, cudaStream_t stream);
 
 // trigger lists -> flat data + element pointers on the device
 void sipm_count_scan_launch(const double* d_rows, long long n_events, int list, int cap, long long* d_elem_ptr, cudaStream_t stream);

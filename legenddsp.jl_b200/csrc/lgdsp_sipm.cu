@@ -3,6 +3,8 @@
 // device routines:
 //   thresholdstats / thresholdstats_mad   /root/reference/src/thresholdstats.jl:19-41, 61-71
 //   IntersectMaximum                      /root/reference/src/intersect_maximum.jl:24-119
+// The same routines, together with saturation, extremestats, tailstats and get_wvf_maximum, serve wfstats_kernel: the
+// per-waveform primitives on whole waveform arrays (lgdsp_wfstats_run).
 //
 // Medians (thresholdstats_mad needs two per call, the chain eight per waveform) are exact order statistics found by
 // value-range refinement: a 2048-bin LINEAR histogram between the current minimum and maximum (bin index is a monotone
@@ -17,6 +19,7 @@
 #include <math_constants.h>
 
 #include <cstdint>
+#include <type_traits>
 
 #include "../../include/lgdsp_b200.h"
 #include "lgdsp_kernels.h"
@@ -30,7 +33,6 @@ constexpr unsigned FULLM = 0xffffffffu;
 constexpr int NBIN = 2048;         // histogram bins of one refinement level
 constexpr int BPT = NBIN / SNT;    // bins per thread in the rank search
 constexpr int CANDCAP = 256;       // candidates ranked by brute force
-constexpr int MAXWORDS = 2048 + 1; // mask words of the single-trace entry (n <= 65536)
 
 struct Scratch {
     unsigned hist[NBIN];
@@ -126,7 +128,7 @@ __device__ __forceinline__ int block_exscan(int v, int& total, Scratch& S)
 // exact order statistics.  The population is described by data, not by a functor, so that ONE copy of the selection code
 // serves all eight medians of the chain (instruction-cache footprint): sample i has the raw value y = sgn * tr[i], takes
 // part if mn <= y <= mx, and enters with the value y (mode 0) or |y - med| (mode 1).
-// SH: the trace lives in shared memory (LDS) or in global memory (single-trace entry).
+// SH: the trace lives in shared memory (LDS) or in global memory (lgdsp_wfstats_run on traces longer than LGDSP_MAX_SAMPLES).
 // ---------------------------------------------------------------------------------------------------
 struct Sel {
     const double* tr;
@@ -429,13 +431,14 @@ __device__ void block_cumsum(Src src, double* dst, int n, int chs, Scratch& S)
     __syncthreads();
 }
 
-// signalstats [RDDSP] on trace[from..until], X_i = t0 + i*dt: mean, sigma, slope, offset
-__device__ void block_signalstats(const double* tr, int from, int until, double t0, double dt, Scratch& S, double out[4])
+// signalstats [RDDSP] on src(i), i in [from, until], X_i = t0 + i*dt: mean, sigma, slope, offset
+template <class Src>
+__device__ void block_signalstats(Src src, int from, int until, double t0, double dt, Scratch& S, double out[4])
 {
     double s[4] = {0.0, 0.0, 0.0, 0.0};   // sum Y, sum Y^2, sum X Y, (unused)
     double sx = 0.0, sxx = 0.0;
     for (int i = from + threadIdx.x; i <= until; i += SNT) {
-        const double x = time_at(i, t0, dt), y = tr[i];
+        const double x = time_at(i, t0, dt), y = src(i);
         s[0] += y; s[1] = fma(y, y, s[1]); s[2] = fma(x, y, s[2]);
         sx += x; sxx = fma(x, x, sxx);
     }
@@ -478,6 +481,103 @@ __device__ void block_extremestats(Src src, int from, int until, Scratch& S, dou
         if (b > vmax || (b == vmax && ib < imax)) { vmax = b; imax = ib; }
     }
     __syncthreads();
+}
+
+// Runs of a predicate over a range of samples: count, length of the leading / trailing run, longest run, whole range set.
+// Ranges are joined in order (a then b), the empty range (full, all 0) is the identity.
+struct Runs {
+    int cnt, pre, suf, best, full;
+};
+__device__ __forceinline__ void runs_cat(Runs& a, const Runs& b)
+{
+    a.best = max(max(a.best, b.best), a.suf + b.pre);
+    a.pre = a.full ? a.pre + b.pre : a.pre;
+    a.suf = b.full ? a.suf + b.suf : b.suf;
+    a.full &= b.full;
+    a.cnt += b.cnt;
+}
+__device__ __forceinline__ void runs_step(Runs& r, bool on)
+{
+    r.cnt += on;
+    if (on) { ++r.suf; return; }
+    if (r.full) { r.pre = r.suf; r.full = 0; }
+    r.best = max(r.best, r.suf);
+    r.suf = 0;
+}
+__device__ __forceinline__ Runs runs_shfl_down(const Runs& r, int o)
+{
+    return Runs{__shfl_down_sync(FULLM, r.cnt, o), __shfl_down_sync(FULLM, r.pre, o), __shfl_down_sync(FULLM, r.suf, o),
+                __shfl_down_sync(FULLM, r.best, o), __shfl_down_sync(FULLM, r.full, o)};
+}
+
+// _saturation_impl  src/saturation.jl:28-65 on src(i), i in [from, until]: the number of samples == low / == high and the
+// longest runs of them (a sample equal to low ends a high run and vice versa; trailing runs count).  Every thread walks a
+// contiguous chunk (odd length: conflict-free on a staged trace), the chunk summaries are joined in thread order.
+// out: n_low, n_high, max_cons_low, max_cons_high (valid in thread 0)
+template <class Src>
+__device__ void block_saturation(Src src, int from, int until, double low, double high, Scratch& S, double out[4])
+{
+    const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
+    const int chs = ((until - from + SNT) / SNT) | 1;
+    const int i0 = from + tid * chs, i1 = min(until + 1, i0 + chs);
+    Runs rl{0, 0, 0, 0, 1}, rh{0, 0, 0, 0, 1};
+    for (int i = i0; i < i1; ++i) {
+        const double v = src(i);
+        const bool is_low = v == low;
+        runs_step(rl, is_low);
+        runs_step(rh, !is_low && v == high);
+    }
+    if (rl.full) rl.pre = rl.suf;
+    if (rh.full) rh.pre = rh.suf;
+    rl.best = max(rl.best, rl.suf);
+    rh.best = max(rh.best, rh.suf);
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const Runs bl = runs_shfl_down(rl, o), bh = runs_shfl_down(rh, o);
+        if ((lane & (2 * o - 1)) == 0) { runs_cat(rl, bl); runs_cat(rh, bh); }
+    }
+    Runs* wr = reinterpret_cast<Runs*>(S.hist);   // [2][SNW]
+    if (lane == 0) { wr[wid] = rl; wr[SNW + wid] = rh; }
+    __syncthreads();
+    if (tid == 0) {
+        Runs a = wr[0], b = wr[SNW];
+        for (int w = 1; w < SNW; ++w) { runs_cat(a, wr[w]); runs_cat(b, wr[SNW + w]); }
+        out[0] = a.cnt; out[1] = b.cnt; out[2] = a.best; out[3] = b.best;
+    }
+    __syncthreads();
+}
+
+// _tailstats_impl  src/tailstats.jl:22-72 on src(i), i in [from, until]: any sample <= 0 gives (0, 0, 0) (:27-33), else the
+// straight-line fit of log(y) over the sample time; out: mean, sigma, tau = -1/slope (unguarded, as the reference)
+template <class Src>
+__device__ void block_tailstats(Src src, int from, int until, double t0, double dt, Scratch& S, double out[3])
+{
+    bool nonpos = false;
+    for (int i = from + threadIdx.x; i <= until; i += SNT) nonpos |= src(i) <= 0.0;
+    if (__syncthreads_or(nonpos)) { out[0] = 0.0; out[1] = 0.0; out[2] = 0.0; return; }
+    double st[4];
+    block_signalstats([&](int i) { return log(src(i)); }, from, until, t0, dt, S, st);
+    out[0] = st[0]; out[1] = st[1]; out[2] = -1.0 / st[2];
+}
+
+// extrema3points  src/interpolation.jl:8-10, rounded operation by operation (no contraction): the oracle's result bit for bit
+__device__ __forceinline__ double extrema3points_rn(double y1, double y2, double y3)
+{
+    const double a = __dadd_rn(__dsub_rn(y3, __dmul_rn(4.0, y2)), __dmul_rn(3.0, y1));
+    const double d = __dmul_rn(8.0, __dadd_rn(__dsub_rn(y3, __dmul_rn(2.0, y2)), y1));
+    return __dsub_rn(y1, __ddiv_rn(__dmul_rn(a, a), d));
+}
+
+// _get_wvf_maximum_impl  src/interpolation.jl:30-46 on src(i), i in [from, until]: the first maximum, refined by the parabola
+// through its neighbours only when it lies strictly inside the WINDOW
+template <class Src>
+__device__ double block_wvf_maximum(Src src, int from, int until, Scratch& S)
+{
+    double vmin, vmax;
+    int imin, imax;
+    block_extremestats(src, from, until, S, vmin, imin, vmax, imax);
+    if (imax > from && imax < until) return extrema3points_rn(src(imax - 1), vmax, src(imax + 1));
+    return vmax;
 }
 
 // ==================================================================================================
@@ -546,9 +646,9 @@ __global__ void __launch_bounds__(SNT, 2) sipm_kernel(const __grid_constant__ Si
             int until = (int)rint((stop - t_sg) / P.dt);
             until = min(until, n_sg - 1);
             double st[4];
-            block_signalstats(bufB, 0, until, t_sg, P.dt, S, st);
+            block_signalstats([&](int i) { return bufB[i]; }, 0, until, t_sg, P.dt, S, st);
             if (tid == 0) { row[LGDSP_SIPM_blmean] = st[0]; row[LGDSP_SIPM_blsigma] = st[1]; row[LGDSP_SIPM_blslope] = st[2]; row[LGDSP_SIPM_bloffset] = st[3]; }
-            block_signalstats(bufB, 0, n_sg - 1, t_sg, P.dt, S, st);
+            block_signalstats([&](int i) { return bufB[i]; }, 0, n_sg - 1, t_sg, P.dt, S, st);
             if (tid == 0) { row[LGDSP_SIPM_wfmean] = st[0]; row[LGDSP_SIPM_wfsigma] = st[1]; row[LGDSP_SIPM_wfslope] = st[2]; row[LGDSP_SIPM_wfoffset] = st[3]; }
         }
         // :118-121 discharges: flipped integrated waveform
@@ -587,24 +687,141 @@ __global__ void __launch_bounds__(SNT, 2) sipm_kernel(const __grid_constant__ Si
     }
 }
 
-// the primitives on one trace of doubles in global memory (tests, small jobs): mode 0 thresholdstats, 1 thresholdstats_mad,
-// 2 IntersectMaximum
-__global__ void __launch_bounds__(SNT) sipm_prim_kernel(int mode, const double* __restrict__ y, int n, double a, double b, double t0, double dt,
-                                                        int min_n, int max_n, int cap, double* __restrict__ out, int* __restrict__ n_found)
+// ==================================================================================================
+// The per-waveform primitives on a batch (lgdsp_wfstats_run): one CTA per waveform, persistent grid; every primitive selected
+// in P.what runs on the same copy of the trace.  SH: the trace is staged once as doubles in shared memory (n <=
+// LGDSP_MAX_SAMPLES); otherwise every primitive reads the samples from global memory, and thresholdstats_mad on non-double
+// samples first converts the trace into the CTA's slice of `work`.
+// Dynamic shared memory: Scratch | double trace[n, even] (SH) | uint16 bin of every sample (SH, MAD) | mask words (IM).
+// ==================================================================================================
+__host__ __device__ constexpr size_t up16(size_t v) { return (v + 15) & ~size_t(15); }
+
+__host__ __device__ inline size_t wfstats_smem_bytes(int n, unsigned what, bool sh)
 {
-    __shared__ Scratch S;
-    __shared__ unsigned mask[MAXWORDS];
-    auto val = [&](int i) { return y[i]; };
-    if (mode == 0) {
-        const double r = block_thresholdstats(val, n, a, b, S);
-        if (threadIdx.x == 0) out[0] = r;
-    } else if (mode == 1) {
-        const double r = block_thresholdstats_mad<false>(y, 1.0, n, a, b, nullptr, S);
-        if (threadIdx.x == 0) out[0] = r;
-    } else {
-        const int c = block_intersect_maximum(val, n, t0, dt, a, min_n, max_n, cap, out, mask, S, nullptr);
-        if (threadIdx.x == 0) *n_found = c;
+    size_t b = up16(sizeof(Scratch));
+    if (sh) {
+        b += up16((size_t)n * sizeof(double));
+        if (what & LGDSP_WFSTAT_THRESHOLDSTATS_MAD) b += up16((size_t)n * sizeof(unsigned short));
     }
+    if (what & LGDSP_WFSTAT_INTERSECT_MAXIMUM) b += (size_t)(((n + 31) >> 5) + 1) * sizeof(unsigned);
+    return b;
+}
+
+template <typename SAMPLE, bool SH>
+__global__ void __launch_bounds__(SNT) wfstats_kernel(const __grid_constant__ WfstatsDev P, const SAMPLE* __restrict__ wf,
+                                                      const double* __restrict__ thr, long long n_events, long long ld,
+                                                      double* __restrict__ rows, double* __restrict__ lists, double* __restrict__ work)
+{
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    Scratch& S = *reinterpret_cast<Scratch*>(smem_raw);
+    const int n = P.n, tid = threadIdx.x;
+    const unsigned what = P.what;
+    unsigned char* p = smem_raw + up16(sizeof(Scratch));
+    double* buf = reinterpret_cast<double*>(p);
+    unsigned short* binbuf = nullptr;
+    if (SH) {
+        p += up16((size_t)n * sizeof(double));
+        if (what & LGDSP_WFSTAT_THRESHOLDSTATS_MAD) { binbuf = reinterpret_cast<unsigned short*>(p); p += up16((size_t)n * sizeof(unsigned short)); }
+    }
+    unsigned* mask = reinterpret_cast<unsigned*>(p);
+
+    for (long long e = blockIdx.x; e < n_events; e += gridDim.x) {
+        const SAMPLE* x = wf + e * ld;
+        double* row = rows + e * LGDSP_WFSTAT_NCOL;
+        if (SH) {
+            for (int i = tid; i < n; i += SNT) buf[i] = (double)x[i];
+            __syncthreads();
+        }
+        auto val = [&](int i) -> double { return SH ? buf[i] : (double)x[i]; };
+        if (what & LGDSP_WFSTAT_SATURATION) {
+            double o[4];
+            block_saturation(val, P.sat_from, P.sat_until, (double)P.sat_low, (double)P.sat_high, S, o);
+            if (tid == 0) {
+                row[LGDSP_WFSTAT_sat_low] = o[0]; row[LGDSP_WFSTAT_sat_high] = o[1];
+                row[LGDSP_WFSTAT_sat_max_cons_low] = o[2]; row[LGDSP_WFSTAT_sat_max_cons_high] = o[3];
+            }
+        } else if (tid == 0) {
+            row[LGDSP_WFSTAT_sat_low] = 0.0; row[LGDSP_WFSTAT_sat_high] = 0.0;
+            row[LGDSP_WFSTAT_sat_max_cons_low] = 0.0; row[LGDSP_WFSTAT_sat_max_cons_high] = 0.0;
+        }
+        if (what & LGDSP_WFSTAT_EXTREMESTATS) {
+            double vmin, vmax;
+            int imin, imax;
+            block_extremestats(val, P.ext_from, P.ext_until, S, vmin, imin, vmax, imax);
+            if (tid == 0) {
+                row[LGDSP_WFSTAT_min] = vmin; row[LGDSP_WFSTAT_max] = vmax;
+                row[LGDSP_WFSTAT_tmin] = time_at(imin, P.t0, P.dt); row[LGDSP_WFSTAT_tmax] = time_at(imax, P.t0, P.dt);
+            }
+        } else if (tid == 0) {
+            row[LGDSP_WFSTAT_min] = 0.0; row[LGDSP_WFSTAT_max] = 0.0; row[LGDSP_WFSTAT_tmin] = 0.0; row[LGDSP_WFSTAT_tmax] = 0.0;
+        }
+        {
+            double o[3] = {0.0, 0.0, 0.0};
+            if (what & LGDSP_WFSTAT_TAILSTATS) block_tailstats(val, P.tail_from, P.tail_until, P.t0, P.dt, S, o);
+            if (tid == 0) { row[LGDSP_WFSTAT_tail_mean] = o[0]; row[LGDSP_WFSTAT_tail_sigma] = o[1]; row[LGDSP_WFSTAT_tail_tau] = o[2]; }
+        }
+        {
+            const double m = (what & LGDSP_WFSTAT_WVF_MAXIMUM) ? block_wvf_maximum(val, P.max_from, P.max_until, S) : 0.0;
+            if (tid == 0) row[LGDSP_WFSTAT_wvf_max] = m;
+        }
+        {
+            const double s = (what & LGDSP_WFSTAT_THRESHOLDSTATS) ? block_thresholdstats(val, n, P.thr_min, P.thr_max, S) : 0.0;
+            if (tid == 0) row[LGDSP_WFSTAT_thr_sigma] = s;
+        }
+        {
+            double mad = 0.0;
+            if (what & LGDSP_WFSTAT_THRESHOLDSTATS_MAD) {
+                if (SH) {
+                    mad = block_thresholdstats_mad<true>(buf, 1.0, n, P.thr_min, P.thr_max, binbuf, S);
+                } else if constexpr (std::is_same<SAMPLE, double>::value) {
+                    mad = block_thresholdstats_mad<false>(x, 1.0, n, P.thr_min, P.thr_max, nullptr, S);
+                } else {
+                    double* w = work + (size_t)blockIdx.x * n;
+                    for (int i = tid; i < n; i += SNT) w[i] = (double)x[i];
+                    __syncthreads();
+                    mad = block_thresholdstats_mad<false>(w, 1.0, n, P.thr_min, P.thr_max, nullptr, S);
+                }
+            }
+            if (tid == 0) row[LGDSP_WFSTAT_thr_mad] = mad;
+        }
+        {
+            int mult = 0;
+            if (what & LGDSP_WFSTAT_INTERSECT_MAXIMUM)
+                mult = block_intersect_maximum(val, n, P.t0, P.dt, thr[e], P.im_min_n, P.im_max_n, P.cap,
+                                               lists + (size_t)e * 4 * P.cap, mask, S, nullptr);
+            if (tid == 0) row[LGDSP_WFSTAT_multiplicity] = (double)mult;
+        }
+        __syncthreads();
+    }
+}
+
+template <typename SAMPLE, bool SH>
+cudaError_t wfstats_configure_one(size_t bytes, int* bps)
+{
+    cudaError_t err = cudaFuncSetAttribute(wfstats_kernel<SAMPLE, SH>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+    if (err != cudaSuccess) return err;
+    return cudaOccupancyMaxActiveBlocksPerMultiprocessor(bps, wfstats_kernel<SAMPLE, SH>, SNT, bytes);
+}
+
+template <typename SAMPLE>
+cudaError_t wfstats_configure_kind(const WfstatsDev& P, int* bps)
+{
+    const bool sh = P.n <= LGDSP_MAX_SAMPLES;
+    const size_t bytes = wfstats_smem_bytes(P.n, P.what, sh);
+    return sh ? wfstats_configure_one<SAMPLE, true>(bytes, bps) : wfstats_configure_one<SAMPLE, false>(bytes, bps);
+}
+
+template <typename SAMPLE>
+void wfstats_launch_kind(const WfstatsDev& P, const void* d_wf, const double* d_thr, long long n_events, long long ld, double* d_rows,
+                         double* d_lists, double* d_work, int grid, cudaStream_t stream)
+{
+    const bool sh = P.n <= LGDSP_MAX_SAMPLES;
+    const size_t bytes = wfstats_smem_bytes(P.n, P.what, sh);
+    const SAMPLE* wf = static_cast<const SAMPLE*>(d_wf);
+    if (sh)
+        wfstats_kernel<SAMPLE, true><<<grid, SNT, bytes, stream>>>(P, wf, d_thr, n_events, ld, d_rows, d_lists, d_work);
+    else
+        wfstats_kernel<SAMPLE, false><<<grid, SNT, bytes, stream>>>(P, wf, d_thr, n_events, ld, d_rows, d_lists, d_work);
 }
 
 // ==================================================================================================
@@ -854,10 +1071,25 @@ void sipm_launch(const SipmDev& P, const void* d_wf, long long n_events, long lo
         sipm_kernel<uint16_t><<<grid, SNT, bytes, stream>>>(P, static_cast<const uint16_t*>(d_wf), n_events, ld, d_rows, d_trig);
 }
 
-void sipm_prim_launch(int mode, const double* d_y, int n, double a, double b, double t0, double dt, int min_n, int max_n, int cap,
-                      double* d_out, int* d_n_found, cudaStream_t stream)
+cudaError_t wfstats_configure(const WfstatsDev& P, int* max_blocks_per_sm)
 {
-    sipm_prim_kernel<<<1, SNT, 0, stream>>>(mode, d_y, n, a, b, t0, dt, min_n, max_n, cap, d_out, d_n_found);
+    if (P.kind == LGDSP_SAMPLE_F64) return wfstats_configure_kind<double>(P, max_blocks_per_sm);
+    if (P.kind == LGDSP_SAMPLE_F32) return wfstats_configure_kind<float>(P, max_blocks_per_sm);
+    return wfstats_configure_kind<uint16_t>(P, max_blocks_per_sm);
+}
+
+long long wfstats_work_doubles(const WfstatsDev& P)
+{
+    const bool sh = P.n <= LGDSP_MAX_SAMPLES;
+    return (!sh && (P.what & LGDSP_WFSTAT_THRESHOLDSTATS_MAD) && P.kind != LGDSP_SAMPLE_F64) ? P.n : 0;
+}
+
+void wfstats_launch(const WfstatsDev& P, const void* d_wf, const double* d_thr, long long n_events, long long ld, double* d_rows,
+                    double* d_lists, double* d_work, int grid, cudaStream_t stream)
+{
+    if (P.kind == LGDSP_SAMPLE_F64) wfstats_launch_kind<double>(P, d_wf, d_thr, n_events, ld, d_rows, d_lists, d_work, grid, stream);
+    else if (P.kind == LGDSP_SAMPLE_F32) wfstats_launch_kind<float>(P, d_wf, d_thr, n_events, ld, d_rows, d_lists, d_work, grid, stream);
+    else wfstats_launch_kind<uint16_t>(P, d_wf, d_thr, n_events, ld, d_rows, d_lists, d_work, grid, stream);
 }
 
 void sipm_count_scan_launch(const double* d_rows, long long n_events, int list, int cap, long long* d_elem_ptr, cudaStream_t stream)

@@ -15,6 +15,7 @@ from . import _abi
 from ._lib import Handle
 from .config import (Q, RddspPolicy, DEFAULT_POLICY, LibBuilders, ns, us, julia_round, _ratio, _fill_sg, _trap, _min_n)
 from .dsp_icpc import RDWaveforms, _as_waveforms, get_handle
+from .stats import wf_samples, wfstats_params, wfstats_rows
 
 
 def example_sipm_config() -> Dict[str, Any]:
@@ -184,35 +185,72 @@ def dsp_sipm_compressed(data: Mapping[str, Any], config: Mapping[str, Any], pars
     return dsp_sipm(d, config, pars_optimization, **kw)
 
 
-# ---- the in-tree primitives on single traces (GPU, through the C ABI) ----
-def thresholdstats(signal, min: float = -np.inf, max: float = np.inf, *, device: int = 0, handle: Optional[Handle] = None) -> float:
-    """standard deviation of the samples inside [min, max]  (src/thresholdstats.jl:19-41)"""
+# ---- the in-tree primitives on single traces or, for a 2-D signal [n_events, n_samples], on every row (GPU, through the C ABI) ----
+def _thresholdstats_rows(signal, mn, mx, what, col, device, handle):
+    sig, kind, _ = wf_samples(signal)
+    P = wfstats_params(sig.shape[1], kind, what, ns(0.0), ns(1.0))
+    P.thr_min, P.thr_max = float(mn), float(mx)
+    return wfstats_rows(sig, P, device=device, handle=handle)[:, _abi.WFSTAT_COL[col]]
+
+
+def thresholdstats(signal, min: float = -np.inf, max: float = np.inf, *, device: int = 0, handle: Optional[Handle] = None):
+    """standard deviation of the samples inside [min, max]  (src/thresholdstats.jl:19-41); one value per row of a 2-D signal"""
+    if np.ndim(signal) == 2:
+        return _thresholdstats_rows(signal, min, max, _abi.WFSTAT_THRESHOLDSTATS, "thr_sigma", device, handle)
     return (handle or get_handle(device)).thresholdstats(np.ascontiguousarray(signal, dtype=np.float64), min, max, mad=False)
 
 
-def thresholdstats_mad(signal, min: float = -np.inf, max: float = np.inf, *, device: int = 0,
-                       handle: Optional[Handle] = None) -> float:
-    """1.4826 * MAD of the samples inside [min, max]  (src/thresholdstats.jl:61-71)"""
+def thresholdstats_mad(signal, min: float = -np.inf, max: float = np.inf, *, device: int = 0, handle: Optional[Handle] = None):
+    """1.4826 * MAD of the samples inside [min, max]  (src/thresholdstats.jl:61-71); one value per row of a 2-D signal"""
+    if np.ndim(signal) == 2:
+        return _thresholdstats_rows(signal, min, max, _abi.WFSTAT_THRESHOLDSTATS_MAD, "thr_mad", device, handle)
     return (handle or get_handle(device)).thresholdstats(np.ascontiguousarray(signal, dtype=np.float64), min, max, mad=True)
 
 
 class IntersectMaximum:
     """IntersectMaximum(mintot, maxtot)(waveform, threshold)  (src/intersect_maximum.jl:12-23): result dict with
-    x, x_high, x_tot, max (arrays, times in ns) and multiplicity"""
+    x, x_high, x_tot, max (arrays, times in ns) and multiplicity.  A 2-D signal [n_events, n_samples] takes a scalar or a
+    per-row threshold and gives x, x_high, x_tot, max as VectorOfVectors and multiplicity as int64[n_events]."""
 
     def __init__(self, mintot: Q, maxtot: Q):
         self.mintot, self.maxtot = mintot, maxtot
 
     def __call__(self, signal, threshold: float, *, t_first: Q = ns(0.0), step: Q = ns(16.0), device: int = 0,
                  handle: Optional[Handle] = None, max_triggers: int = 256):
-        y = np.ascontiguousarray(signal, dtype=np.float64)
         min_n, max_n = _min_n(self.mintot, step), _min_n(self.maxtot, step)
+        if np.ndim(signal) == 2:
+            return self._rows(signal, threshold, t_first, step, min_n, max_n, device, handle, max_triggers)
+        y = np.ascontiguousarray(signal, dtype=np.float64)
         h = handle or get_handle(device)
         while True:
             r = h.intersect_maximum(y, t_first.ns(), step.ns(), float(threshold), min_n, max_n, max_triggers)
             if r["multiplicity"] <= max_triggers:
                 return r
             max_triggers = r["multiplicity"]
+
+    @staticmethod
+    def _rows(signal, threshold, t_first, step, min_n, max_n, device, handle, cap):
+        sig, kind, _ = wf_samples(signal)
+        thr = np.asarray(threshold, dtype=np.float64)
+        if thr.ndim not in (0, 1) or (thr.ndim == 1 and len(thr) != sig.shape[0]):
+            raise ValueError("threshold: a scalar or one value per waveform")
+        P = wfstats_params(sig.shape[1], kind, _abi.WFSTAT_INTERSECT_MAXIMUM, t_first, step)
+        P.im_min_n, P.im_max_n = min_n, max_n
+        while True:
+            P.max_triggers = min(int(cap), _abi.WFSTAT_MAX_TRIGGERS)
+            rows, lists = wfstats_rows(sig, P, thr, device=device, handle=handle)
+            cnt = rows[:, _abi.WFSTAT_COL["multiplicity"]].astype(np.int64)
+            most = int(cnt.max()) if len(cnt) else 0
+            if most <= P.max_triggers:
+                break
+            if P.max_triggers >= _abi.WFSTAT_MAX_TRIGGERS:
+                raise RuntimeError(f"a waveform has {most} triggers, more than {_abi.WFSTAT_MAX_TRIGGERS}")
+            cap = max(2 * P.max_triggers, most)
+        ptr = np.concatenate(([0], np.cumsum(cnt)))
+        keep = np.arange(lists.shape[2])[None, :] < cnt[:, None]
+        out = {k: VectorOfVectors(lists[:, f, :][keep], ptr) for f, k in enumerate(("x", "x_high", "x_tot", "max"))}
+        out["multiplicity"] = cnt
+        return out
 
 
 class MultiIntersect:
