@@ -217,7 +217,13 @@ def test_sweep_run_ext_baseline_and_aux(L, handle, fixed_pool, kind):
     wf, bl = fixed_pool
     n = len(wf)
     S = L.resolve_sweep_params(L.example_config(), L.us(500.0), n_samples=1024, out_f64=True, external_baseline=True)
-    var = L.trap_sweep_variants([L.us(1.0), L.us(2.0)], [L.us(0.5), L.us(1.0)], L.ns(16.0), mode="ft")
+    trap = L.trap_sweep_variants([L.us(1.0), L.us(2.0)], [L.us(0.5), L.us(1.0)], L.ns(16.0), mode="ft")
+    # one FIR (CUSP, 500 taps) and one Savitzky-Golay variant (window set on the 1 024-sample trace) besides the trapezoids
+    fir = L.cuspzac_sweep_variants(cfg4096(L), "cusp", [L.us(1.0)], [L.us(0.5)], L.ns(16.0), mode="ft")
+    sg = L.sg_sweep_variants(cfg4096(L), [L.ns(200.0)], n_samples=4096, t_first=L.ns(0.0), step=L.ns(16.0))
+    sg.array[0].win_from, sg.array[0].win_until = 300, 700
+    from test_gpu_sweeps_random import concat_variants
+    var = concat_variants(L, [(trap, i) for i in range(len(trap))] + [(fir, 0), (sg, 0)])
     dev = Dev(handle)
     handle.gsweep_run_ext_device(S, dev.put(wf), 2, dev.put(bl), n, 1024, var.array, dev.out((n, len(var)), np.float64),
                                  dev.out((n, 4), np.float64))
