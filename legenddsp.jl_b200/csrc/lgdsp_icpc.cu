@@ -208,19 +208,8 @@ __device__ __forceinline__ double extrema3(double y1, double y2, double y3)
     return y1 - a * a / (8.0 * (y3 - 2.0 * y2 + y1));
 }
 
-// ---- single-sample evaluations on the prefix sums TT (TT[i] = sum_{k<i} y[k]); used by the scalar tail ----
-__device__ __noinline__ double trap_eval(const double* TT, int a, int ag, int L, double inv1, double inv2, int j)
-{
-    const double s1 = TT[j + a] - TT[j];
-    const double s2 = TT[j + L] - TT[j + ag];
-    return __fma_rn(s2, inv2, -__dmul_rn(s1, inv1));
-}
-__device__ __forceinline__ double trap_at(const double* TT, const TrapDev& t, int j)
-{
-    return trap_eval(TT, t.a, t.a + t.g, t.L, t.inv1, t.inv2, j);
-}
-// the same arithmetic inlined at the call site (the split pipeline's extract kernel: no call frame, the trapezoid's
-// constants stay in uniform registers)
+// ---- single-sample evaluations on the prefix sums TT (TT[i] = sum_{k<i} y[k]) ----
+// trapezoid output j, inlined at every call site (no call frame; the trapezoid's constants stay in uniform registers)
 __device__ __forceinline__ double trap_at_i(const double* TT, const TrapDev& t, int j)
 {
     const double* p = TT + j;
@@ -987,6 +976,99 @@ __device__ __forceinline__ bool sum_exceeds_u32(const SAMPLE* xp, int cvalid, ui
     return total > 4294967295.0;
 }
 
+// ---------------------------------------------------------------------------------------------------
+// Per-event arithmetic of both dsp_icpc paths: icpc_kernel and the split pipeline (lgdsp_icpc_split.cuh) call these
+// functions, so both compute each of these values with the same expressions in the same order.
+// ---------------------------------------------------------------------------------------------------
+// SG trace sample j of filter f; sgg: shared-memory copy of the zero-padded taps of the short filters
+__device__ __forceinline__ double sg_sample(const IcpcDev& P, const double* TT, const double (*sgg)[8], int f, int j)
+{
+    return (P.sg[f].n_taps + 1 <= 8) ? sg_eval8(TT, sgg[f], j) : sg_eval(TT, P.sg[f].gg, P.sg[f].n_taps, j);
+}
+// t10..t99 [us] from the resolved position pos of threshold th on the PZ waveform; NaN -> 0
+__device__ __forceinline__ double tx_us_at(const double* TT, int pos, double th, double t_first, double dt)
+{
+    double t = 0.0;
+    if (pos >= 1) t = cross_x(th, y_at(TT, pos - 1), y_at(TT, pos), t_first + (double)(pos - 1) * dt, dt) * 0.001;
+    return t != t ? 0.0 : t;
+}
+// t0 / t0_inv [us] from the resolved position of the t0 (inv: t0_inv) mask; NaN -> 0
+__device__ __forceinline__ double t0_us_at(const IcpcDev& P, const double* TT, bool inv, int pos, double t_first, double dt)
+{
+    const TrapDev& tr = inv ? P.t0inv : P.t0;
+    double t = 0.0;
+    if (pos >= 1) {
+        const double tl = t_first + (double)(pos - 1 + tr.L - 1) * dt;
+        const double sgn = inv ? -1.0 : 1.0;
+        t = cross_x(P.t0_thr, sgn * trap_at_i(TT, tr, pos - 1), sgn * trap_at_i(TT, tr, pos), tl, dt) * 0.001;
+    }
+    return t != t ? 0.0 : t;
+}
+// get_qdrift  src/dsp_routines.jl:51-64 on the integrator trace I[i] = TT[i+1] at t_us, one warp
+__device__ __forceinline__ double qdrift_at(const IcpcDev& P, const double* TT, const double* A_int, int n, double t_first, double dt,
+                                            double t_us, double first, double last, int lane)
+{
+    const double tns = t_us * 1000.0;
+    if (P.int_dni.n_w <= 8) {
+        // the three estimates in parallel, 8 lanes each
+        const int g = lane >> 3;
+        const double ts = g == 0 ? tns : (g == 1 ? tns + first : tns + last);
+        double pc;
+        int from;
+        dni_window(P.int_dni.n_w, n, (ts - t_first) / dt, pc, from);
+        const double r = dni3_warp(A_int, P.int_dni.n_w, P.int_dni.m, TT + 1, from, pc - (double)from, lane);
+        const double a0 = __shfl_sync(FULL, r, 0), a1 = __shfl_sync(FULL, r, 8), a2 = __shfl_sync(FULL, r, 16);
+        return (a2 - a1) - (a1 - a0);
+    }
+    double a[3];
+#pragma unroll 1
+    for (int q = 0; q < 3; ++q) {
+        const double ts = q == 0 ? tns : (q == 1 ? tns + first : tns + last);
+        double pc;
+        int from;
+        dni_window(P.int_dni.n_w, n, (ts - t_first) / dt, pc, from);
+        a[q] = dni_eval_warp(A_int, P.int_dni.n_w, P.int_dni.m, TT + from + 1, pc - (double)from, lane);
+    }
+    const double area1 = a[1] - a[0], area2 = a[2] - a[1];
+    return area2 - area1;
+}
+
+// CUSP/ZAC candidate chunk: Lipschitz bound on (33 tid, 33 tid + 33) against the best coarse values Mc / Mz; chunks that
+// hold part of a pick-off window (pk_from[ic] for CUSP, pk_from[iz] for ZAC, nw samples each) are always evaluated.
+// czco: the coarse values [2][NT]
+__device__ __forceinline__ bool cz_candidate(const CzDev& Z, const CzState& st, double oc, double oz, const double* czco, int tid, int i0,
+                                             double Ymax, double Mc, double Mz, bool want_cusp, bool want_zac, const int* pk_from,
+                                             int ic, int iz, int nw)
+{
+    bool cand = false;
+    if (st.active) {
+        const int t1 = min(tid + 1, NT - 1);
+        const double kap = Ymax * 1.000001;
+        const int jlo = i0 - Z.L + 1, jhi = jlo + CH - 1;
+        if (want_cusp) {
+            const double a = oc, b = (tid + 1 < NT) ? czco[t1] : -CUDART_INF;
+            const double kc = kap * Z.lip_cusp;
+            double bound;
+            if (a > -CUDART_INF) bound = interval_bound(a, b, b > -CUDART_INF, kc);
+            else if (b > -CUDART_INF) bound = fma((double)CH, kc, b);
+            else bound = CUDART_INF;
+            cand |= bound + 1e-6 * (fabs(Mc) + Ymax * fabs(Z.g)) >= Mc;
+            cand |= (jhi >= pk_from[ic] && jlo < pk_from[ic] + nw);
+        }
+        if (want_zac) {
+            const double a = oz, b = (tid + 1 < NT) ? czco[NT + t1] : -CUDART_INF;
+            const double kz = kap * Z.lip_zac;
+            double bound;
+            if (a > -CUDART_INF) bound = interval_bound(a, b, b > -CUDART_INF, kz);
+            else if (b > -CUDART_INF) bound = fma((double)CH, kz, b);
+            else bound = CUDART_INF;
+            cand |= bound + 1e-6 * (fabs(Mz) + Ymax * fabs(Z.g)) >= Mz;
+            cand |= (jhi >= pk_from[iz] && jlo < pk_from[iz] + nw);
+        }
+    }
+    return cand;
+}
+
 // SAMPLE = uint16_t (raw FADC samples) or uint32_t (presummed waveforms of dsp_icpc_compressed, n <= 4096).
 // bl_ext != NULL: the baseline mean of event e is bl_ext[e] instead of the bl_window mean (windowed waveforms of
 // dsp_icpc_compressed are shifted by blmean_presummed / presum_rate, src/dsp_icpc.jl:350).
@@ -1032,9 +1114,7 @@ icpc_kernel(const __grid_constant__ IcpcDev P, const SAMPLE* __restrict__ wf, lo
     }
     __syncthreads();
     // SG trace sample j of filter f
-    auto sg_at = [&](int f, int j) -> double {
-        return (P.sg[f].n_taps + 1 <= 8) ? sg_eval8(TT, spar->sgg[f], j) : sg_eval(TT, P.sg[f].gg, P.sg[f].n_taps, j);
-    };
+    auto sg_at = [&](int f, int j) -> double { return sg_sample(P, TT, spar->sgg, f, j); };
     long long e = blockIdx.x;
     if (tid == 0 && e < n_events) {
         mbar_expect_tx(bar, wf_bytes);
@@ -1410,18 +1490,18 @@ icpc_kernel(const __grid_constant__ IcpcDev P, const SAMPLE* __restrict__ wf, lo
         {
             const int ja = i0, jb = i0 + CH;
             if (G & LGDSP_GROUP_TIMING) {
-                if (ja < P.t0.nout) c0a = trap_at(TT, P.t0, ja);
-                if (jb < P.t0.nout) c0b = trap_at(TT, P.t0, jb);
+                if (ja < P.t0.nout) c0a = trap_at_i(TT, P.t0, ja);
+                if (jb < P.t0.nout) c0b = trap_at_i(TT, P.t0, jb);
                 if (!P.t0inv_same) {
-                    if (ja < P.t0inv.nout) cia = trap_at(TT, P.t0inv, ja);
-                    if (jb < P.t0inv.nout) cib = trap_at(TT, P.t0inv, jb);
+                    if (ja < P.t0inv.nout) cia = trap_at_i(TT, P.t0inv, ja);
+                    if (jb < P.t0inv.nout) cib = trap_at_i(TT, P.t0inv, jb);
                 }
             }
             if (G & LGDSP_GROUP_TRAPS) {
-                if (ja < P.e535.nout) c5a = trap_at(TT, P.e535, ja);
-                if (jb < P.e535.nout) c5b = trap_at(TT, P.e535, jb);
-                if (ja < P.etrap.nout) cea = trap_at(TT, P.etrap, ja);
-                if (jb < P.etrap.nout) ceb = trap_at(TT, P.etrap, jb);
+                if (ja < P.e535.nout) c5a = trap_at_i(TT, P.e535, ja);
+                if (jb < P.e535.nout) c5b = trap_at_i(TT, P.e535, jb);
+                if (ja < P.etrap.nout) cea = trap_at_i(TT, P.etrap, ja);
+                if (jb < P.etrap.nout) ceb = trap_at_i(TT, P.etrap, jb);
                 const double w5 = wmax_d(c5a), we = wmax_d(cea);
                 red_put(red, R_C535, wid, lane, w5);
                 red_put(red, R_CET, wid, lane, we);
@@ -1528,7 +1608,7 @@ icpc_kernel(const __grid_constant__ IcpcDev P, const SAMPLE* __restrict__ wf, lo
         const double Ymax = red_max(red, R_YMAX);     // bound of max |y| of the PZ waveform
         const double kslack = 1e-7 * Ymax;            // >> float64 rounding of any trace
         // the 44 trap(rt,ft) outputs of the e_trap pick-off window
-        if ((G & LGDSP_GROUP_TRAPS) && tid < P.sig_dni.n_w) stash[tid] = trap_at(TT, P.etrap, pk_from[0] + tid);
+        if ((G & LGDSP_GROUP_TRAPS) && tid < P.sig_dni.n_w) stash[tid] = trap_at_i(TT, P.etrap, pk_from[0] + tid);
 
         // ---- thresholds of the sg[0] masks (t50_current at half the trace maximum; pile-up at n sigma of the baseline
         //      window, sigma exactly as signalstats computes it) ----
@@ -1554,7 +1634,7 @@ icpc_kernel(const __grid_constant__ IcpcDev P, const SAMPLE* __restrict__ wf, lo
                 const double th = P.t0_thr;
                 const int j = q * CH + 1 + lane;
                 const bool v = j < tr.nout;
-                const double o = v ? trap_at(TT, tr, j) : 0.0;
+                const double o = v ? trap_at_i(TT, tr, j) : 0.0;
                 const unsigned mp = __ballot_sync(FULL, v && (o >= th));
                 const unsigned mn_ = __ballot_sync(FULL, v && (-o >= th));
                 commit_pair(type == 0 ? masks + M_T0 * NWORDS : nullptr, (unsigned long long)mp << 1,
@@ -1563,13 +1643,13 @@ icpc_kernel(const __grid_constant__ IcpcDev P, const SAMPLE* __restrict__ wf, lo
             } else if (type == 2) {
                 const int j = q * CH + 1 + lane;
                 if (j < P.e535.nout) {
-                    const double o = trap_at(TT, P.e535, j);
+                    const double o = trap_at_i(TT, P.e535, j);
                     e535 = o > e535 ? o : e535;
                 }
             } else if (type == 3) {
                 const int j = q * CH + 1 + lane;
                 if (j < P.etrap.nout) {
-                    const double o = trap_at(TT, P.etrap, j);
+                    const double o = trap_at_i(TT, P.etrap, j);
                     if (o > etmax || (o == etmax && j < etarg)) { etmax = o; etarg = j; }
                 }
             } else {
@@ -1696,47 +1776,12 @@ icpc_kernel(const __grid_constant__ IcpcDev P, const SAMPLE* __restrict__ wf, lo
         //      while the candidate warps step their recurrences (scalar_jobs), the two CUSP/ZAC jobs after B6 ----
         // t10..t99 [us] (k = 0..4) and t0 / t0_inv [us] from the resolved positions; NaN -> 0
         auto tx_us = [&](int k) -> double {
-            const int pos = ibuf[IB_POS0 + M_T10 + k];
             const double th = k == 0 ? thr[0] : k == 1 ? thr[1] : k == 2 ? thr[2] : k == 3 ? thr[3] : thr[4];
-            double t = 0.0;
-            if (pos >= 1) t = cross_x(th, y_at(TT, pos - 1), y_at(TT, pos), t_first + (double)(pos - 1) * dt, dt) * 0.001;
-            return t != t ? 0.0 : t;
+            return tx_us_at(TT, ibuf[IB_POS0 + M_T10 + k], th, t_first, dt);
         };
-        auto t0_us = [&](bool inv, int pos) -> double {
-            const TrapDev& tr = inv ? P.t0inv : P.t0;
-            double t = 0.0;
-            if (pos >= 1) {
-                const double tl = t_first + (double)(pos - 1 + tr.L - 1) * dt;
-                const double sgn = inv ? -1.0 : 1.0;
-                t = cross_x(P.t0_thr, sgn * trap_at(TT, tr, pos - 1), sgn * trap_at(TT, tr, pos), tl, dt) * 0.001;
-            }
-            return t != t ? 0.0 : t;
-        };
-        // get_qdrift  src/dsp_routines.jl:51-64 on the integrator trace I[i] = TT[i+1], one warp
+        auto t0_us = [&](bool inv, int pos) -> double { return t0_us_at(P, TT, inv, pos, t_first, dt); };
         auto qdrift_warp = [&](double t_us, double first, double last) -> double {
-            const double tns = t_us * 1000.0;
-            if (P.int_dni.n_w <= 8) {
-                // the three estimates in parallel, 8 lanes each
-                const int g = lane >> 3;
-                const double ts = g == 0 ? tns : (g == 1 ? tns + first : tns + last);
-                double pc;
-                int from;
-                dni_window(P.int_dni.n_w, n, (ts - t_first) / dt, pc, from);
-                const double r = dni3_warp(A_int, P.int_dni.n_w, P.int_dni.m, TT + 1, from, pc - (double)from, lane);
-                const double a0 = __shfl_sync(FULL, r, 0), a1 = __shfl_sync(FULL, r, 8), a2 = __shfl_sync(FULL, r, 16);
-                return (a2 - a1) - (a1 - a0);
-            }
-            double a[3];
-#pragma unroll 1
-            for (int q = 0; q < 3; ++q) {
-                const double ts = q == 0 ? tns : (q == 1 ? tns + first : tns + last);
-                double pc;
-                int from;
-                dni_window(P.int_dni.n_w, n, (ts - t_first) / dt, pc, from);
-                a[q] = dni_eval_warp(A_int, P.int_dni.n_w, P.int_dni.m, TT + from + 1, pc - (double)from, lane);
-            }
-            const double area1 = a[1] - a[0], area2 = a[2] - a[1];
-            return area2 - area1;
+            return qdrift_at(P, TT, A_int, n, t_first, dt, t_us, first, last, lane);
         };
         auto scalar_jobs = [&]() {
         if (wid == 0) {
@@ -1937,32 +1982,8 @@ icpc_kernel(const __grid_constant__ IcpcDev P, const SAMPLE* __restrict__ wf, lo
             // hold part of a pick-off window are always evaluated
             double Mc = 0.0, Mz = 0.0;
             if (czp) { Mc = red_max(red, R_CZC0); Mz = red_max(red, R_CZC1); }
-            bool cand = false;
-            if (czp && st.active) {
-                const int t1 = min(tid + 1, NT - 1);
-                const double kap = Ymax * 1.000001;
-                const int jlo = i0 - Z.L + 1, jhi = jlo + CH - 1;
-                if (want_cusp) {
-                    const double a = oc, b = (tid + 1 < NT) ? czco[t1] : -CUDART_INF;
-                    const double kc = kap * Z.lip_cusp;
-                    double bound;
-                    if (a > -CUDART_INF) bound = interval_bound(a, b, b > -CUDART_INF, kc);
-                    else if (b > -CUDART_INF) bound = fma((double)CH, kc, b);
-                    else bound = CUDART_INF;
-                    cand |= bound + 1e-6 * (fabs(Mc) + Ymax * fabs(Z.g)) >= Mc;
-                    cand |= (jhi >= pk_from[1] && jlo < pk_from[1] + P.sig_dni.n_w);
-                }
-                if (want_zac) {
-                    const double a = oz, b = (tid + 1 < NT) ? czco[NT + t1] : -CUDART_INF;
-                    const double kz = kap * Z.lip_zac;
-                    double bound;
-                    if (a > -CUDART_INF) bound = interval_bound(a, b, b > -CUDART_INF, kz);
-                    else if (b > -CUDART_INF) bound = fma((double)CH, kz, b);
-                    else bound = CUDART_INF;
-                    cand |= bound + 1e-6 * (fabs(Mz) + Ymax * fabs(Z.g)) >= Mz;
-                    cand |= (jhi >= pk_from[2] && jlo < pk_from[2] + P.sig_dni.n_w);
-                }
-            }
+            const bool cand = czp && cz_candidate(Z, st, oc, oz, czco, tid, i0, Ymax, Mc, Mz, want_cusp, want_zac, pk_from, 1, 2,
+                                                  P.sig_dni.n_w);
             // slot of every candidate chunk in the output buffer (rounds of CZCAP chunks)
             int slot = -1;
             {

@@ -14,7 +14,9 @@
 //
 // (reference lines: /root/reference/src/dsp_icpc.jl).  The three kernels of one event batch run back to back on a stream;
 // the batch is sized so that its prefix sums (65.6 KB per event) are still in L2 when the consumers read them.
-// Every value is produced by the same expressions as in icpc_kernel (same helpers, same operation order).
+// Every value is produced by the same expressions as in icpc_kernel (same helpers, same operation order); the crossing, t0
+// and Q-drift evaluations of phase C, sg_sample and the CUSP/ZAC candidate bound are functions in lgdsp_icpc.cu that both
+// paths call.
 
 constexpr int TTG_LEN = TT_LEN;     // doubles per event slot of the global prefix-sum ring
 constexpr int AUX_LEN = 16;         // doubles per event: values handed from the prefix kernel to the consumers
@@ -552,9 +554,7 @@ icpc_extract_kernel(const __grid_constant__ IcpcDev P, const double* __restrict_
     if (tid < TT_LEN - 2 - n) TT[n + 2 + tid] = 0.0;   // finite padding behind the loaded part (zero-padded SG kernels read it)
     if (tid < 24) sgg[tid >> 3][tid & 7] = P.sg[tid >> 3].gg[tid & 7];
     __syncthreads();
-    auto sg_at = [&](int f, int j) -> double {
-        return (P.sg[f].n_taps + 1 <= 8) ? sg_eval8(TT, sgg[f], j) : sg_eval(TT, P.sg[f].gg, P.sg[f].n_taps, j);
-    };
+    auto sg_at = [&](int f, int j) -> double { return sg_sample(P, TT, sgg, f, j); };
     const int i0 = tid * CH;
     const int nsg = P.sg[0].nout;
     const bool want_cur = (G & LGDSP_GROUP_CURRENT) != 0, want_intr = (G & LGDSP_GROUP_INTRACE) != 0;
@@ -717,13 +717,7 @@ icpc_extract_kernel(const __grid_constant__ IcpcDev P, const double* __restrict_
         const double Ymax = aux[AX_YMAX];
         const double kslack = 1e-7 * Ymax;
         // t10..t99 [us] from the positions the prefix kernel resolved; NaN -> 0
-        auto tx_us = [&](int k) -> double {
-            const int pos = (int)aux[AX_POS + k];
-            const double th = aux[AX_THR + k];
-            double t = 0.0;
-            if (pos >= 1) t = cross_x(th, y_at(TT, pos - 1), y_at(TT, pos), t_first + (double)(pos - 1) * dt, dt) * 0.001;
-            return t != t ? 0.0 : t;
-        };
+        auto tx_us = [&](int k) -> double { return tx_us_at(TT, (int)aux[AX_POS + k], aux[AX_THR + k], t_first, dt); };
         // DNI window of the trap(rt,ft) energy pick-off at t50 + pick (every thread: uniform values)
         double pk_p;
         int pk_from;
@@ -875,39 +869,9 @@ icpc_extract_kernel(const __grid_constant__ IcpcDev P, const double* __restrict_
         // ==========================================================================================
         // phase C: scalar results, one self-contained job per warp
         // ==========================================================================================
-        auto t0_us = [&](bool inv, int pos) -> double {
-            const TrapDev& tr = inv ? P.t0inv : P.t0;
-            double t = 0.0;
-            if (pos >= 1) {
-                const double tl = t_first + (double)(pos - 1 + tr.L - 1) * dt;
-                const double sgn = inv ? -1.0 : 1.0;
-                t = cross_x(P.t0_thr, sgn * trap_at_i(TT, tr, pos - 1), sgn * trap_at_i(TT, tr, pos), tl, dt) * 0.001;
-            }
-            return t != t ? 0.0 : t;
-        };
+        auto t0_us = [&](bool inv, int pos) -> double { return t0_us_at(P, TT, inv, pos, t_first, dt); };
         auto qdrift_warp = [&](double t_us, double first, double last) -> double {
-            const double tns = t_us * 1000.0;
-            if (P.int_dni.n_w <= 8) {
-                const int g = lane >> 3;
-                const double ts = g == 0 ? tns : (g == 1 ? tns + first : tns + last);
-                double pc;
-                int from;
-                dni_window(P.int_dni.n_w, n, (ts - t_first) / dt, pc, from);
-                const double r = dni3_warp(A_int, P.int_dni.n_w, P.int_dni.m, TT + 1, from, pc - (double)from, lane);
-                const double a0 = __shfl_sync(FULL, r, 0), a1 = __shfl_sync(FULL, r, 8), a2 = __shfl_sync(FULL, r, 16);
-                return (a2 - a1) - (a1 - a0);
-            }
-            double a[3];
-#pragma unroll 1
-            for (int q = 0; q < 3; ++q) {
-                const double ts = q == 0 ? tns : (q == 1 ? tns + first : tns + last);
-                double pc;
-                int from;
-                dni_window(P.int_dni.n_w, n, (ts - t_first) / dt, pc, from);
-                a[q] = dni_eval_warp(A_int, P.int_dni.n_w, P.int_dni.m, TT + from + 1, pc - (double)from, lane);
-            }
-            const double area1 = a[1] - a[0], area2 = a[2] - a[1];
-            return area2 - area1;
+            return qdrift_at(P, TT, A_int, n, t_first, dt, t_us, first, last, lane);
         };
         if (wid == 0 && !lean) {
             // PZ tail statistics (signalstats on the tail window, src/dsp_icpc.jl:123)
@@ -1107,34 +1071,7 @@ __device__ __forceinline__ void cz_select(const CzDev& Z, const double* TT, int 
     int Ac, Az;
     red_argmax(red, K3R_CZMAX0, K3R_CZARG0, Mc, Ac);
     red_argmax(red, K3R_CZMAX1, K3R_CZARG1, Mz, Az);
-    // candidate chunks: Lipschitz bound on (33 tid, 33 tid + 33) against the best coarse value; chunks that
-    // hold part of a pick-off window are always evaluated
-    bool cand = false;
-    if (st.active) {
-        const int t1 = min(tid + 1, NT - 1);
-        const double kap = Ymax * 1.000001;
-        const int jlo = i0 - Z.L + 1, jhi = jlo + CH - 1;
-        if (want_cusp) {
-            const double a = oc, b = (tid + 1 < NT) ? czco[t1] : -CUDART_INF;
-            const double kc = kap * Z.lip_cusp;
-            double bound;
-            if (a > -CUDART_INF) bound = interval_bound(a, b, b > -CUDART_INF, kc);
-            else if (b > -CUDART_INF) bound = fma((double)CH, kc, b);
-            else bound = CUDART_INF;
-            cand |= bound + 1e-6 * (fabs(Mc) + Ymax * fabs(Z.g)) >= Mc;
-            cand |= (jhi >= pk_from[0] && jlo < pk_from[0] + nw);
-        }
-        if (want_zac) {
-            const double a = oz, b = (tid + 1 < NT) ? czco[NT + t1] : -CUDART_INF;
-            const double kz = kap * Z.lip_zac;
-            double bound;
-            if (a > -CUDART_INF) bound = interval_bound(a, b, b > -CUDART_INF, kz);
-            else if (b > -CUDART_INF) bound = fma((double)CH, kz, b);
-            else bound = CUDART_INF;
-            cand |= bound + 1e-6 * (fabs(Mz) + Ymax * fabs(Z.g)) >= Mz;
-            cand |= (jhi >= pk_from[1] && jlo < pk_from[1] + nw);
-        }
-    }
+    const bool cand = cz_candidate(Z, st, oc, oz, czco, tid, i0, Ymax, Mc, Mz, want_cusp, want_zac, pk_from, 0, 1, nw);
     // candidate records: the window states at the chunk start + the chunk index
     {
         const unsigned bc = __ballot_sync(FULL, cand);
