@@ -48,12 +48,12 @@ static_assert(NWORDS == NT, "one mask word per thread");
 // T10..T99 last: their 5 KB are reused for the coarse CUSP/ZAC values once they are resolved
 enum { M_T0 = 0, M_T0INV, M_CUR, M_PILE, M_T10, M_T50, M_T80, M_T90, M_T99, NMASK };
 
-// reduction slots: red[slot][warp]
+// reduction slots: red[slot][warp].  The slots of the raw-sample pass (raw_pass) come first in icpc_kernel and in
+// icpc_prefix_kernel alike.
+enum { R_BLS = 0, R_BLSS, R_BLSX, R_MX /* + R_MN: 4 x NWARP uint32 */, R_MN, R_SLEN, R_SS, R_SQ, R_RAW_N };
 enum {
-    // stage A (after P1)
-    R_BLS = 0, R_BLSS, R_BLSX, R_NLOW, R_NHIGH, R_MX, R_MN, R_SLEN, R_SS, R_SQ,
     // stage C (after P2/P3)
-    R_TLS, R_TLSS, R_TLSX, R_TLBAD, R_PZS, R_PZSS, R_PZSX, R_YMIN, R_YMAX,
+    R_TLS = R_RAW_N, R_TLSS, R_TLSX, R_TLBAD, R_PZS, R_PZSS, R_PZSX, R_YMIN, R_YMAX,
     R_E104, R_E104N, R_E313, R_E313N, R_C535, R_CET, R_SGMAX, R_SGS, R_SGSS,
     R_CMAX0, R_CMAX1, R_CMAX2, R_CMAX3, R_CARG0, R_CARG1, R_CARG2, R_CARG3,
     // stage D
@@ -981,9 +981,9 @@ __device__ __forceinline__ bool sum_exceeds_u32(const SAMPLE* xp, int cvalid, ui
 // functions, so both compute each of these values with the same expressions in the same order.
 // ---------------------------------------------------------------------------------------------------
 // SG trace sample j of filter f; sgg: shared-memory copy of the zero-padded taps of the short filters
-__device__ __forceinline__ double sg_sample(const IcpcDev& P, const double* TT, const double (*sgg)[8], int f, int j)
+__device__ __forceinline__ double sg_sample(const SgDev* sg, const double* TT, const double (*sgg)[8], int f, int j)
 {
-    return (P.sg[f].n_taps + 1 <= 8) ? sg_eval8(TT, sgg[f], j) : sg_eval(TT, P.sg[f].gg, P.sg[f].n_taps, j);
+    return (sg[f].n_taps + 1 <= 8) ? sg_eval8(TT, sgg[f], j) : sg_eval(TT, sg[f].gg, sg[f].n_taps, j);
 }
 // t10..t99 [us] from the resolved position pos of threshold th on the PZ waveform; NaN -> 0
 __device__ __forceinline__ double tx_us_at(const double* TT, int pos, double th, double t_first, double dt)
@@ -1069,6 +1069,239 @@ __device__ __forceinline__ bool cz_candidate(const CzDev& Z, const CzState& st, 
     return cand;
 }
 
+// Raw-sample pass of one event: this thread's chunk of cvalid samples at xs + i0 and block-wide results.  Writes the
+// R_BLS .. R_SQ slots of red, ends behind one block barrier.  lean: the baseline slope / sigma sums are not wanted.
+struct RawPass {
+    uint32_t cmn, cmx;      // chunk min / max
+    uint32_t mn, mx;        // block min / max
+    int nlow, nhigh;        // block-wide saturation counts
+    uint32_t P_excl;        // exclusive prefixes of the chunk: cumsum(x) and cumsum(cumsum(x)) before sample i0
+    double PP_excl;
+};
+template <typename SAMPLE>
+__device__ __forceinline__ RawPass raw_pass(const SAMPLE* xs, int i0, int cvalid, int bl_from, int bl_until, int sat_low, int sat_high,
+                                            bool lean, double* red, int tid, int lane, int wid)
+{
+    RawPass r;
+    const SAMPLE* xp = xs + i0;
+    uint32_t csum = 0, cq = 0, cmn = 0xFFFFFFFFu, cmx = 0;
+#pragma unroll 3
+    for (int k = 0; k < cvalid; ++k) {
+        const uint32_t x = xp[k];
+        csum += x;
+        cq += csum;
+        cmn = min(cmn, x);
+        cmx = max(cmx, x);
+    }
+    r.cmn = cmn; r.cmx = cmx;
+    // baseline regression sums (exact integers), samples of the window strided over ALL threads (the window covers the
+    // first chunks only: summed chunk-wise, three warps would do the whole job while the others wait at the barrier)
+    {
+        unsigned long long blSS = 0, blSX = 0;
+        uint32_t blS = 0;
+#pragma unroll 2
+        for (int idx = bl_from + tid; idx <= bl_until; idx += NT) {
+            const uint32_t x = xs[idx];
+            blS += x;
+            if (!lean) {
+                blSX += (unsigned long long)x * (unsigned long long)idx;
+                blSS += (unsigned long long)x * (unsigned long long)x;
+            }
+        }
+        // (all sums < 2^53: exact in double, in any order)
+        const double a = wsum_d((double)blS), bq = wsum_d((double)blSS), c = wsum_d((double)blSX);
+        if (lane == 0) { red[R_BLS * NWARP + wid] = a; red[R_BLSS * NWARP + wid] = bq; red[R_BLSX * NWARP + wid] = c; }
+    }
+    // saturation counts: a sample can only equal low/high if the chunk's min/max says so
+    int nlow = 0, nhigh = 0;
+    if ((int)cmn == sat_low || (int)cmx == sat_high) {
+        for (int k = 0; k < cvalid; ++k) {
+            const int x = xp[k];
+            nlow += (x == sat_low);
+            nhigh += (x == sat_high);
+        }
+    }
+    {
+        const uint32_t wmn = __reduce_min_sync(FULL, cmn), wmx = __reduce_max_sync(FULL, cmx);
+        const uint32_t wl = __reduce_add_sync(FULL, (uint32_t)nlow), wh = __reduce_add_sync(FULL, (uint32_t)nhigh);
+        if (lane == 0) {
+            uint32_t* ured = reinterpret_cast<uint32_t*>(red + R_MX * NWARP);
+            ured[wid] = wmx; ured[NWARP + wid] = wmn; ured[2 * NWARP + wid] = wl; ured[3 * NWARP + wid] = wh;
+        }
+    }
+    // one scan for P = cumsum(x) and PP = cumsum(P): segments (len, s = sum x, q = sum of the inclusive
+    // prefix sums inside the segment) combine as (lenA+lenB, sA+sB, qA+qB+lenB*sA); all values exact
+    int sl = cvalid;
+    uint32_t ss = csum;
+    double sq = (double)cq;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const int l2 = __shfl_up_sync(FULL, sl, o);
+        const uint32_t s2 = __shfl_up_sync(FULL, ss, o);
+        const double q2 = __shfl_up_sync(FULL, sq, o);
+        if (lane >= o) {
+            sq = q2 + sq + (double)sl * (double)s2;
+            ss += s2;
+            sl += l2;
+        }
+    }
+    if (lane == 31) {
+        red[R_SLEN * NWARP + wid] = (double)sl;
+        red[R_SS * NWARP + wid] = (double)ss;
+        red[R_SQ * NWARP + wid] = sq;
+    }
+    int el = __shfl_up_sync(FULL, sl, 1);
+    uint32_t es = __shfl_up_sync(FULL, ss, 1);
+    double eq = __shfl_up_sync(FULL, sq, 1);
+    if (lane == 0) { el = 0; es = 0; eq = 0.0; }
+    __syncthreads();
+
+    {
+        double cs = 0.0, cqd = 0.0;
+#pragma unroll 1
+        for (int w = 0; w < wid; ++w) {
+            const double lw = red[R_SLEN * NWARP + w], sw = red[R_SS * NWARP + w], qw = red[R_SQ * NWARP + w];
+            cqd = cqd + qw + lw * cs;
+            cs += sw;
+        }
+        r.P_excl = (uint32_t)cs + es;
+        r.PP_excl = cqd + eq + (double)el * cs;
+    }
+    {
+        const uint32_t* ured = reinterpret_cast<const uint32_t*>(red + R_MX * NWARP);
+        const int l8 = lane & 7;
+        r.mx = __reduce_max_sync(FULL, ured[l8]);
+        r.mn = __reduce_min_sync(FULL, ured[NWARP + l8]);
+        r.nlow = (int)__reduce_add_sync(FULL, lane < 8 ? ured[2 * NWARP + l8] : 0u);
+        r.nhigh = (int)__reduce_add_sync(FULL, lane < 8 ? ured[3 * NWARP + l8] : 0u);
+    }
+    return r;
+}
+
+// Closed-form prefix sums of the pole-zero waveform y = w + km1 * cumsum(w), w = x - m, along one chunk:
+// next(x) turns the following raw sample into TT[i + 1] = cumsum(y)[i]
+struct PzScan {
+    uint32_t Pr;     // cumsum(x)[i]
+    double PPr;      // cumsum(cumsum(x))[i]
+    double ip1;      // i + 1 after the update
+    double tri;      // (i + 1)(i + 2) / 2 after the update
+    __device__ __forceinline__ double next(uint32_t x, double m, double km1)
+    {
+        Pr += x;
+        const double Pd = u2d(Pr);
+        PPr += Pd;
+        ip1 += 1.0;
+        tri += ip1;
+        const double Sd = fma(-ip1, m, Pd);    // cumsum(w)[i]
+        const double SS = fma(-tri, m, PPr);   // cumsum(cumsum(w))[i]
+        return fma(km1, SS, Sd);
+    }
+};
+// Start of the chunk at i0 from its exclusive prefixes, and conservative bounds ylo / yhi (+- guard) of y on the chunk from
+// the integer min / max of its raw samples: cumsum(w)[i0+k] lies between S0 + (k+1)*wmin and S0 + (k+1)*wmax.
+struct PzChunk {
+    PzScan scan;
+    double TT0;                // TT[i0] (bit-identical to the neighbour's)
+    double ylo, yhi, guard;
+};
+__device__ __forceinline__ PzChunk pz_chunk(int i0, double m, double km1, uint32_t P_excl, double PP_excl, uint32_t cmn, uint32_t cmx)
+{
+    PzChunk c;
+    const double Sd0 = fma(-(double)i0, m, u2d(P_excl));   // cumsum(w)[i0-1]
+    const double tri0 = 0.5 * (double)i0 * ((double)i0 + 1.0);
+    c.TT0 = fma(km1, fma(-tri0, m, PP_excl), Sd0);
+    c.scan = {P_excl, PP_excl, (double)i0, tri0};
+    const double wmin = (double)cmn - m, wmax = (double)cmx - m;
+    const double ak = fabs(km1);
+    const double srange = (double)CH * fmax(fabs(wmin), fabs(wmax));
+    c.ylo = wmin + km1 * Sd0 - ak * srange;
+    c.yhi = wmax + km1 * Sd0 + ak * srange;
+    c.guard = 1e-9 * (fabs(c.ylo) + fabs(c.yhi)) + 1e-6;   // >> rounding of the TT differences
+    return c;
+}
+
+// Saturation run lengths (n_sat_low_cons, n_sat_high_cons) of an event with a saturated sample; block-wide, two barriers.
+// ired: int[8 * NWARP] of scratch.
+template <typename SAMPLE>
+__device__ __forceinline__ int2 sat_runs(int sat_low, int sat_high, const SAMPLE* xp, int cvalid, int lane, int wid, int* ired)
+{
+    Run rl = {0, 0, 0, cvalid}, rh = {0, 0, 0, cvalid};
+    {
+        int cl = 0, chh = 0;
+        bool pl = true, ph = true;
+        for (int k = 0; k < cvalid; ++k) {
+            const int x = xp[k];
+            const bool il = (x == sat_low), ih = (x == sat_high);
+            cl = il ? cl + 1 : 0;
+            chh = ih ? chh + 1 : 0;
+            rl.best = max(rl.best, cl);
+            rh.best = max(rh.best, chh);
+            if (pl && il) rl.pre = cl; else pl = false;
+            if (ph && ih) rh.pre = chh; else ph = false;
+        }
+        rl.suf = cl; rh.suf = chh;
+    }
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        Run bl_ = run_shfl_down(rl, o), bh_ = run_shfl_down(rh, o);
+        if ((lane & (2 * o - 1)) == 0) { rl = run_merge(rl, bl_); rh = run_merge(rh, bh_); }
+    }
+    if (lane == 0) {
+        ired[wid * 8 + 0] = rl.pre; ired[wid * 8 + 1] = rl.suf; ired[wid * 8 + 2] = rl.best; ired[wid * 8 + 3] = rl.len;
+        ired[wid * 8 + 4] = rh.pre; ired[wid * 8 + 5] = rh.suf; ired[wid * 8 + 6] = rh.best; ired[wid * 8 + 7] = rh.len;
+    }
+    __syncthreads();
+    Run al = {ired[0], ired[1], ired[2], ired[3]}, ah = {ired[4], ired[5], ired[6], ired[7]};
+    for (int w = 1; w < NWARP; ++w) {
+        Run bl_ = {ired[w * 8], ired[w * 8 + 1], ired[w * 8 + 2], ired[w * 8 + 3]};
+        Run bh_ = {ired[w * 8 + 4], ired[w * 8 + 5], ired[w * 8 + 6], ired[w * 8 + 7]};
+        al = run_merge(al, bl_);
+        ah = run_merge(ah, bh_);
+    }
+    __syncthreads();   // the scratch may be reused behind this barrier
+    return make_int2(al.best, ah.best);
+}
+
+// get_wvf_maximum  src/interpolation.jl:30-46 of current trace f = lane (0..2: sg[f], 3: the derivative), lanes 0..3,
+// from the block-wide first argmax in the slots cmax0 + f / carg0 + f of red: parabola only if strictly inside the window
+__device__ __forceinline__ void currents_job(const double* TT, const SgDev* sg, const double (*sgg)[8], const int* sg_alias,
+                                             const int* cur_from, const int* cur_until, const double* red, int cmax0, int carg0,
+                                             double* row, int lane)
+{
+    double vv[4];
+    int aa[4];
+#pragma unroll
+    for (int f = 0; f < 4; ++f) {
+        const int fs = (f < 3 && sg_alias[f] >= 0) ? sg_alias[f] : f;   // aliased filter: same trace and window
+        red_argmax(red, cmax0 + fs, carg0 + fs, vv[f], aa[f]);
+    }
+    if (lane < 4) {
+        const int f = lane;
+        double v = f == 0 ? vv[0] : f == 1 ? vv[1] : f == 2 ? vv[2] : vv[3];
+        const int a = f == 0 ? aa[0] : f == 1 ? aa[1] : f == 2 ? aa[2] : aa[3];
+        if (a > cur_from[f] && a < cur_until[f]) {
+            const double y1 = (f < 3) ? sg_sample(sg, TT, sgg, f, a - 1) : deriv_at(TT, a - 1);
+            const double y3 = (f < 3) ? sg_sample(sg, TT, sgg, f, a + 1) : deriv_at(TT, a + 1);
+            v = extrema3(y1, v, y3);
+        }
+        row[LGDSP_COL_a_sg + f] = v;
+    }
+}
+
+// Levels of an event from its baseline mean m and its sample min / max: e_max, e_min and the t10..t99 thresholds
+// (lean: only t50)
+struct Levels { double e_max, e_min, thr[5]; };
+__device__ __forceinline__ Levels event_levels(double m, uint32_t mx, uint32_t mn, const double* tx_frac, bool lean)
+{
+    Levels v;
+    v.e_max = (double)mx - m;
+    v.e_min = (double)mn - m;
+#pragma unroll
+    for (int k = 0; k < 5; ++k) v.thr[k] = v.e_max * tx_frac[k];
+    if (lean) { v.thr[0] = CUDART_INF; v.thr[2] = CUDART_INF; v.thr[3] = CUDART_INF; v.thr[4] = CUDART_INF; }
+    return v;
+}
+
 // SAMPLE = uint16_t (raw FADC samples) or uint32_t (presummed waveforms of dsp_icpc_compressed, n <= 4096).
 // bl_ext != NULL: the baseline mean of event e is bl_ext[e] instead of the bl_window mean (windowed waveforms of
 // dsp_icpc_compressed are shifted by blmean_presummed / presum_rate, src/dsp_icpc.jl:350).
@@ -1114,7 +1347,7 @@ icpc_kernel(const __grid_constant__ IcpcDev P, const SAMPLE* __restrict__ wf, lo
     }
     __syncthreads();
     // SG trace sample j of filter f
-    auto sg_at = [&](int f, int j) -> double { return sg_sample(P, TT, spar->sgg, f, j); };
+    auto sg_at = [&](int f, int j) -> double { return sg_sample(P.sg, TT, spar->sgg, f, j); };
     long long e = blockIdx.x;
     if (tid == 0 && e < n_events) {
         mbar_expect_tx(bar, wf_bytes);
@@ -1134,178 +1367,42 @@ icpc_kernel(const __grid_constant__ IcpcDev P, const SAMPLE* __restrict__ wf, lo
         // ==========================================================================================
         mbar_wait(bar, phase);
         phase ^= 1;
-        const SAMPLE* xp = xs + i0;
-        uint32_t csum = 0, cq = 0, cmn = 0xFFFFFFFFu, cmx = 0;
-#pragma unroll 1
-        for (int k = 0; k < cvalid; ++k) {
-            const uint32_t x = xp[k];
-            csum += x;
-            cq += csum;
-            cmn = min(cmn, x);
-            cmx = max(cmx, x);
-        }
-        // baseline regression sums (exact integers), samples of the window strided over ALL threads (the window covers the
-        // first chunks only: summed chunk-wise, three warps would do the whole job while the others wait at B1)
-        {
-            unsigned long long blSS = 0, blSX = 0;
-            uint32_t blS = 0;
-#pragma unroll 1
-            for (int idx = P.bl_from + tid; idx <= P.bl_until; idx += NT) {
-                const uint32_t x = xs[idx];
-                blS += x;
-                blSX += (unsigned long long)x * (unsigned long long)idx;
-                blSS += (unsigned long long)x * (unsigned long long)x;
-            }
-            // (all sums < 2^53: exact in double, in any order)
-            const double a = wsum_d((double)blS), b = wsum_d((double)blSS), c = wsum_d((double)blSX);
-            if (lane == 0) { red[R_BLS * NWARP + wid] = a; red[R_BLSS * NWARP + wid] = b; red[R_BLSX * NWARP + wid] = c; }
-        }
-        // saturation counts: a sample can only equal low/high if the chunk's min/max says so
-        int nlow = 0, nhigh = 0;
-        if ((int)cmn == P.sat_low || (int)cmx == P.sat_high) {
-            for (int k = 0; k < cvalid; ++k) {
-                const int x = xp[k];
-                nlow += (x == P.sat_low);
-                nhigh += (x == P.sat_high);
-            }
-        }
-        {
-            const uint32_t wmn = __reduce_min_sync(FULL, cmn), wmx = __reduce_max_sync(FULL, cmx);
-            const uint32_t wl = __reduce_add_sync(FULL, (uint32_t)nlow), wh = __reduce_add_sync(FULL, (uint32_t)nhigh);
-            if (lane == 0) {
-                uint32_t* ured = reinterpret_cast<uint32_t*>(red + R_MX * NWARP);   // 4 x NWARP uint32 in the R_MX/R_MN slots
-                ured[wid] = wmx; ured[NWARP + wid] = wmn; ured[2 * NWARP + wid] = wl; ured[3 * NWARP + wid] = wh;
-            }
-        }
-        // one scan for P = cumsum(x) and PP = cumsum(P): segments (len, s = sum x, q = sum of the inclusive
-        // prefix sums inside the segment) combine as (lenA+lenB, sA+sB, qA+qB+lenB*sA); all values exact
-        int sl = cvalid;
-        uint32_t ss = csum;
-        double sq = (double)cq;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            const int l2 = __shfl_up_sync(FULL, sl, o);
-            const uint32_t s2 = __shfl_up_sync(FULL, ss, o);
-            const double q2 = __shfl_up_sync(FULL, sq, o);
-            if (lane >= o) {
-                sq = q2 + sq + (double)sl * (double)s2;
-                ss += s2;
-                sl += l2;
-            }
-        }
-        if (lane == 31) {
-            red[R_SLEN * NWARP + wid] = (double)sl;
-            red[R_SS * NWARP + wid] = (double)ss;
-            red[R_SQ * NWARP + wid] = sq;
-        }
-        int el = __shfl_up_sync(FULL, sl, 1);
-        uint32_t es = __shfl_up_sync(FULL, ss, 1);
-        double eq = __shfl_up_sync(FULL, sq, 1);
-        if (lane == 0) { el = 0; es = 0; eq = 0.0; }
         // zero the masks and the queue counters of this event (committed with atomics later)
 #pragma unroll
         for (int q = 0; q < NMASK; ++q) masks[q * NWORDS + tid] = 0u;
         if (tid == 0) { ibuf[IB_QN] = 0; ibuf[IB_CZN] = 0; }
-        __syncthreads();   // ---- B1 ----
-
-        // exclusive prefixes of this thread's chunk
-        uint32_t P_excl;
-        double PP_excl;
-        {
-            double cs = 0.0, cqd = 0.0;
-#pragma unroll 1
-            for (int w = 0; w < wid; ++w) {
-                const double lw = red[R_SLEN * NWARP + w], sw = red[R_SS * NWARP + w], qw = red[R_SQ * NWARP + w];
-                cqd = cqd + qw + lw * cs;
-                cs += sw;
-            }
-            P_excl = (uint32_t)cs + es;
-            PP_excl = cqd + eq + (double)el * cs;
-        }
-        uint32_t mx, mn;
-        {
-            const uint32_t* ured = reinterpret_cast<const uint32_t*>(red + R_MX * NWARP);
-            const int l8 = lane & 7;
-            mx = __reduce_max_sync(FULL, ured[l8]);
-            mn = __reduce_min_sync(FULL, ured[NWARP + l8]);
-            nlow = (int)__reduce_add_sync(FULL, lane < 8 ? ured[2 * NWARP + l8] : 0u);
-            nhigh = (int)__reduce_add_sync(FULL, lane < 8 ? ured[3 * NWARP + l8] : 0u);
-        }
-
+        const SAMPLE* xp = xs + i0;
+        const RawPass rp = raw_pass<SAMPLE>(xs, i0, cvalid, P.bl_from, P.bl_until, P.sat_low, P.sat_high, (G & LGDSP_GROUP_LEAN) != 0,
+                                            red, tid, lane, wid);   // ---- B1 ----
+        const uint32_t mx = rp.mx, mn = rp.mn;
+        const int nlow = rp.nlow, nhigh = rp.nhigh;
         // saturation run lengths (only when a saturated sample exists; block-uniform branch)
         int cons_low = 0, cons_high = 0;
         if (nlow + nhigh > 0) {
-            Run rl = {0, 0, 0, cvalid}, rh = {0, 0, 0, cvalid};
-            {
-                int cl = 0, chh = 0;
-                bool pl = true, ph = true;
-                for (int k = 0; k < cvalid; ++k) {
-                    const int x = xp[k];
-                    const bool il = (x == P.sat_low), ih = (x == P.sat_high);
-                    cl = il ? cl + 1 : 0;
-                    chh = ih ? chh + 1 : 0;
-                    rl.best = max(rl.best, cl);
-                    rh.best = max(rh.best, chh);
-                    if (pl && il) rl.pre = cl; else pl = false;
-                    if (ph && ih) rh.pre = chh; else ph = false;
-                }
-                rl.suf = cl; rh.suf = chh;
-            }
-#pragma unroll
-            for (int o = 1; o < 32; o <<= 1) {
-                Run bl_ = run_shfl_down(rl, o), bh_ = run_shfl_down(rh, o);
-                if ((lane & (2 * o - 1)) == 0) { rl = run_merge(rl, bl_); rh = run_merge(rh, bh_); }
-            }
-            int* ired = reinterpret_cast<int*>(stash);   // stash is idle here
-            if (lane == 0) {
-                ired[wid * 8 + 0] = rl.pre; ired[wid * 8 + 1] = rl.suf; ired[wid * 8 + 2] = rl.best; ired[wid * 8 + 3] = rl.len;
-                ired[wid * 8 + 4] = rh.pre; ired[wid * 8 + 5] = rh.suf; ired[wid * 8 + 6] = rh.best; ired[wid * 8 + 7] = rh.len;
-            }
-            __syncthreads();
-            Run al = {ired[0], ired[1], ired[2], ired[3]}, ah = {ired[4], ired[5], ired[6], ired[7]};
-            for (int w = 1; w < NWARP; ++w) {
-                Run bl_ = {ired[w * 8], ired[w * 8 + 1], ired[w * 8 + 2], ired[w * 8 + 3]};
-                Run bh_ = {ired[w * 8 + 4], ired[w * 8 + 5], ired[w * 8 + 6], ired[w * 8 + 7]};
-                al = run_merge(al, bl_);
-                ah = run_merge(ah, bh_);
-            }
-            cons_low = al.best; cons_high = ah.best;
-            __syncthreads();
+            const int2 c = sat_runs<SAMPLE>(P.sat_low, P.sat_high, xp, cvalid, lane, wid, reinterpret_cast<int*>(stash));   // stash is idle here
+            cons_low = c.x; cons_high = c.y;
         }
 
         // (32-bit samples whose sum leaves 32 bits: the row is NaN instead of silently wrong)
         const bool wrapped = sum_exceeds_u32<SAMPLE>(xp, cvalid, mx, n, red + R_TLS * NWARP);
         // blmean = mean_Y = sum_Y * inv_n exactly as signalstats computes it (the other baseline statistics: P5)
         const double m = bl_ext ? div_rn(bl_ext[e * bl_stride], bl_div) : mul_rn(red_sum(red, R_BLS), P.bl_inv_n);
-        const double e_max = (double)mx - m, e_min = (double)mn - m;
+        const Levels lv = event_levels(m, mx, mn, P.tx_frac, (G & LGDSP_GROUP_LEAN) != 0);
+        const double e_max = lv.e_max, e_min = lv.e_min;
         double thr[5];
 #pragma unroll
-        for (int k = 0; k < 5; ++k) thr[k] = e_max * P.tx_frac[k];
+        for (int k = 0; k < 5; ++k) thr[k] = lv.thr[k];
 
         // ==========================================================================================
         // P2: prefix sums of the pole-zero waveform; t10..t99 masks; tail log-regression
         // ==========================================================================================
         {
             const double km1 = P.km1;
-            const double Sd0 = fma(-(double)i0, m, u2d(P_excl));                      // cumsum(w)[i0-1]
-            const double tri0 = 0.5 * (double)i0 * ((double)i0 + 1.0);
-            const double TT0 = fma(km1, fma(-tri0, m, PP_excl), Sd0);                 // TT[i0] (bit-identical to the neighbour's)
+            PzChunk pz = pz_chunk(i0, m, km1, rp.P_excl, rp.PP_excl, rp.cmn, rp.cmx);
+            const double TT0 = pz.TT0, ylo = pz.ylo, yhi = pz.yhi, guard = pz.guard;
             {
-                uint32_t Pr = P_excl;
-                double PPr = PP_excl;
-                double ip1 = (double)i0;                                  // becomes i+1 inside the loop
-                double tri = tri0;                                        // (i+1)(i+2)/2 after the update
                 double* tp = TT + i0 + 1;
-                auto body = [&](int k) {
-                    Pr += xp[k];
-                    const double Pd = u2d(Pr);
-                    PPr += Pd;
-                    ip1 += 1.0;
-                    tri += ip1;
-                    const double Sd = fma(-ip1, m, Pd);                // cumsum(w)[i]
-                    const double SS = fma(-tri, m, PPr);                // cumsum(cumsum(w))[i]
-                    tp[k] = fma(km1, SS, Sd);                           // cumsum(y)[i]
-                };
+                auto body = [&](int k) { tp[k] = pz.scan.next(xp[k], m, km1); };
                 int k = 0;
 #pragma unroll 1
                 for (; k + 3 <= cvalid; k += 3) { body(k); body(k + 1); body(k + 2); }
@@ -1313,13 +1410,6 @@ icpc_kernel(const __grid_constant__ IcpcDev P, const SAMPLE* __restrict__ wf, lo
                 for (; k < cvalid; ++k) body(k);
                 if (tid == 0) TT[0] = 0.0;
             }
-            // Conservative bounds of y = w + km1*cumsum(w) on the chunk from the integer min/max of the raw samples:
-            // cumsum(w)[i0+k] lies between S0 + (k+1)*wmin and S0 + (k+1)*wmax.
-            const double wmin = (double)cmn - m, wmax = (double)cmx - m;
-            const double ak = fabs(km1);
-            const double srange = (double)CH * fmax(fabs(wmin), fabs(wmax));
-            const double ylo = wmin + km1 * Sd0 - ak * srange, yhi = wmax + km1 * Sd0 + ak * srange;
-            const double guard = 1e-9 * (fabs(ylo) + fabs(yhi)) + 1e-6;   // >> rounding of the TT differences
             // t10..t99: a chunk entirely below (above) a threshold contributes zeros (ones) without a compare
             if (G & LGDSP_GROUP_TIMING) {
                 uint32_t lo[5] = {0, 0, 0, 0, 0}, hi = 0;   // bits 0..31 of every threshold; bit t of hi = sample 32
@@ -1848,25 +1938,7 @@ icpc_kernel(const __grid_constant__ IcpcDev P, const SAMPLE* __restrict__ wf, lo
             }
         } else if (wid == 5) {
             if (G & LGDSP_GROUP_CURRENT) {
-                // get_wvf_maximum  src/interpolation.jl:30-46: parabola only if strictly inside the window
-                double vv[4];
-                int aa[4];
-#pragma unroll
-                for (int f = 0; f < 4; ++f) {
-                    const int fs = (f < 3 && P.sg_alias[f] >= 0) ? P.sg_alias[f] : f;   // aliased filter: same trace and window
-                    red_argmax(red, R_CMAX0 + fs, R_CARG0 + fs, vv[f], aa[f]);
-                }
-                if (lane < 4) {
-                    const int f = lane;
-                    double v = f == 0 ? vv[0] : f == 1 ? vv[1] : f == 2 ? vv[2] : vv[3];
-                    const int a = f == 0 ? aa[0] : f == 1 ? aa[1] : f == 2 ? aa[2] : aa[3];
-                    if (a > P.cur_from[f] && a < P.cur_until[f]) {
-                        const double y1 = (f < 3) ? sg_at(f, a - 1) : deriv_at(TT, a - 1);
-                        const double y3 = (f < 3) ? sg_at(f, a + 1) : deriv_at(TT, a + 1);
-                        v = extrema3(y1, v, y3);
-                    }
-                    row[LGDSP_COL_a_sg + f] = v;
-                }
+                currents_job(TT, P.sg, spar->sgg, P.sg_alias, P.cur_from, P.cur_until, red, R_CMAX0, R_CARG0, row, lane);
             }
             if (G & LGDSP_GROUP_INTRACE) {
                 // crossing resolution of the sg[0] masks (complete since Bq), then t50_current and the in-trace pile-up

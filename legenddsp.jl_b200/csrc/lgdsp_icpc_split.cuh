@@ -14,17 +14,19 @@
 //
 // (reference lines: /root/reference/src/dsp_icpc.jl).  The three kernels of one event batch run back to back on a stream;
 // the batch is sized so that its prefix sums (65.6 KB per event) are still in L2 when the consumers read them.
-// Every value is produced by the same expressions as in icpc_kernel (same helpers, same operation order); the crossing, t0
-// and Q-drift evaluations of phase C, sg_sample and the CUSP/ZAC candidate bound are functions in lgdsp_icpc.cu that both
-// paths call.
+// Every value is produced by the same expressions as in icpc_kernel (same helpers, same operation order).  Functions in
+// lgdsp_icpc.cu that both paths call: the raw-sample pass (raw_pass), the saturation run lengths (sat_runs), the levels
+// e_max / e_min / thresholds (event_levels), the closed-form pole-zero prefix sums (pz_chunk / PzScan), the crossing, t0
+// and Q-drift evaluations of phase C (tx_us_at, t0_us_at, qdrift_at), the currents job (currents_job), sg_sample and the
+// CUSP/ZAC candidate bound (cz_candidate).  The PZ tail sums, the SG window pass, the mask thresholds, the flagged-interval
+// rules and evaluation and the t50_current / in-trace evaluations are still written in both kernels (DESIGN.md 4.1).
 
 constexpr int TTG_LEN = TT_LEN;     // doubles per event slot of the global prefix-sum ring
 constexpr int AUX_LEN = 16;         // doubles per event: values handed from the prefix kernel to the consumers
 enum { AX_M = 0, AX_EMAX = 1, AX_YMAX = 2, AX_THR = 3 /* 5 */, AX_POS = 8 /* 5 */, AX_BAD = 13 /* 1: sample sum beyond 32 bits */ };
 
 // ---- prefix kernel: shared memory ----
-enum { K1R_BLS = 0, K1R_BLSS, K1R_BLSX, K1R_MX /* + K1R_MN: 4 x NWARP uint32 */, K1R_MN, K1R_SLEN, K1R_SS, K1R_SQ,
-       K1R_TLS, K1R_TLSS, K1R_TLSX, K1R_TLBAD, K1R_YMAX, K1R_N };
+enum { K1R_TLS = R_RAW_N, K1R_TLSS, K1R_TLSX, K1R_TLBAD, K1R_YMAX, K1R_N };
 
 constexpr int K1_XS = 0;                                   // 2 x (MAXN * 2) bytes: double-buffered raw samples
 constexpr int K1_MASK = K1_XS + 2 * MAXN * 2;              // uint32 masks[5][NWORDS]: t10..t99
@@ -89,141 +91,25 @@ icpc_prefix_kernel(const __grid_constant__ IcpcDev P, const SAMPLE* __restrict__
         // raw samples (same as P1 of icpc_kernel)
         // ==========================================================================================
         const SAMPLE* xp = xs + i0;
-        uint32_t csum = 0, cq = 0, cmn = 0xFFFFFFFFu, cmx = 0;
-#pragma unroll 3
-        for (int k = 0; k < cvalid; ++k) {
-            const uint32_t x = xp[k];
-            csum += x;
-            cq += csum;
-            cmn = min(cmn, x);
-            cmx = max(cmx, x);
-        }
-        {
-            unsigned long long blSS = 0, blSX = 0;
-            uint32_t blS = 0;
-#pragma unroll 2
-            for (int idx = P.bl_from + tid; idx <= P.bl_until; idx += NT) {
-                const uint32_t x = xs[idx];
-                blS += x;
-                if (!lean) {   // (slope / sigma of the baseline are not among the lean columns)
-                    blSX += (unsigned long long)x * (unsigned long long)idx;
-                    blSS += (unsigned long long)x * (unsigned long long)x;
-                }
-            }
-            const double a = wsum_d((double)blS), bq = wsum_d((double)blSS), c = wsum_d((double)blSX);
-            if (lane == 0) { red[K1R_BLS * NWARP + wid] = a; red[K1R_BLSS * NWARP + wid] = bq; red[K1R_BLSX * NWARP + wid] = c; }
-        }
-        int nlow = 0, nhigh = 0;
-        if ((int)cmn == P.sat_low || (int)cmx == P.sat_high) {
-            for (int k = 0; k < cvalid; ++k) {
-                const int x = xp[k];
-                nlow += (x == P.sat_low);
-                nhigh += (x == P.sat_high);
-            }
-        }
-        {
-            const uint32_t wmn = __reduce_min_sync(FULL, cmn), wmx = __reduce_max_sync(FULL, cmx);
-            const uint32_t wl = __reduce_add_sync(FULL, (uint32_t)nlow), wh = __reduce_add_sync(FULL, (uint32_t)nhigh);
-            if (lane == 0) {
-                uint32_t* ured = reinterpret_cast<uint32_t*>(red + K1R_MX * NWARP);
-                ured[wid] = wmx; ured[NWARP + wid] = wmn; ured[2 * NWARP + wid] = wl; ured[3 * NWARP + wid] = wh;
-            }
-        }
-        int sl = cvalid;
-        uint32_t ss = csum;
-        double sq = (double)cq;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            const int l2 = __shfl_up_sync(FULL, sl, o);
-            const uint32_t s2 = __shfl_up_sync(FULL, ss, o);
-            const double q2 = __shfl_up_sync(FULL, sq, o);
-            if (lane >= o) {
-                sq = q2 + sq + (double)sl * (double)s2;
-                ss += s2;
-                sl += l2;
-            }
-        }
-        if (lane == 31) {
-            red[K1R_SLEN * NWARP + wid] = (double)sl;
-            red[K1R_SS * NWARP + wid] = (double)ss;
-            red[K1R_SQ * NWARP + wid] = sq;
-        }
-        int el = __shfl_up_sync(FULL, sl, 1);
-        uint32_t es = __shfl_up_sync(FULL, ss, 1);
-        double eq = __shfl_up_sync(FULL, sq, 1);
-        if (lane == 0) { el = 0; es = 0; eq = 0.0; }
-        __syncthreads();   // ---- B1 ----
-
-        uint32_t P_excl;
-        double PP_excl;
-        {
-            double cs = 0.0, cqd = 0.0;
-#pragma unroll 1
-            for (int w = 0; w < wid; ++w) {
-                const double lw = red[K1R_SLEN * NWARP + w], sw = red[K1R_SS * NWARP + w], qw = red[K1R_SQ * NWARP + w];
-                cqd = cqd + qw + lw * cs;
-                cs += sw;
-            }
-            P_excl = (uint32_t)cs + es;
-            PP_excl = cqd + eq + (double)el * cs;
-        }
-        uint32_t mx, mn;
-        {
-            const uint32_t* ured = reinterpret_cast<const uint32_t*>(red + K1R_MX * NWARP);
-            const int l8 = lane & 7;
-            mx = __reduce_max_sync(FULL, ured[l8]);
-            mn = __reduce_min_sync(FULL, ured[NWARP + l8]);
-            nlow = (int)__reduce_add_sync(FULL, lane < 8 ? ured[2 * NWARP + l8] : 0u);
-            nhigh = (int)__reduce_add_sync(FULL, lane < 8 ? ured[3 * NWARP + l8] : 0u);
-        }
+        const RawPass rp = raw_pass<SAMPLE>(xs, i0, cvalid, P.bl_from, P.bl_until, P.sat_low, P.sat_high, lean, red, tid, lane, wid);
+        const uint32_t mx = rp.mx, mn = rp.mn;
+        const int nlow = rp.nlow, nhigh = rp.nhigh;
         int cons_low = 0, cons_high = 0;
         if (nlow + nhigh > 0) {
-            Run rl = {0, 0, 0, cvalid}, rh = {0, 0, 0, cvalid};
-            {
-                int cl = 0, chh = 0;
-                bool pl = true, ph = true;
-                for (int k = 0; k < cvalid; ++k) {
-                    const int x = xp[k];
-                    const bool il = (x == P.sat_low), ih = (x == P.sat_high);
-                    cl = il ? cl + 1 : 0;
-                    chh = ih ? chh + 1 : 0;
-                    rl.best = max(rl.best, cl);
-                    rh.best = max(rh.best, chh);
-                    if (pl && il) rl.pre = cl; else pl = false;
-                    if (ph && ih) rh.pre = chh; else ph = false;
-                }
-                rl.suf = cl; rh.suf = chh;
-            }
-#pragma unroll
-            for (int o = 1; o < 32; o <<= 1) {
-                Run bl_ = run_shfl_down(rl, o), bh_ = run_shfl_down(rh, o);
-                if ((lane & (2 * o - 1)) == 0) { rl = run_merge(rl, bl_); rh = run_merge(rh, bh_); }
-            }
-            if (lane == 0) {
-                ired[wid * 8 + 0] = rl.pre; ired[wid * 8 + 1] = rl.suf; ired[wid * 8 + 2] = rl.best; ired[wid * 8 + 3] = rl.len;
-                ired[wid * 8 + 4] = rh.pre; ired[wid * 8 + 5] = rh.suf; ired[wid * 8 + 6] = rh.best; ired[wid * 8 + 7] = rh.len;
-            }
-            __syncthreads();
-            Run al = {ired[0], ired[1], ired[2], ired[3]}, ah = {ired[4], ired[5], ired[6], ired[7]};
-            for (int w = 1; w < NWARP; ++w) {
-                Run bl_ = {ired[w * 8], ired[w * 8 + 1], ired[w * 8 + 2], ired[w * 8 + 3]};
-                Run bh_ = {ired[w * 8 + 4], ired[w * 8 + 5], ired[w * 8 + 6], ired[w * 8 + 7]};
-                al = run_merge(al, bl_);
-                ah = run_merge(ah, bh_);
-            }
-            cons_low = al.best; cons_high = ah.best;
-            __syncthreads();   // the partials share their storage with the threshold masks written below
+            // (the partials share their storage with the threshold masks written below)
+            const int2 c = sat_runs<SAMPLE>(P.sat_low, P.sat_high, xp, cvalid, lane, wid, ired);
+            cons_low = c.x; cons_high = c.y;
         }
 
         // 32-bit samples: the prefix sums are exact uint32 only while the waveform sums to < 2^32 (any 16-bit trace does; a
         // presummed trace does up to a mean of 2^20).  Beyond that the event's row is NaN instead of silently wrong.
         const bool wrapped = sum_exceeds_u32<SAMPLE>(xp, cvalid, mx, n, red + K1R_TLS * NWARP);
-        const double m = bl_ext ? div_rn(bl_ext[e * bl_stride], bl_div) : mul_rn(red_sum(red, K1R_BLS), P.bl_inv_n);
-        const double e_max = (double)mx - m, e_min = (double)mn - m;
+        const double m = bl_ext ? div_rn(bl_ext[e * bl_stride], bl_div) : mul_rn(red_sum(red, R_BLS), P.bl_inv_n);
+        const Levels lv = event_levels(m, mx, mn, P.tx_frac, lean);
+        const double e_max = lv.e_max, e_min = lv.e_min;
         double thr[5];
 #pragma unroll
-        for (int k = 0; k < 5; ++k) thr[k] = e_max * P.tx_frac[k];
-        if (lean) { thr[0] = CUDART_INF; thr[2] = CUDART_INF; thr[3] = CUDART_INF; thr[4] = CUDART_INF; }   // only t50
+        for (int k = 0; k < 5; ++k) thr[k] = lv.thr[k];
 
         // ==========================================================================================
         // prefix sums of the pole-zero waveform -> global ring; t10..t99 masks from the values in flight
@@ -231,14 +117,8 @@ icpc_prefix_kernel(const __grid_constant__ IcpcDev P, const SAMPLE* __restrict__
         double* tg = ttg + e * TTG_LEN;
         {
             const double km1 = P.km1;
-            const double Sd0 = fma(-(double)i0, m, u2d(P_excl));
-            const double tri0 = 0.5 * (double)i0 * ((double)i0 + 1.0);
-            const double TT0 = fma(km1, fma(-tri0, m, PP_excl), Sd0);
-            const double wmin = (double)cmn - m, wmax = (double)cmx - m;
-            const double ak = fabs(km1);
-            const double srange = (double)CH * fmax(fabs(wmin), fabs(wmax));
-            const double ylo = wmin + km1 * Sd0 - ak * srange, yhi = wmax + km1 * Sd0 + ak * srange;
-            const double guard = 1e-9 * (fabs(ylo) + fabs(yhi)) + 1e-6;
+            PzChunk pz = pz_chunk(i0, m, km1, rp.P_excl, rp.PP_excl, rp.cmn, rp.cmx);
+            const double ylo = pz.ylo, yhi = pz.yhi, guard = pz.guard;
             bool straddle = false;
             if (G & LGDSP_GROUP_TIMING) {
 #pragma unroll
@@ -249,25 +129,11 @@ icpc_prefix_kernel(const __grid_constant__ IcpcDev P, const SAMPLE* __restrict__
             const bool wstr = __any_sync(FULL, straddle);   // warp-uniform: compare inside the loop or not
             uint32_t lo[5] = {0, 0, 0, 0, 0}, hi = 0;
             {
-                uint32_t Pr = P_excl;
-                double PPr = PP_excl;
-                double ip1 = (double)i0;
-                double tri = tri0;
-                auto body = [&](int k) -> double {
-                    Pr += xp[k];
-                    const double Pd = u2d(Pr);
-                    PPr += Pd;
-                    ip1 += 1.0;
-                    tri += ip1;
-                    const double Sd = fma(-ip1, m, Pd);
-                    const double SS = fma(-tri, m, PPr);
-                    return fma(km1, SS, Sd);
-                };
                 // The chunk values go to HBM through a per-warp staging tile, eight samples of every chunk at a time: the warp then
                 // stores runs of eight consecutive doubles (whole 32-byte sectors) instead of 32 scattered 8-byte words per
                 // instruction, which quartered the L2 write traffic of this kernel.
                 double* tile = reinterpret_cast<double*>(smem + K1_TILE) + wid * (32 * TILE_LD);
-                double tprev = TT0;
+                double tprev = pz.TT0;
                 const int cbase = wid * 32;   // first chunk of this warp
                 // store pass: lane -> (chunk 4r + lane/8, sample kb + lane%8); everything but r and kb is loop invariant.
                 // (tile rows 1 apart share one bank pair per half warp: 17 % of this kernel's SMEM wavefronts are that 2-way
@@ -279,7 +145,7 @@ icpc_prefix_kernel(const __grid_constant__ IcpcDev P, const SAMPLE* __restrict__
                 const bool wfull = (cbase + 32) * CH <= n;                        // every chunk of this warp is complete
                 // sample k of the chunk: prefix sum, threshold bits, scan step
                 auto sample = [&](int k, bool with_thr) -> double {
-                    const double tn = body(k);
+                    const double tn = pz.scan.next(xp[k], m, km1);
                     if (with_thr) {
                         const double y = tn - tprev;     // = TT[i+1] - TT[i] as every consumer forms it
                         if (k < 32) {
@@ -468,7 +334,7 @@ icpc_prefix_kernel(const __grid_constant__ IcpcDev P, const SAMPLE* __restrict__
             if (lane == 0) { ax[AX_POS + wid] = (double)pos; ax[AX_THR + wid] = thr[wid == 0 ? 0 : wid == 1 ? 1 : wid == 2 ? 2 : wid == 3 ? 3 : 4]; }
         } else if (wid == 5) {
             // baseline [:102] and tailstats [:115] (lane 0 / lane 1, same code path)
-            const double blS = red_sum(red, K1R_BLS), blSS = red_sum(red, K1R_BLSS), blSX = red_sum(red, K1R_BLSX);
+            const double blS = red_sum(red, R_BLS), blSS = red_sum(red, R_BLSS), blSX = red_sum(red, R_BLSX);
             const double tlS = red_sum(red, K1R_TLS), tlSS = red_sum(red, K1R_TLSS), tlSX = red_sum(red, K1R_TLSX);
             const double tlbad = red_sum(red, K1R_TLBAD);
             if (lane < 2) {
@@ -554,7 +420,7 @@ icpc_extract_kernel(const __grid_constant__ IcpcDev P, const double* __restrict_
     if (tid < TT_LEN - 2 - n) TT[n + 2 + tid] = 0.0;   // finite padding behind the loaded part (zero-padded SG kernels read it)
     if (tid < 24) sgg[tid >> 3][tid & 7] = P.sg[tid >> 3].gg[tid & 7];
     __syncthreads();
-    auto sg_at = [&](int f, int j) -> double { return sg_sample(P, TT, sgg, f, j); };
+    auto sg_at = [&](int f, int j) -> double { return sg_sample(P.sg, TT, sgg, f, j); };
     const int i0 = tid * CH;
     const int nsg = P.sg[0].nout;
     const bool want_cur = (G & LGDSP_GROUP_CURRENT) != 0, want_intr = (G & LGDSP_GROUP_INTRACE) != 0;
@@ -923,25 +789,7 @@ icpc_extract_kernel(const __grid_constant__ IcpcDev P, const double* __restrict_
             }
         } else if (wid == 3) {
             if (G & LGDSP_GROUP_CURRENT) {
-                // get_wvf_maximum  src/interpolation.jl:30-46: parabola only if strictly inside the window
-                double vv[4];
-                int aa[4];
-#pragma unroll
-                for (int f = 0; f < 4; ++f) {
-                    const int fs = (f < 3 && P.sg_alias[f] >= 0) ? P.sg_alias[f] : f;
-                    red_argmax(red, K2R_CMAX0 + fs, K2R_CARG0 + fs, vv[f], aa[f]);
-                }
-                if (lane < 4) {
-                    const int f = lane;
-                    double v = f == 0 ? vv[0] : f == 1 ? vv[1] : f == 2 ? vv[2] : vv[3];
-                    const int a = f == 0 ? aa[0] : f == 1 ? aa[1] : f == 2 ? aa[2] : aa[3];
-                    if (a > P.cur_from[f] && a < P.cur_until[f]) {
-                        const double y1 = (f < 3) ? sg_at(f, a - 1) : deriv_at(TT, a - 1);
-                        const double y3 = (f < 3) ? sg_at(f, a + 1) : deriv_at(TT, a + 1);
-                        v = extrema3(y1, v, y3);
-                    }
-                    row[LGDSP_COL_a_sg + f] = v;
-                }
+                currents_job(TT, P.sg, sgg, P.sg_alias, P.cur_from, P.cur_until, red, K2R_CMAX0, K2R_CARG0, row, lane);
             }
         } else if (wid == 4) {
             if (G & LGDSP_GROUP_INTRACE) {
